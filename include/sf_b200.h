@@ -151,8 +151,8 @@ int sf_render(sf_handle* h, uint8_t* d_obs, int flags, void* stream);
  * straight from/to the caller's buffers (use sf_host_alloc for them). h_obs may be NULL. Runs on streams the handle
  * owns: the slab is stepped in slices of consecutive envs so that the kernel of one slice overlaps the device->host
  * copy of the previous one. Ordered after everything queued with stream == NULL; work queued on any OTHER stream for
- * this handle must have completed before the call (sf_set_ticks, sf_get_state and sf_set_state synchronise the
- * device themselves).
+ * this handle (sf_save_envs and sf_load_envs included) must have completed before the call (sf_set_ticks, sf_get_state
+ * and sf_set_state synchronise the device themselves).
  * SF_FLAG_HOST_DELTA: the caller promises that h_obs is page-locked (sf_host_alloc / cudaHostAlloc / cudaHostRegister,
  * 16-byte aligned) and that nothing but sf_step_host of this handle has written to it since the previous call that
  * passed the same pointer with this flag (see sf_host_forget). The frames of consecutive steps differ in a few dozen
@@ -178,6 +178,31 @@ int sf_host_free(void* p);
 /* State records, host side (synchronous). first..first+count-1. */
 int sf_get_state(sf_handle* h, int first, int count, sf_state_record* h_out);
 int sf_set_state(sf_handle* h, int first, int count, const sf_state_record* h_in);
+
+/* Env blobs: one env's complete game state as one fixed-size row, written and read on the device (checkpoint and resume,
+ * forking an env into many slots, moving envs between handles or GPUs). Byte layout of a row (little endian):
+ *     0  header: uint32 SF_ENV_BLOB_MAGIC, uint32 SF_ENV_BLOB_VERSION, uint32 gametype (0 youturn, 1 autoturn,
+ *        2 test-youturn, 3 test-autoturn), uint32 0
+ *    16  ship pos (double x, y), vel (double vx, vy)
+ *    48  q0..q3 (int4 each: core word, live-slot mask, timers, points, tick, running episode return, prev_vlner)
+ *   112  st0..st3 (int4 each: the 13 Stats counters, rand() ring index, rand() calls consumed, seed)
+ *   176  missile pos[20] (double x, y)           496  shell pos[4], 560 shell vel[4] (double x, y)
+ *   624  shell angle[4] (double)                 656  missile angle[20] (int16, degrees)
+ *   696  rand() ring[31] (uint32)                820  zero up to SF_ENV_BLOB_BYTES
+ * Rows are canonical: dead missile and shell slots and all padding are zero, so two envs in the same state give
+ * byte-identical rows. Not in a row: the render caches (memos: a load invalidates them), the per-handle episode-stat
+ * accumulators and the handle's first_global_env label. */
+#define SF_ENV_BLOB_BYTES 832
+#define SF_ENV_BLOB_VERSION 1
+#define SF_ENV_BLOB_MAGIC 0x42465353u /* "SSFB" */
+/* Row k of d_blob <- env d_env_idx[k] (d_env_idx == NULL: envs 0..count-1). An index outside [0, n) gives an all-zero
+ * row (which a load rejects). d_blob is 16-byte aligned. Asynchronous on `stream`. */
+int sf_save_envs(sf_handle* h, const int32_t* d_env_idx, int count, uint8_t* d_blob, void* stream);
+/* Env d_env_idx[k] <- row k of d_blob (d_env_idx == NULL: envs 0..count-1). Rows with a bad header (magic, version or a
+ * gametype other than the handle's) or a target index outside [0, n) are skipped and added to *d_rejected (int32,
+ * device, may be NULL). Target indices must not repeat within one call; the same row may be loaded into many envs.
+ * The loaded envs' render caches are invalidated. d_blob is 16-byte aligned. Asynchronous on `stream`. */
+int sf_load_envs(sf_handle* h, const uint8_t* d_blob, const int32_t* d_env_idx, int count, int32_t* d_rejected, void* stream);
 
 /* Finished-episode statistics accumulated on the device since the last call with reset!=0:
  * int64[SF_NUM_EPISODE_STATS] = {episodes, sum_return, sum_return^2, sum_length, sum of the 13 Stats

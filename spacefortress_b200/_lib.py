@@ -22,6 +22,9 @@ KEY_FIRE, KEY_THRUST, KEY_LEFT, KEY_RIGHT = 1, 2, 4, 8
 MAX_HOST_MIRRORS = 4  # SF_MAX_MIRRORS: host observation buffers whose contents the library remembers per handle
 FLAG_RENDER, FLAG_NO_AUTORESET, FLAG_ACTIONS_ARE_KEYMASKS, FLAG_NATIVE_OBS, FLAG_RAW_REWARD, FLAG_HOST_DELTA = 1, 2, 4, 8, 16, 32
 
+ENV_BLOB_BYTES = 832  # SF_ENV_BLOB_BYTES: one env's complete game state as one row (sf_save_envs / sf_load_envs)
+ENV_BLOB_VERSION = 1  # SF_ENV_BLOB_VERSION
+
 OBS_TYPES = {"image": 0, "features": 1, "normalized-features": 2, "monitors": 3}  # ssf_env.py:51
 
 EVENT_BITS = {
@@ -94,6 +97,8 @@ _PROTOTYPES = {
     "sf_host_free": (C.c_int, [C.c_void_p]),
     "sf_get_state": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "sf_set_state": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
+    "sf_save_envs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "sf_load_envs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "sf_episode_stats": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "sf_num_features": (C.c_int, [C.c_void_p, C.c_int]),
     "sf_features": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),

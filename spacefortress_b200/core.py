@@ -89,6 +89,35 @@ class Game(object):
         _lib.check(self.L.sf_set_state(self.h, 0, 1, arr))
         self._rec = None
 
+    def clone_state(self):
+        """The complete game state as a host uint8 array [ENV_BLOB_BYTES] (one sf_save_envs row; it pickles). Unlike
+        the record it holds the rand() stream itself, so restore_state does not replay it."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        with torch.cuda.device(dev):
+            o = torch.empty((1, _lib.ENV_BLOB_BYTES), dtype=torch.uint8, device=dev)
+            _lib.check(self.L.sf_save_envs(self.h, None, 1, C.c_void_p(o.data_ptr()), C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+            return o[0].cpu().numpy()
+
+    def restore_state(self, blob):
+        """Continue from a state clone_state returned (of a Game of the same config). Key presses since the last tick
+        are dropped."""
+        import torch
+        b = np.asarray(blob)
+        if b.dtype != np.uint8 or b.shape != (_lib.ENV_BLOB_BYTES,):
+            raise ValueError("blob must be a uint8 array of shape (%d,)" % _lib.ENV_BLOB_BYTES)
+        dev = torch.device("cuda", self.device)
+        with torch.cuda.device(dev):
+            t = torch.from_numpy(np.ascontiguousarray(b).reshape(1, -1)).to(dev)
+            rejected = torch.zeros(1, dtype=torch.int32, device=dev)
+            _lib.check(self.L.sf_load_envs(self.h, C.c_void_p(t.data_ptr()), None, 1, C.c_void_p(rejected.data_ptr()),
+                                           C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)))
+            if int(rejected.item()):
+                raise _lib.SFError("restore_state: not a state of a %r game (bad magic, version or game type)" % self.gametype)
+        self._rec = None
+        self._keys = None
+        self._touched = []
+
     def _current_keymask(self):
         r = self.record
         return (_lib.KEY_FIRE if r.fire_flag else 0) | (_lib.KEY_THRUST if r.thrust_flag else 0) | \

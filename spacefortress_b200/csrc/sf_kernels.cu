@@ -594,6 +594,154 @@ __global__ void sf_set_state_kernel(SfDev D, int first, int count, const sf_stat
   sf_store_env(D, i, e);
 }
 
+// ---- env blobs (sf_save_envs / sf_load_envs): SoA <-> one SF_ENV_BLOB_BYTES row per env, layout in sf_b200.h ----
+// One warp per block moves a tile of 32 envs through shared memory. On the SoA side lane l handles env l of the tile (a
+// warp access is 512 B per int4 array and 128 B per rand() word when the indices are contiguous); on the blob side the
+// lanes run over the 16-byte chunks of the tile's 32 consecutive rows, so the rows are read and written fully coalesced.
+// Global -> shared moves are cp.async: a warp has the whole tile in flight without holding it in registers.
+#define SF_BLOB_CHUNKS (SF_ENV_BLOB_BYTES / 16)
+#define SF_BLOB_PITCH (SF_BLOB_CHUNKS + 1)  // shared row pitch in chunks: odd, so the 8 lanes of a 16-byte phase hit 8 bank quads
+#define SF_BLOB_BLOCKS_PER_SM 8             // 8 x 27 KB of shared memory
+enum { SF_BO_POS = 16, SF_BO_VEL = 32, SF_BO_Q = 48, SF_BO_ST = 112, SF_BO_MPOS = 176, SF_BO_SPOS = 496, SF_BO_SVEL = 560,
+       SF_BO_SANG = 624, SF_BO_MANG = 656, SF_BO_RNG = 696, SF_BO_END = 820 };
+static_assert(SF_BO_MANG + 2 * SF_MAX_MISSILES == SF_BO_RNG && SF_BO_RNG + 4 * SF_RNG_WORDS == SF_BO_END, "blob layout");
+static_assert(SF_BO_END <= SF_ENV_BLOB_BYTES && SF_ENV_BLOB_BYTES % 16 == 0, "blob size");
+
+__device__ __forceinline__ void sf_cp_async(void* smem, const void* gmem, int bytes) {
+  const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
+  if (bytes == 16) asm volatile("cp.async.cg.shared.global [%0], [%1], 16;\n" ::"r"(s), "l"(gmem) : "memory");
+  else if (bytes == 8) asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(s), "l"(gmem) : "memory");
+  else asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(s), "l"(gmem) : "memory");
+}
+__device__ __forceinline__ void sf_cp_async_wait() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
+
+__global__ void __launch_bounds__(32) sf_save_envs_kernel(SfDev D, int gametype, const int* __restrict__ idx, int count, int4* __restrict__ blob) {
+  __shared__ int4 tile[32 * SF_BLOB_PITCH];
+  const int lane = threadIdx.x;
+  const size_t np = (size_t)D.n_pad;
+  int4* row = tile + lane * SF_BLOB_PITCH;
+  char* rb = reinterpret_cast<char*>(row);
+  const int4 z = make_int4(0, 0, 0, 0);
+  for (int base = blockIdx.x * 32; base < count; base += gridDim.x * 32) {
+    const int k = base + lane;
+    const int i = k < count ? (idx ? idx[k] : k) : -1;
+    if (i >= 0 && i < D.n) {
+      const int4 q0 = D.q0[i];
+      const unsigned pm = (unsigned)q0.y;
+      row[0] = make_int4((int)SF_ENV_BLOB_MAGIC, SF_ENV_BLOB_VERSION, gametype, 0);
+      sf_cp_async(rb + SF_BO_POS, &D.pos[i], 16);
+      sf_cp_async(rb + SF_BO_VEL, &D.vel[i], 16);
+      row[SF_BO_Q / 16] = q0;
+      sf_cp_async(rb + SF_BO_Q + 16, &D.q1[i], 16);
+      sf_cp_async(rb + SF_BO_Q + 32, &D.q2[i], 16);
+      sf_cp_async(rb + SF_BO_Q + 48, &D.q3[i], 16);
+      sf_cp_async(rb + SF_BO_ST, &D.st0[i], 16);
+      sf_cp_async(rb + SF_BO_ST + 16, &D.st1[i], 16);
+      sf_cp_async(rb + SF_BO_ST + 32, &D.st2[i], 16);
+      sf_cp_async(rb + SF_BO_ST + 48, &D.st3[i], 16);
+      short* mang = reinterpret_cast<short*>(rb + SF_BO_MANG);
+#pragma unroll
+      for (int s = 0; s < SF_MAX_MISSILES; s++) {
+        const bool live = (pm >> s) & 1u;
+        if (live) sf_cp_async(rb + SF_BO_MPOS + 16 * s, &D.mpos[s * np + i], 16);
+        else row[SF_BO_MPOS / 16 + s] = z;  // dead slots are zero: equal states give equal rows
+        mang[s] = live ? D.mang[s * np + i] : (short)0;
+      }
+#pragma unroll
+      for (int s = 0; s < SF_DEV_SHELLS; s++) {
+        if ((pm >> (SF_PMASK_SHELL_SHIFT + s)) & 1u) {
+          sf_cp_async(rb + SF_BO_SPOS + 16 * s, &D.spos[s * np + i], 16);
+          sf_cp_async(rb + SF_BO_SVEL + 16 * s, &D.svel[s * np + i], 16);
+          sf_cp_async(rb + SF_BO_SANG + 8 * s, &D.sang[s * np + i], 8);
+        } else {
+          row[SF_BO_SPOS / 16 + s] = z;
+          row[SF_BO_SVEL / 16 + s] = z;
+          reinterpret_cast<double*>(rb + SF_BO_SANG)[s] = 0.0;
+        }
+      }
+#pragma unroll
+      for (int w = 0; w < SF_RNG_WORDS; w++) sf_cp_async(rb + SF_BO_RNG + 4 * w, &D.rng[w * np + i], 4);
+      for (int b = SF_BO_END; b < SF_ENV_BLOB_BYTES; b += 4) *reinterpret_cast<int*>(rb + b) = 0;
+    } else if (k < count) {
+      for (int c = 0; c < SF_BLOB_CHUNKS; c++) row[c] = z;  // no such env
+    }
+    sf_cp_async_wait();
+    __syncwarp();
+    const int rows = min(32, count - base);
+    int4* out = blob + (size_t)base * SF_BLOB_CHUNKS;
+#pragma unroll 4
+    for (int c = lane; c < rows * SF_BLOB_CHUNKS; c += 32) {
+      const int r = c / SF_BLOB_CHUNKS;
+      out[c] = tile[r * SF_BLOB_PITCH + (c - r * SF_BLOB_CHUNKS)];
+    }
+    __syncwarp();  // the tile is reused
+  }
+}
+
+// Rows with a bad header or target index are skipped and counted into *rejected (one atomic per warp). Writes only the
+// live missile and shell slots (the others are never read), and resets the env's render caches: a cached explosion is
+// keyed by the rand() calls consumed at the ship's spawn, which envs of equal seeds reach at different positions.
+__global__ void __launch_bounds__(32) sf_load_envs_kernel(SfDev D, int gametype, const int4* __restrict__ blob, const int* __restrict__ idx, int count,
+                                                          int* rejected) {
+  __shared__ int4 tile[32 * SF_BLOB_PITCH];
+  const int lane = threadIdx.x;
+  const size_t np = (size_t)D.n_pad;
+  const int4* row = tile + lane * SF_BLOB_PITCH;
+  const char* rb = reinterpret_cast<const char*>(row);
+  for (int base = blockIdx.x * 32; base < count; base += gridDim.x * 32) {
+    const int rows = min(32, count - base);
+    const int4* in = blob + (size_t)base * SF_BLOB_CHUNKS;
+#pragma unroll 4
+    for (int c = lane; c < rows * SF_BLOB_CHUNKS; c += 32) {
+      const int r = c / SF_BLOB_CHUNKS;
+      sf_cp_async(&tile[r * SF_BLOB_PITCH + (c - r * SF_BLOB_CHUNKS)], &in[c], 16);
+    }
+    sf_cp_async_wait();
+    __syncwarp();
+    const int k = base + lane;
+    const int i = k < count ? (idx ? idx[k] : k) : -1;
+    bool ok = false;
+    if (k < count) {
+      const int4 hd = row[0];
+      ok = (unsigned)hd.x == SF_ENV_BLOB_MAGIC && hd.y == SF_ENV_BLOB_VERSION && hd.z == gametype && i >= 0 && i < D.n;
+    }
+    const unsigned bad = __ballot_sync(0xFFFFFFFFu, k < count && !ok);
+    if (lane == 0 && bad && rejected) atomicAdd(rejected, __popc(bad));
+    if (ok) {
+      const int4 q0 = row[SF_BO_Q / 16];
+      const unsigned pm = (unsigned)q0.y;
+      D.pos[i] = *reinterpret_cast<const double2*>(rb + SF_BO_POS);
+      D.vel[i] = *reinterpret_cast<const double2*>(rb + SF_BO_VEL);
+      D.q0[i] = q0;
+      D.q1[i] = row[SF_BO_Q / 16 + 1];
+      D.q2[i] = row[SF_BO_Q / 16 + 2];
+      D.q3[i] = row[SF_BO_Q / 16 + 3];
+      D.st0[i] = row[SF_BO_ST / 16];
+      D.st1[i] = row[SF_BO_ST / 16 + 1];
+      D.st2[i] = row[SF_BO_ST / 16 + 2];
+      D.st3[i] = row[SF_BO_ST / 16 + 3];
+      const short* mang = reinterpret_cast<const short*>(rb + SF_BO_MANG);
+#pragma unroll
+      for (int s = 0; s < SF_MAX_MISSILES; s++) if ((pm >> s) & 1u) {
+        D.mpos[s * np + i] = *reinterpret_cast<const double2*>(rb + SF_BO_MPOS + 16 * s);
+        D.mang[s * np + i] = mang[s];
+      }
+#pragma unroll
+      for (int s = 0; s < SF_DEV_SHELLS; s++) if ((pm >> (SF_PMASK_SHELL_SHIFT + s)) & 1u) {
+        D.spos[s * np + i] = *reinterpret_cast<const double2*>(rb + SF_BO_SPOS + 16 * s);
+        D.svel[s * np + i] = *reinterpret_cast<const double2*>(rb + SF_BO_SVEL + 16 * s);
+        D.sang[s * np + i] = reinterpret_cast<const double*>(rb + SF_BO_SANG)[s];
+      }
+      const unsigned* rng = reinterpret_cast<const unsigned*>(rb + SF_BO_RNG);
+#pragma unroll
+      for (int w = 0; w < SF_RNG_WORDS; w++) D.rng[w * np + i] = rng[w];
+      D.expstamp[i] = 0;
+      D.expo_meta[i] = make_uint2(0u, 0u);
+    }
+    __syncwarp();  // the tile is reused
+  }
+}
+
 // ================================================================================================
 // C-ABI
 // ================================================================================================
@@ -741,6 +889,8 @@ extern "C" int sf_create(const char* gametype, int action_set, int n_envs, int d
   if ((ce = cudaFuncSetAttribute(sf_rollout_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK))) != cudaSuccess) return bail("shared memory opt-in (rollout, host delta)", ce);
   if ((ce = cudaFuncSetAttribute(sf_render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK))) != cudaSuccess) return bail("shared memory opt-in (render)", ce);
   if ((ce = cudaFuncSetAttribute(sf_pack_static_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK))) != cudaSuccess) return bail("shared memory opt-in (pack)", ce);
+  if ((ce = cudaFuncSetAttribute(sf_save_envs_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared)) != cudaSuccess) return bail("shared memory carveout (save envs)", ce);
+  if ((ce = cudaFuncSetAttribute(sf_load_envs_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared)) != cudaSuccess) return bail("shared memory carveout (load envs)", ce);
   sf_pack_static_kernel<<<1, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK)>>>(d, const_cast<unsigned char*>(d.static_image));
   if ((ce = cudaGetLastError()) != cudaSuccess) return bail("static image kernel launch", ce);
   // default seeding: every env replays srand(1) — the reference never seeds libc (game.cpp:137-148)
@@ -1239,6 +1389,32 @@ extern "C" int sf_set_state(sf_handle* h, int first, int count, const sf_state_r
   }
   cudaFree(d);
   if (ce != cudaSuccess) return fail(SF_ERR_CUDA, std::string("set_state: ") + cudaGetErrorString(ce));
+  return SF_OK;
+}
+
+static int blob_args(const sf_handle* h, const int32_t* d_env_idx, int count, const void* d_blob) {
+  if (!h || !d_blob) return fail(SF_ERR_INVALID, "handle or blob is NULL");
+  if (count < 0 || (!d_env_idx && count > h->dev.n)) return fail(SF_ERR_INVALID, "count out of range");
+  if ((uintptr_t)d_blob & 15) return fail(SF_ERR_INVALID, "the blob must be 16-byte aligned");
+  return SF_OK;
+}
+static int blob_blocks(const sf_handle* h, int count) { return std::min((count + 31) / 32, h->num_sms * SF_BLOB_BLOCKS_PER_SM); }
+
+extern "C" int sf_save_envs(sf_handle* h, const int32_t* d_env_idx, int count, uint8_t* d_blob, void* stream) {
+  if (int rc = blob_args(h, d_env_idx, count, d_blob)) return rc;
+  if (count == 0) return SF_OK;
+  CUDA_TRY(cudaSetDevice(h->device));
+  sf_save_envs_kernel<<<blob_blocks(h, count), 32, 0, (cudaStream_t)stream>>>(h->dev, h->gametype, d_env_idx, count, reinterpret_cast<int4*>(d_blob));
+  CUDA_TRY(cudaGetLastError());
+  return SF_OK;
+}
+
+extern "C" int sf_load_envs(sf_handle* h, const uint8_t* d_blob, const int32_t* d_env_idx, int count, int32_t* d_rejected, void* stream) {
+  if (int rc = blob_args(h, d_env_idx, count, d_blob)) return rc;
+  if (count == 0) return SF_OK;
+  CUDA_TRY(cudaSetDevice(h->device));
+  sf_load_envs_kernel<<<blob_blocks(h, count), 32, 0, (cudaStream_t)stream>>>(h->dev, h->gametype, reinterpret_cast<const int4*>(d_blob), d_env_idx, count, d_rejected);
+  CUDA_TRY(cudaGetLastError());
   return SF_OK;
 }
 

@@ -96,6 +96,18 @@ class SSF_Env(object):
         self.game_state = np.array([])
         return self._get_features(), reward, done, fort_kill
 
+    def clone_state(self):
+        """ALE-style snapshot of the game (Game.clone_state): a host uint8 array that restore_state takes back."""
+        return self.g.clone_state()
+
+    def restore_state(self, blob):
+        self.g.restore_state(blob)
+        if self.obs_type == "image":
+            self.game_state = self.g.gray_frame()
+            self.game_gray_rgb = np.repeat(self.game_state[..., None], 3, axis=2)
+        else:
+            self.game_state = np.array([])  # render() draws the restored frame
+
     def obs84(self):
         return self.g.obs84()
 

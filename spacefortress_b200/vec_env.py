@@ -325,6 +325,71 @@ class SFVecEnv(object):
         arr = records if isinstance(records, C.Array) else (_lib.StateRecord * count)(*records)
         _lib.check(self.L.sf_set_state(self.h, first, count, arr))
 
+    def _env_index(self, idx):
+        """idx (None, a sequence, a numpy array or a tensor of env indices) -> None or an int32 CUDA tensor on the env's
+        device. Host indices are range-checked here (SFError), device indices by the kernels: save_envs writes an all-zero
+        row for an index outside [0, num_envs), load_envs rejects the row."""
+        torch = _torch()
+        if idx is None:
+            return None
+        if isinstance(idx, torch.Tensor):
+            if idx.dtype.is_floating_point or idx.dtype == torch.bool:
+                raise TypeError("env indices must be integers")
+            return idx.to(device=self._device(), dtype=torch.int32).reshape(-1).contiguous()
+        arr = np.asarray(idx).reshape(-1)
+        if arr.size and not np.issubdtype(arr.dtype, np.integer):
+            raise TypeError("env indices must be integers")
+        if arr.size and (arr.min() < 0 or arr.max() >= self.num_envs):
+            raise _lib.SFError("env index out of range [0, %d)" % self.num_envs)
+        return torch.from_numpy(arr.astype(np.int32)).to(self._device())
+
+    def save_envs(self, idx=None, out=None):
+        """Complete game state of envs idx (None: all) as a uint8 CUDA tensor [k, ENV_BLOB_BYTES] on the env's device,
+        one canonical row per env (layout: SF_ENV_BLOB_BYTES in include/sf_b200.h). The result is an ordinary tensor:
+        index it, torch.save it, move it to another GPU. out: a contiguous uint8 tensor of that shape to write into."""
+        torch = _torch()
+        ix = self._env_index(idx)
+        k = self.num_envs if ix is None else ix.numel()
+        shape = (k, _lib.ENV_BLOB_BYTES)
+        if out is None:
+            out = torch.empty(shape, dtype=torch.uint8, device=self._device())
+        elif out.dtype != torch.uint8 or tuple(out.shape) != shape or out.device != self._device() or not out.is_contiguous():
+            raise ValueError("out must be a contiguous uint8 tensor of shape %r on %s" % (shape, self._device()))
+        _lib.check(self.L.sf_save_envs(self.h, C.c_void_p(ix.data_ptr()) if ix is not None else None, k,
+                                       C.c_void_p(out.data_ptr()), self._stream_ptr()))
+        return out
+
+    def load_envs(self, blob, idx=None, check=True):
+        """Env idx[k] <- row k of blob (rows from save_envs of a handle of the same game type, on any device; idx=None:
+        row i -> env i, which needs one row per env). Target indices must not repeat. The loaded envs continue exactly
+        where the saved ones were; the render caches are rebuilt on the next frame. check=True waits for the load and
+        raises SFError if any row had a bad header or target index (those rows are skipped either way)."""
+        torch = _torch()
+        dev = self._device()
+        if isinstance(blob, np.ndarray):
+            blob = torch.from_numpy(blob)
+        if blob.dtype != torch.uint8 or blob.dim() != 2 or blob.shape[1] != _lib.ENV_BLOB_BYTES:
+            raise ValueError("blob must be a uint8 tensor of shape [k, %d]" % _lib.ENV_BLOB_BYTES)
+        blob = blob.to(dev).contiguous()
+        k = blob.shape[0]
+        ix = self._env_index(idx)
+        if ix is None:
+            if k != self.num_envs:
+                raise ValueError("%d rows for %d envs: pass idx to load a subset" % (k, self.num_envs))
+        else:
+            if ix.numel() != k:
+                raise ValueError("%d rows for %d target indices" % (k, ix.numel()))
+            if torch.unique(ix).numel() != k:
+                raise ValueError("repeated target index")
+        rejected = torch.zeros(1, dtype=torch.int32, device=dev) if check else None
+        _lib.check(self.L.sf_load_envs(self.h, C.c_void_p(blob.data_ptr()), C.c_void_p(ix.data_ptr()) if ix is not None else None, k,
+                                       C.c_void_p(rejected.data_ptr()) if check else None, self._stream_ptr()))
+        if check:
+            bad = int(rejected.item())
+            if bad:
+                raise _lib.SFError("load_envs: %d of %d rows rejected (bad magic, version or game type, or target index out of "
+                                   "range); the other rows were loaded" % (bad, k))
+
     def episode_stats(self, reset=True, all_reduce=True):
         """Finished-episode statistics since the last reset of the accumulators, summed over all ranks when
         torch.distributed is initialised (one small all-reduce per rollout; replaces rl/train.py:81-88)."""
