@@ -224,19 +224,21 @@ __device__ __noinline__ void sf_step_group(const SfDev& D, const SfRollArgs& A, 
 // The two roles of the rollout kernel, out of line (separate register allocations, see sf_stepper_ticks). Both walk the
 // same sequence of groups: the block's first group is blockIdx.x, further ones are handed out first come first served
 // (the groups differ in cost, and so do the SMs' speeds). Warp 0 fetches the id of the NEXT group when it starts a group
-// and leaves it in shared memory (two slots, alternating); the other warps read it when they are done with the current
-// group, many barriers later. The step of tick t + 1 (warp 0) runs while the other warps draw tick t, across groups too.
+// and leaves it in shared memory (a ring indexed by the group count, SF_NEXT_GROUPS); the other warps read it when they
+// are done with the current group, many barriers later. The steps of the next ticks (warp 0) run while the other warps
+// draw the ticks before them, across groups too.
 __device__ __noinline__ void sf_rollout_stepper(const SfDev& D, const SfRollArgs& A) {
   const int lane = threadIdx.x & 31;
   SfBlockSmem& B = sf_block_smem();
   const bool native = (A.flags & SF_FLAG_NATIVE_OBS) != 0;
   int stage = 0, group = blockIdx.x;
 #pragma unroll 1
-  for (int k = 1; group < A.ngroups; k ^= 1) {
+  for (int k = 0; group < A.ngroups; k = (k + 1) % SF_NEXT_GROUPS) {
     if (lane == 0) B.next_group[k] = A.sched ? (int)gridDim.x + atomicAdd(&A.sched->next_group, 1) : group + (int)gridDim.x;
-    sf_stepper_ticks(D, B, lane, native, A.T, stage, [&](int t, SfTeamSmem& Tm, int h) { sf_step_group(D, A, group, t, &Tm.env[32 * h]); });
+    sf_stepper_ticks(D, B, lane, native, A.T, stage, [&](int t, SfStagePrep& Tm, int h) { sf_step_group(D, A, group, t, &Tm.env[32 * h]); });
     group = B.next_group[k];
   }
+  sf_stepper_drain(stage);
   // the last block to leave re-arms the counters for the next launch (every block has made its last fetch by then)
   if (lane == 0 && A.sched) {
     __threadfence();
@@ -256,7 +258,7 @@ __device__ __forceinline__ void sf_rollout_drawer(const SfDev& D, const SfRollAr
   st.stage = 0; st.prev_used = 0;
   int group = blockIdx.x;
 #pragma unroll 1
-  for (int k = 1; group < A.ngroups; k ^= 1) {
+  for (int k = 0; group < A.ngroups; k = (k + 1) % SF_NEXT_GROUPS) {
     sf_drawer_ticks(D, B, W, lane, out, A.T, st);
     group = B.next_group[k];
   }
@@ -363,7 +365,7 @@ __global__ void __launch_bounds__(SF_BLOCK, SF_BLOCKS_PER_SM) sf_render_kernel(S
     int stage = 0;
 #pragma unroll 1
     for (int group = blockIdx.x; group < ngroups; group += gridDim.x)
-      sf_stepper_ticks(D, B, lane, native, 1, stage, [&](int, SfTeamSmem& Tm, int) {
+      sf_stepper_ticks(D, B, lane, native, 1, stage, [&](int, SfStagePrep& Tm, int) {
         const int env = group * EB + lane;
         const bool mine = lane < EB && env < D.n && (!mask || mask[env]);
         if (mine) {
@@ -373,6 +375,7 @@ __global__ void __launch_bounds__(SF_BLOCK, SF_BLOCKS_PER_SM) sf_render_kernel(S
         } else Tm.env[lane].env = -1;
         __syncwarp();
       });
+    sf_stepper_drain(stage);
   } else {
     SfFrameOut out;
     out.native = native ? 1 : 0;

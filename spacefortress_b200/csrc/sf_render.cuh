@@ -106,22 +106,39 @@ __device__ __forceinline__ unsigned sf_expo_key(const SfEnvRec& r) {
   const int bst = r.kill_bar ? 11 : min(r.vuln, 10);
   return (unsigned)fst | ((unsigned)bst << 6) | (((unsigned)r.points_i & 0x3FFFFu) << 10);
 }
-// one moving wireframe of the round: desc = kind | angle<<2 | env slot<<12; region = index into the block's list, -1: none
-struct __align__(8) SfStrokeRec { double x, y; int desc, region; };
+// one moving wireframe of the round: desc = kind | angle<<2 | env slot<<12 (its region is in SfStagePool::stroke_region)
+struct __align__(8) SfStrokeRec { double x, y; int desc; };
 
-// One STAGE = one round of one tick of the block's group of envs: the records, the round's stroke list and control
-// values (written by the stepping warp while the previous stage is drawn) and the pools the drawing warps fill.
-// Two copies: stage s is drawn from copy s & 1 while warp 0 prepares stage s + 1 in the other one.
-struct __align__(16) SfTeamSmem {
+// One STAGE = one round of up to SF_STAGE_TICKS ticks of the block's group of envs. What it needs is split by writer:
+//  * SfStagePrep: the records, the round's stroke list and control values, written by the stepping warp before the stage
+//    is handed to the drawing warps and only read after that. A ring of SF_PREP_SLOTS: stage s is prepared in slot
+//    s % SF_PREP_SLOTS, so warp 0 can be up to SF_PREP_SLOTS - 1 stages ahead of the stage being drawn.
+//  * SfStagePool: what the drawing warps write while they draw a stage (regions, coverage cells, explosion build
+//    scratch, work counters). One copy: stages are drawn one after the other.
+#ifndef SF_PREP_SLOTS
+#define SF_PREP_SLOTS 3   // 2: warp 0 prepares stage s + 1 while stage s is drawn; 3: up to s + 2
+#endif
+static_assert(SF_PREP_SLOTS >= 2 && SF_PREP_SLOTS <= 6, "named barriers 3 .. 3 + 2 * SF_PREP_SLOTS - 1 must exist (16 per block)");
+// Ring of the block's next group ids (rollout kernel), indexed by the block's group count. Warp 0 writes the entry of
+// group j when it starts preparing j; the drawing warps read the entry of group g after their last stage of g. Warp 0 can
+// only have passed the wait for stage s - 1 - SF_PREP_SLOTS when it starts group j at stage s, so the readers of the groups
+// from j - 1 - SF_PREP_SLOTS on may still be pending: the ring needs more than SF_PREP_SLOTS + 1 entries.
+#define SF_NEXT_GROUPS 8
+static_assert(SF_PREP_SLOTS + 2 <= SF_NEXT_GROUPS, "next-group ring too small for the lead of the stepping warp");
+struct __align__(16) SfStagePrep {
   SfEnvRec env[SF_STAGE_SLOTS];
   SfStrokeRec stroke[SF_ROUND_STROKES];
-  int4 region[SF_POOL_REGIONS];      // {x0, y0, w | h<<16, first cell | tag<<15 | colour<<16}
   int r0, r1, nstrokes, build_env;   // the current round: env slots [r0, r1), strokes in the list, the env slot whose explosion is built (-1)
-  int next_task, netask, next_patch, chunk;  // phase C work queue; env tasks of the round; base patches handed out; strokes per batch of phase B1
-  int more, nticks, build_env2, base_ready;  // env slots of the stage are left for another round; ticks the stage covers (1 .. SF_STAGE_TICKS);
-                                             // the round's bulk copies have landed (set by the warp that issued them)
-  int nregions, cells_used, dbg_max_b, dbg_max_c;
+  int netask, chunk, more, nticks;   // env tasks of the round; strokes per batch of phase B1; env slots of the stage are left for
+                                     // another round; ticks the stage covers (1 .. SF_STAGE_TICKS)
+  int build_env2, padp[3];
   unsigned short etask[SF_STAGE_SLOTS * 5];  // env slot | kind<<6: kind 0..3 = quarter of a dead ship's explosion box, 4 = score strip
+};
+struct __align__(16) SfStagePool {
+  int4 region[SF_POOL_REGIONS];      // {x0, y0, w | h<<16, first cell | tag<<15 | colour<<16}
+  short stroke_region[SF_ROUND_STROKES];  // region of stroke k of the round's list, -1: none
+  int next_task, next_patch, nregions, cells_used;  // phase C work queue; base patches handed out; regions / cells opened
+  int base_ready, dbg_max_b, dbg_max_c, padq;       // the round's bulk copies have landed (set by the warp that issued them)
   unsigned short exp_item0[SF_EXP_QUADS];   // build: copies of the y phase's per-quad table entries (SfExpPhase) for the sprite pass
   short exp_qxmin[SF_EXP_QUADS];
   signed char exp_row0[SF_EXP_QUADS];
@@ -162,9 +179,10 @@ struct __align__(16) SfBlockSmem {
 #ifdef SF_TIMELINE
   int tl_n[4];
 #endif
-  int next_group[2], padg[2];  // rollout kernel: the block's next groups (written by warp 0 one group ahead)
+  int next_group[SF_NEXT_GROUPS];  // rollout kernel: the block's next groups (written by warp 0 ahead of the drawing warps)
   SfStepSmem step;             // rollout kernel: the group's scalar state between ticks
-  SfTeamSmem team[2];
+  SfStagePrep prep[SF_PREP_SLOTS];
+  SfStagePool pool;
 };
 
 // Everything above `init_mbar` is static (a function of the tables only). sf_pack_static_kernel builds it once per
@@ -177,18 +195,46 @@ struct __align__(16) SfBlockSmem {
 // Helpers that are kept out of line re-derive their slots from it, so the compiler still knows the address space.
 extern __shared__ __align__(16) unsigned char sf_smem_raw[];
 __device__ __forceinline__ SfBlockSmem& sf_block_smem() { return *reinterpret_cast<SfBlockSmem*>(sf_smem_raw); }
-__device__ __forceinline__ SfTeamSmem& sf_team(int sg) { return sf_block_smem().team[sg]; }  // sg: the stage copy being drawn (0 / 1), handed down in a register
+__device__ __forceinline__ SfStagePrep& sf_prep(int sg) { return sf_block_smem().prep[sg]; }  // sg: the ring slot of the stage being drawn, handed down in a register
+__device__ __forceinline__ SfStagePool& sf_pool() { return sf_block_smem().pool; }
 #ifdef SF_BARRIER_TIMING  // tools/gpu_barrier_timing.py: cycles the warps spend at the barriers
-__device__ unsigned long long sf_bar_cycles[16];  // [8..15]: sections of the step (SF_ST in sf_step.cuh / sf_step_group); [0] stage barrier (drawing warps), [1] drawing-warp barriers, [2] stage barrier (warp 0)
+__device__ unsigned long long sf_bar_cycles[16];  // [8..15]: sections of the step (SF_ST in sf_step.cuh / sf_step_group); [0] wait for a prepared stage (drawing warps), [1] drawing-warp barriers, [2] wait for a free ring slot (warp 0)
 __device__ __forceinline__ void sf_bar_add(int k, long long t0) { if ((threadIdx.x & 31) == 0) atomicAdd(&sf_bar_cycles[k], (unsigned long long)(clock64() - t0)); }
 #endif
-__device__ __forceinline__ void sf_team_sync() {  // every warp of the block (named barrier 1)
+// Hand-over of ring slot i between the two roles: two named hardware barriers of 768 threads each, full[i] = 3 + i and
+// empty[i] = 3 + SF_PREP_SLOTS + i (bar 0: __syncthreads, bar 2: the drawing warps).
+//  * full[i]: warp 0 ARRIVES when it has written the stage into slot i; the 23 drawing warps SYNC on it before they read it.
+//  * empty[i]: the drawing warps ARRIVE when they have drawn the stage in slot i; warp 0 SYNCS on it before it rewrites it.
+// Memory ordering (PTX memory model, CTA scope): bar.arrive is a release of everything the arriving thread wrote or read
+// before it, and bar.sync is an acquire of what the threads that arrived at the same barrier instance released. So the
+// records warp 0 wrote are visible to every drawing warp that returns from full[i], and every read of the slot by a
+// drawing warp is done before warp 0 returns from empty[i] and overwrites it. Nobody polls: a warp that waits sleeps in
+// the barrier. A barrier instance is reused only after it completed: warp 0 arrives at full[i] again (stage s + N) only
+// after its sync on empty[i], which needs the drawing warps' arrival after stage s, which followed their sync on full[i]
+// for stage s; the same chain orders two uses of empty[i]. Since the drawing warps draw the stages in order and all of
+// them sync on full[i], that barrier also separates the pool use of one stage from the next (see sf_drawer_ticks).
+__device__ __forceinline__ void sf_stage_full_arrive(int sg) {  // warp 0
+  asm volatile("bar.arrive %0, %1;" :: "r"(3 + sg), "r"(32 * SF_RENDER_WARPS) : "memory");
+}
+__device__ __forceinline__ void sf_stage_full_wait(int sg) {  // drawing warps
 #ifdef SF_BARRIER_TIMING
   const long long t0 = clock64();
 #endif
-  asm volatile("bar.sync 1, %0;" :: "r"(32 * SF_RENDER_WARPS) : "memory");
+  asm volatile("bar.sync %0, %1;" :: "r"(3 + sg), "r"(32 * SF_RENDER_WARPS) : "memory");
 #ifdef SF_BARRIER_TIMING
-  sf_bar_add(threadIdx.x < 32 ? 2 : 0, t0);
+  sf_bar_add(0, t0);
+#endif
+}
+__device__ __forceinline__ void sf_stage_empty_arrive(int sg) {  // drawing warps
+  asm volatile("bar.arrive %0, %1;" :: "r"(3 + SF_PREP_SLOTS + sg), "r"(32 * SF_RENDER_WARPS) : "memory");
+}
+__device__ __forceinline__ void sf_stage_empty_wait(int sg) {  // warp 0
+#ifdef SF_BARRIER_TIMING
+  const long long t0 = clock64();
+#endif
+  asm volatile("bar.sync %0, %1;" :: "r"(3 + SF_PREP_SLOTS + sg), "r"(32 * SF_RENDER_WARPS) : "memory");
+#ifdef SF_BARRIER_TIMING
+  sf_bar_add(2, t0);
 #endif
 }
 __device__ __forceinline__ void sf_render_sync() {  // the warps that draw: all but warp 0, which steps (named barrier 2)
@@ -305,14 +351,11 @@ __device__ __forceinline__ void sf_block_smem_init(const unsigned char* image) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
                  :: "r"((unsigned)__cvta_generic_to_shared(&B)), "l"(image), "r"((unsigned)SF_STATIC_BYTES), "r"(bar) : "memory");
   }
-  for (int c = 0; c < 2; c++) {
-    for (int k = threadIdx.x; k < SF_POOL_CELLS / 2; k += blockDim.x) reinterpret_cast<unsigned*>(B.team[c].cells)[k] = 0u;
-    for (int k = threadIdx.x; k < SF_EXP_W * SF_EXP_W * 4; k += blockDim.x) (&B.team[c].arc_mask[0][0])[k] = 0u;
-    if (threadIdx.x == 32) {
-      SfTeamSmem& Tm = B.team[c];
-      Tm.next_task = 0; Tm.next_patch = 0; Tm.netask = 0; Tm.chunk = 8; Tm.nregions = 0; Tm.cells_used = 0;
-    }
-  }
+  for (int k = threadIdx.x; k < SF_POOL_CELLS / 2; k += blockDim.x) reinterpret_cast<unsigned*>(B.pool.cells)[k] = 0u;
+  for (int k = threadIdx.x; k < SF_EXP_W * SF_EXP_W * 4; k += blockDim.x) (&B.pool.arc_mask[0][0])[k] = 0u;
+  if (threadIdx.x == 32) { B.pool.next_task = 0; B.pool.next_patch = 0; B.pool.nregions = 0; B.pool.cells_used = 0; B.pool.base_ready = 0; }
+  // no env in the ring yet (sf_publish_recs compares a new record with the ones of the rounds before it)
+  for (int k = threadIdx.x; k < SF_PREP_SLOTS * SF_STAGE_SLOTS; k += blockDim.x) B.prep[k / SF_STAGE_SLOTS].env[k % SF_STAGE_SLOTS].env = -1;
   // the bulk-copy engine (async proxy) reads bg_obs: make generic-proxy writes visible to it
   asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
   __syncthreads();   // (also: the mbarrier is initialised before anybody polls it)
@@ -427,8 +470,8 @@ __device__ __forceinline__ int sf_row_of(int g) { return (g >= 0) ? g / SF_GRID_
 // Append one region per participating lane (`want`) to the block's list, in lane order: region ids and coverage
 // cells come from the block-wide pools (one atomic per batch each). Returns the lane's region id, or -1 when the
 // stroke is off the surface (or a pool is full: cannot happen, the round scan admits envs by worst-case need).
-__device__ __forceinline__ int sf_open_regions(int lane, bool want, int ymin_g, int ymax_g, int xmin, int xmax, unsigned colour, int tag, int sg) {
-  SfTeamSmem& Tm = sf_team(sg);
+__device__ __forceinline__ int sf_open_regions(int lane, bool want, int ymin_g, int ymax_g, int xmin, int xmax, unsigned colour, int tag) {
+  SfStagePool& Tm = sf_pool();
   int cx0 = 0, py0 = 0, w = 0, h = 0;
   bool ok = want && ymin_g < ymax_g;
   if (ok) {
@@ -457,8 +500,8 @@ __device__ __forceinline__ int sf_open_regions(int lane, bool want, int ymin_g, 
 // the region of its stroke; the first lane of every stroke slot (`head`: nq consecutive lanes starting here hold the
 // quads of the stroke, [s0, s1) = union of their live sub-rows) stores the stroke record and appends the stroke's
 // work groups of 8 consecutive sub-rows. rid = the stroke's region (-1: none).
-__device__ __forceinline__ void sf_publish_quads(SfWarpSmem& W, int lane, const SfQuadGeom& G, bool has, int rid, bool head, int slot, int nq, int ymin_g, int ymax_g, int sg) {
-  const SfTeamSmem& Tm = sf_team(sg);
+__device__ __forceinline__ void sf_publish_quads(SfWarpSmem& W, int lane, const SfQuadGeom& G, bool has, int rid, bool head, int slot, int nq, int ymin_g, int ymax_g) {
+  const SfStagePool& Tm = sf_pool();
   int len = 0;
   int4 R = make_int4(0, 0, 0, 0);
   if (rid >= 0) R = Tm.region[rid];
@@ -520,11 +563,11 @@ __device__ __forceinline__ void sf_emit_span_pred(unsigned* acc32, int cell0, in
 // One pass (4 work groups = 32 (stroke, sub-row) items) of the batch that warp `owner` published, starting at its
 // work group g0. Any warp of the block can run any pass: the records are read-only after the block barrier that
 // follows the geometry, and the cells are updated with atomics.
-__device__ __noinline__ void sf_accumulate_pass(int owner, int g0, int sg) {
+__device__ __noinline__ void sf_accumulate_pass(int owner, int g0) {
   const SfWarpSmem& W = sf_warp_smem(owner);
   const int lane = threadIdx.x & 31;
   const int ngroups = W.ngroups;
-  unsigned* acc32 = reinterpret_cast<unsigned*>(sf_team(sg).cells);
+  unsigned* acc32 = reinterpret_cast<unsigned*>(sf_pool().cells);
   const int gi = min(g0 + (lane >> 3), ngroups - 1);
   const int ent = W.glist[gi];
   const int4 S = W.srec[ent & 31];
@@ -569,9 +612,9 @@ __device__ __forceinline__ void sf_patch_init(SfWarpSmem& W, const SfTables* T, 
 }
 
 // Blend region `rid` of the round (its coverage cells) into this warp's window (clipped to it).
-__device__ __noinline__ void sf_blend_region(int rid, int win, int sg) {
+__device__ __noinline__ void sf_blend_region(int rid, int win) {
   SfWarpSmem& W = sf_my_smem();
-  const SfTeamSmem& O = sf_team(sg);
+  const SfStagePool& O = sf_pool();
   const int lane = threadIdx.x & 31;
   const int4 R = O.region[rid];
   const int w = R.z & 0xFFFF, h = (R.z >> 16) & 0xFFFF;
@@ -597,7 +640,7 @@ __device__ __noinline__ void sf_blend_region(int rid, int win, int sg) {
 __device__ __noinline__ bool sf_composite(const SfTables* T, unsigned char* expcache, int e, int win, int sg) {
   SfWarpSmem& W = sf_my_smem();
   const SfBlockSmem& B = sf_block_smem();
-  const SfEnvRec& rec = sf_team(sg).env[e];
+  const SfEnvRec& rec = sf_prep(sg).env[e];
   const int lane = threadIdx.x & 31;
   const unsigned core = rec.core;
   const int nx0 = SF_WIN_X0(win), ny0 = SF_WIN_Y0(win);
@@ -609,9 +652,9 @@ __device__ __noinline__ bool sf_composite(const SfTables* T, unsigned char* expc
   int sr = -1, tag = SF_TAG_PROJECTILE;
   bool hit = false;
   if (lane < rec.ns) {
-    sr = sf_team(sg).stroke[rec.s0 + lane].region;
+    sr = sf_pool().stroke_region[rec.s0 + lane];
     if (sr >= 0) {
-      const int4 R = sf_team(sg).region[sr];
+      const int4 R = sf_pool().region[sr];
       hit = R.x < nx1 && R.x + (R.z & 0xFFFF) > nx0 && R.y < ny1 && R.y + ((R.z >> 16) & 0xFFFF) > ny0;
       tag = (R.w >> 15) & 1;
     }
@@ -622,7 +665,7 @@ __device__ __noinline__ bool sf_composite(const SfTables* T, unsigned char* expc
   SF_PROF(23);
   // ---- ship wireframe | ship explosion (draw.cpp:233-237) ----
   if (core & SF_CORE_SHIP_ALIVE) {
-    if ((rmask & 1u) && first_is_ship) { const int s0r = __shfl_sync(0xffffffffu, sr, 0); sf_blend_region(s0r, win, sg); rmask &= ~1u; }
+    if ((rmask & 1u) && first_is_ship) { const int s0r = __shfl_sync(0xffffffffu, sr, 0); sf_blend_region(s0r, win); rmask &= ~1u; }
   } else {
     const int ebox = rec.ebox;
     const int bx0 = (ebox & 255) - 64, by0 = ((ebox >> 8) & 255) - 64;
@@ -700,7 +743,7 @@ __device__ __noinline__ bool sf_composite(const SfTables* T, unsigned char* expc
     const int q = __ffs(rmask) - 1;
     rmask &= rmask - 1;
     const int sq = __shfl_sync(0xffffffffu, sr, q);
-    sf_blend_region(sq, win, sg);
+    sf_blend_region(sq, win);
   }
   SF_PROF(26);
   // ---- score digits (draw.cpp:160-173,267): "%07d" of (int)mPoints ----
@@ -795,7 +838,7 @@ __device__ __forceinline__ bool sf_window_orect(const SfTables* T, unsigned char
 // Geometry for up to 8 strokes at once: lane = 4*slot + line. kind: 0 ship, 1 missile, 2 shell, -1 none.
 // Every lane passes the description of ITS slot's stroke. Appends one region per visible stroke and publishes the
 // quads. Returns the region of the lane's slot (-1 invisible).
-__device__ __forceinline__ int sf_wire_geometry(SfWarpSmem& W, int lane, const SfTables* T, int kind, double px, double py, int angle, int sg) {
+__device__ __forceinline__ int sf_wire_geometry(SfWarpSmem& W, int lane, const SfTables* T, int kind, double px, double py, int angle) {
   SF_PROF(31);
   const int slot = lane >> 2, line = lane & 3;
   SfQuadGeom G;
@@ -827,10 +870,10 @@ __device__ __forceinline__ int sf_wire_geometry(SfWarpSmem& W, int lane, const S
   }
   SF_PROF(16);
   // one region per slot, opened in slot order by the slot's first lane
-  int rid = sf_open_regions(lane, line == 0 && kind >= 0, ymin_g, ymax_g, xmin, xmax, sf_block_smem().colour_white, kind == 0 ? SF_TAG_SHIP : SF_TAG_PROJECTILE, sg);
+  int rid = sf_open_regions(lane, line == 0 && kind >= 0, ymin_g, ymax_g, xmin, xmax, sf_block_smem().colour_white, kind == 0 ? SF_TAG_SHIP : SF_TAG_PROJECTILE);
   SF_PROF(17);
   rid = __shfl_sync(0xffffffffu, rid, lane & ~3);
-  sf_publish_quads(W, lane, G, has, rid, line == 0 && kind >= 0, slot, kind >= 0 ? sf_block_smem().wf_nlines[kind] : 0, ymin_g, ymax_g, sg);
+  sf_publish_quads(W, lane, G, has, rid, line == 0 && kind >= 0, slot, kind >= 0 ? sf_block_smem().wf_nlines[kind] : 0, ymin_g, ymax_g);
   SF_PROF(18);
   return rid;
 }
@@ -841,8 +884,8 @@ __device__ __forceinline__ int sf_wire_geometry(SfWarpSmem& W, int lane, const S
 // spans of the item, shifted by the centre's x, into the item's <= SF_EXPT_NC cells (registers: nobody else adds to
 // them) and tells every pixel it covers which quad did. wi / nw: this warp's index among the drawing warps.
 __device__ __forceinline__ void sf_phase_exp_items(const SfDev& D, int be, int lane, int wi, int nw, int sg) {
-  SfTeamSmem& Tm = sf_team(sg);
-  const SfEnvRec& rec = Tm.env[be];
+  SfStagePool& Tm = sf_pool();
+  const SfEnvRec& rec = sf_prep(sg).env[be];
   const SfPt c = sf_xform_base(rec.px, rec.py);
   const SfExpPhase& P = D.tab->exp_phase[c.y & 255];
   const int Y = c.y >> 8, bx0 = (c.x >> 8) - 13, by0 = Y - 13;  // the explosion box (sf_make_env_rec)
@@ -882,9 +925,9 @@ __device__ __forceinline__ void sf_phase_exp_items(const SfDev& D, int be, int l
 // are ONE stroke: their lengths add up), over the background (hexagons) and stores the sprite in the env's cache;
 // the windows of phase C read it like any cached sprite. wi / nw: this warp's index among the drawing warps.
 __device__ __forceinline__ void sf_phase_sprite(const SfDev& D, SfBlockSmem& B, int be, int lane, int wi, int nw, int sg) {
-  SfTeamSmem& Tm = sf_team(sg);
+  SfStagePool& Tm = sf_pool();
   const SfTables* T = D.tab;
-  SfEnvRec& rec = Tm.env[be];
+  const SfEnvRec& rec = sf_prep(sg).env[be];
   const SfPt c = sf_xform_base(rec.px, rec.py);
   const SfExpPhase& P = T->exp_phase[c.y & 255];
   const int Y = c.y >> 8, bx0 = (c.x >> 8) - 13, by0 = Y - 13;
@@ -973,7 +1016,7 @@ __device__ __forceinline__ void sf_scan_begin(SfScanState& S) {
   S.closed = false; S.later_any = 0u;
 }
 // slots 32h .. 32h + 31 (tick h of the stage); r_begin: first slot that still has to be drawn
-__device__ __forceinline__ void sf_scan_half(SfTeamSmem& Tm, int lane, int h, int r_begin, SfScanState& S) {
+__device__ __forceinline__ void sf_scan_half(SfStagePrep& Tm, int lane, int h, int r_begin, SfScanState& S) {
   if (!S.closed) S.r1 = 32 * (h + 1);
   const int slot = 32 * h + lane;
   SfEnvRec& rec = Tm.env[slot];
@@ -1019,13 +1062,12 @@ __device__ __forceinline__ void sf_scan_half(SfTeamSmem& Tm, int lane, int h, in
   if (inr) S.carry_task += __shfl_sync(0xffffffffu, inclt_all, 31 - __clz((int)inr));
   S.carry_cnt = __shfl_sync(0xffffffffu, incl, 31); S.carry_need = __shfl_sync(0xffffffffu, incl_need, 31);
 }
-__device__ __forceinline__ void sf_scan_finish(SfTeamSmem& Tm, int lane, int r_begin, const SfScanState& S) {
+__device__ __forceinline__ void sf_scan_finish(SfStagePrep& Tm, int lane, int r_begin, const SfScanState& S) {
   if (lane == 0) {
     Tm.more = S.later_any != 0u;
     Tm.r0 = r_begin; Tm.r1 = S.r1; Tm.nstrokes = S.nst;
     Tm.build_env = (S.build_env >= 0 && S.build_env < S.r1) ? S.build_env : -1;
     Tm.build_env2 = (Tm.build_env >= 0 && S.build_env2 >= 0 && S.build_env2 < S.r1) ? S.build_env2 : -1;
-    Tm.base_ready = 0;
     // phase B1 hands the strokes out in equal batches of <= 8, one per drawing warp
     // (the last drawing warps get no batch: one of them issues the round's bulk copies instead, see sf_draw_stage)
 #ifndef SF_CHUNK_WARPS  // B1 is latency bound (a batch of 8 strokes takes as long as one of 4), and every batch rounds its last pass of B3 up:
@@ -1037,7 +1079,7 @@ __device__ __forceinline__ void sf_scan_finish(SfTeamSmem& Tm, int lane, int r_b
   __syncwarp();
 }
 // the whole scan at once (a later round of a stage: slots r_begin .. nslots - 1)
-__device__ __forceinline__ void sf_round_scan(SfTeamSmem& Tm, int lane, int r_begin, int nslots) {
+__device__ __forceinline__ void sf_round_scan(SfStagePrep& Tm, int lane, int r_begin, int nslots) {
   SfScanState S;
   sf_scan_begin(S);
 #pragma unroll
@@ -1050,7 +1092,7 @@ __device__ __forceinline__ void sf_round_scan(SfTeamSmem& Tm, int lane, int r_be
 // out as ONE asynchronous bulk copy from the block's shared-memory copy (TMA engine, 7056 bytes; one copy per lane of
 // the issuing warp, see sf_draw_stage)...
 __device__ __forceinline__ void sf_env_base_issue(const SfBlockSmem& B, int e, const SfFrameOut& out, int sg) {
-  const int env = sf_team(sg).env[e].env;
+  const int env = sf_prep(sg).env[e].env;
   if (env < 0) return;
   const unsigned src = (unsigned)__cvta_generic_to_shared(B.bg_obs);
   unsigned char* gb = sf_frame_ptr(out, e, env);
@@ -1062,7 +1104,7 @@ __device__ __forceinline__ void sf_env_base_issue(const SfBlockSmem& B, int e, c
 // pre-resampled state tables.
 __device__ __forceinline__ void sf_env_base_patch(const SfDev& D, const SfBlockSmem& B, int lane, int e, const SfFrameOut& out, int sg) {
   const SfTables* T = D.tab;
-  const SfEnvRec& rec = sf_team(sg).env[e];
+  const SfEnvRec& rec = sf_prep(sg).env[e];
   const int env = rec.env;
   if (env < 0) return;
   const unsigned core = rec.core;
@@ -1139,14 +1181,14 @@ __device__ __forceinline__ void sf_env_base_patch(const SfDev& D, const SfBlockS
 // Stepping warp, after the round scan of the stage it prepares: the strokes of the round's slots of tick `h` of the
 // stage, one env per lane, from the SoA state (which holds exactly that tick): [ship] + live missiles (slot order) +
 // visible shells (slot order) == draw order.
-__device__ __forceinline__ void sf_gather_strokes(const SfDev& D, SfTeamSmem& Tm, int lane, int h) {
+__device__ __forceinline__ void sf_gather_strokes(const SfDev& D, SfStagePrep& Tm, int lane, int h) {
   const int slot = 32 * h + lane;
   const SfEnvRec& rec = Tm.env[slot];
   if (slot >= Tm.r0 && slot < Tm.r1 && rec.env >= 0) {
     const int env = rec.env, np = D.n_pad;
     const unsigned core = rec.core;
     SfStrokeRec* S = &Tm.stroke[rec.s0];
-    if (core & SF_CORE_SHIP_ALIVE) { S->x = rec.px; S->y = rec.py; S->desc = 0 | ((int)(core & SF_CORE_ANGLE_MASK) << 2) | (slot << 12); S->region = -1; S++; }
+    if (core & SF_CORE_SHIP_ALIVE) { S->x = rec.px; S->y = rec.py; S->desc = 0 | ((int)(core & SF_CORE_ANGLE_MASK) << 2) | (slot << 12); S++; }
     // (up to three missiles per trip: the loads of a trip are in flight together — each is an L2 round trip for this one
     // warp. Plain scalars: indexed arrays end up in local memory here)
     for (unsigned m = rec.pmask & SF_PMASK_MISSILES; m;) {
@@ -1155,16 +1197,16 @@ __device__ __forceinline__ void sf_gather_strokes(const SfDev& D, SfTeamSmem& Tm
       const int k2 = m ? __ffs(m) - 1 : k0; m &= m - 1;
       const double2 p0 = D.mpos[(size_t)k0 * np + env], p1 = D.mpos[(size_t)k1 * np + env], p2 = D.mpos[(size_t)k2 * np + env];
       const int a0 = D.mang[(size_t)k0 * np + env], a1 = D.mang[(size_t)k1 * np + env], a2 = D.mang[(size_t)k2 * np + env];
-      S->x = p0.x; S->y = p0.y; S->desc = 1 | (a0 << 2) | (slot << 12); S->region = -1; S++;
-      if (k1 != k0) { S->x = p1.x; S->y = p1.y; S->desc = 1 | (a1 << 2) | (slot << 12); S->region = -1; S++; }
-      if (k2 != k0) { S->x = p2.x; S->y = p2.y; S->desc = 1 | (a2 << 2) | (slot << 12); S->region = -1; S++; }
+      S->x = p0.x; S->y = p0.y; S->desc = 1 | (a0 << 2) | (slot << 12); S++;
+      if (k1 != k0) { S->x = p1.x; S->y = p1.y; S->desc = 1 | (a1 << 2) | (slot << 12); S++; }
+      if (k2 != k0) { S->x = p2.x; S->y = p2.y; S->desc = 1 | (a2 << 2) | (slot << 12); S++; }
     }
     for (unsigned m = (unsigned)rec.shell_vis; m; m &= m - 1) {
       const int k = __ffs(m) - 1;
       const double2 p = D.spos[(size_t)k * np + env];
       int angle = __double2int_rz(D.sang[(size_t)k * np + env]);  // `int angle` truncation, quirk Q10
       if (angle >= 360) angle -= 360;
-      S->x = p.x; S->y = p.y; S->desc = 2 | (angle << 2) | (slot << 12); S->region = -1; S++;
+      S->x = p.x; S->y = p.y; S->desc = 2 | (angle << 2) | (slot << 12); S++;
     }
   }
   __syncwarp();
@@ -1176,7 +1218,7 @@ __device__ __forceinline__ void sf_gather_strokes(const SfDev& D, SfTeamSmem& Tm
 // the size of the individual strokes.
 __device__ __forceinline__ void sf_phase_strokes(const SfDev& D, SfBlockSmem& B, SfWarpSmem& W, int lane, int wi, int nw, int nst, int sg) {
   const SfTables* T = D.tab;
-  SfTeamSmem& Tm = sf_team(sg);
+  const SfStagePrep& Tm = sf_prep(sg);
   const int chunk = Tm.chunk;
   // B2, first half: the items of the explosion of a ship that died in this stage. They are dealt from the LAST
   // drawing warp down: the geometry batches go to the first warps, so the two overlap.
@@ -1195,8 +1237,8 @@ __device__ __forceinline__ void sf_phase_strokes(const SfDev& D, SfBlockSmem& B,
       const SfStrokeRec& S = Tm.stroke[idx];
       x = S.x; y = S.y; kind = S.desc & 3; angle = (S.desc >> 2) & 1023;
     }
-    const int rid = sf_wire_geometry(W, lane, T, kind, x, y, angle, sg);
-    if (valid && (lane & 3) == 0) Tm.stroke[idx].region = rid;
+    const int rid = sf_wire_geometry(W, lane, T, kind, x, y, angle);
+    if (valid && (lane & 3) == 0) sf_pool().stroke_region[idx] = (short)rid;
   } else {
     if (lane == 0) W.ngroups = 0;
   }
@@ -1224,7 +1266,7 @@ __device__ __forceinline__ void sf_phase_strokes(const SfDev& D, SfBlockSmem& B,
   for (int g = wi; g < total; g += nw) {
     const int owner = __popc(__ballot_sync(0xffffffffu, incl <= g));  // first warp whose inclusive count exceeds g
     const int first = __shfl_sync(0xffffffffu, incl - mine, owner);
-    sf_accumulate_pass(owner + 1, (g - first) << 2, sg);
+    sf_accumulate_pass(owner + 1, (g - first) << 2);
   }
   SF_PROF(20);
 }
@@ -1235,9 +1277,9 @@ __device__ __forceinline__ void sf_phase_window(const SfDev& D, SfBlockSmem& B, 
   int e, j0, i0, j1, i1;
   int quarter = -1, corigin = 0;
   if (t < netask) {
-    const int et = sf_team(sg).etask[t], kind = et >> 6;
+    const int et = sf_prep(sg).etask[t], kind = et >> 6;
     e = et & 63;
-    const SfEnvRec& rec = sf_team(sg).env[e];
+    const SfEnvRec& rec = sf_prep(sg).env[e];
     int x0, y0, x1, y1;
     if (kind < 4) {  // dead ship: a quarter (in output rows) of the explosion box
       const int bx0 = (rec.ebox & 255) - 64, by0 = ((rec.ebox >> 8) & 255) - 64;
@@ -1252,22 +1294,21 @@ __device__ __forceinline__ void sf_phase_window(const SfDev& D, SfBlockSmem& B, 
       corigin = (j0 & ~3) | (i0 << 8);  // cache columns are aligned with the 32-bit words of the observation row
       i0 += kind * hb; i1 = min(i1, i0 + hb - 1);
       if (i0 > i1) return;
-      quarter = kind;
+      quarter = (rec.building & 2) ? kind : -1;  // may this round refresh the env's cache (sf_publish_recs)?
     }
   } else {
-    const SfStrokeRec& S = sf_team(sg).stroke[t - netask];
-    const int sr = S.region;
+    const int sr = sf_pool().stroke_region[t - netask];
     if (sr < 0) return;
-    e = S.desc >> 12;
-    const int4 R = sf_team(sg).region[sr];
+    e = sf_prep(sg).stroke[t - netask].desc >> 12;
+    const int4 R = sf_pool().region[sr];
     j0 = B.col_out0[R.x]; j1 = B.col_out1[R.x + (R.z & 0xFFFF) - 1]; i0 = B.row_out0[R.y]; i1 = B.row_out1[R.y + ((R.z >> 16) & 0xFFFF) - 1];
   }
-  const int env = sf_team(sg).env[e].env;
+  const int env = sf_prep(sg).env[e].env;
   const bool cached = sf_window_orect(T, D.expc + (size_t)env * (SF_EXP_W * SF_EXP_W), e, j0, i0, j1, i1, sf_frame_ptr(out, e, env),
                                       quarter >= 0 ? D.expo + (size_t)env * SF_EXPO_BYTES : nullptr, corigin, sg);
   if (cached && lane == 0) {
     // mark the quarter valid, unless the stepping warp has already re-keyed the cache for the next tick
-    const SfEnvRec& rec = sf_team(sg).env[e];
+    const SfEnvRec& rec = sf_prep(sg).env[e];
     const unsigned long long want = (unsigned long long)rec.life | ((unsigned long long)sf_expo_key(rec) << 32);
     unsigned long long* m = reinterpret_cast<unsigned long long*>(&D.expo_meta[env]);
     unsigned long long old = *reinterpret_cast<volatile unsigned long long*>(m);
@@ -1282,7 +1323,7 @@ __device__ __forceinline__ void sf_phase_window(const SfDev& D, SfBlockSmem& B, 
 
 // native output (SSF_Env.step returns the 92x90 frame): tile `tile` (30x30 windows, 3 x 4 of them) of env slot e
 __device__ __forceinline__ void sf_phase_native_tile(const SfDev& D, SfBlockSmem& B, SfWarpSmem& W, int lane, int e, int tile, const SfFrameOut& out, int sg) {
-  const int env = sf_team(sg).env[e].env;
+  const int env = sf_prep(sg).env[e].env;
   if (env < 0) return;
   const int tx = (tile % 3) * 30, ty = (tile / 3) * 30;
   const int pw = min(30, SF_NAT_W - tx), ph = min(30, SF_NAT_H - ty);
@@ -1301,49 +1342,70 @@ __device__ __forceinline__ void sf_phase_native_tile(const SfDev& D, SfBlockSmem
 #define SF_WTICK(k) ((void)0)
 #endif
 
-// warp 0, one env per lane, on the records of the stage being prepared: a dead ship whose explosion sprite is not the
-// cached one gets it built in this tick; which quarters of its resampled explosion box are still valid. Runs while
-// the previous tick is drawn: a sprite stamp or valid bit that is set later than this is read only delays the use of
-// the memo by a tick (the rebuild is idempotent); sf_phase_window sets valid bits with a compare-and-swap against
-// the key, so a key written here is never combined with the bits of another one.
-__device__ __forceinline__ void sf_publish_recs(const SfDev& D, SfTeamSmem& Tm, int lane, int h, bool native) {
-  SfEnvRec& r = Tm.env[32 * h + lane];
+// warp 0, one env per lane, on the records of tick h of the stage being prepared in ring slot `cur`: a dead ship whose
+// explosion sprite is neither cached nor built by an earlier round gets it built in this round (bit 0); which quarters
+// of its resampled explosion box are valid (bits 4..7) and whether this round may refresh them (bit 1).
+// The stages still in the ring (the other slots, and the earlier tick of this one) were prepared before this one and
+// may not have been drawn yet; everything older has (warp 0 waited for the slot it now fills). Stages are drawn in the
+// order they were prepared, and a stage's writes to the caches are complete before the next one starts.
+//  * Sprite (expc / expstamp; written only by the build of (env, life)). A stamp equal to the life means the build has
+//    been drawn. An earlier record of the same env and life in the ring means that stage builds the sprite, or found it
+//    cached or scheduled itself: either way it exists before this stage is drawn, so it is not built again (with two
+//    stages of lead a death would otherwise be built three times; the round scan takes two builds per round). Nothing
+//    overwrites it in between: an earlier undrawn stage builds only for a life it holds, and a different life of the same
+//    env earlier in time would put this life's death (and its first build) after that stage.
+//  * Resampled box (expo / expo_meta). Warp 0 re-keys the meta, in preparation order, to (life, key) whenever a record
+//    differs from it; a window sets a quarter's valid bit with a compare-and-swap against its own (life, key), so bits are
+//    only ever set on the key they were computed for, and a stage trusts the bits it finds on its own key. The hazard of
+//    a lead: a window of an earlier, still undrawn stage with ANOTHER key overwriting the bytes of a quarter whose bit a
+//    stage of this key has set (or will set) after the re-key. So a stage may write the cache only if no record of the
+//    env in the ring has another (life, key) (bit 1). Then the last write of a quarter before a stage X that trusts it
+//    came from a stage W of X's key: a W with another key prepared after the re-key R would have re-keyed again, and one
+//    prepared before R was drawn after the stage Z of X's key that set the bit, so Z was undrawn and in the ring when W
+//    was prepared, which denies W the write. This costs the cache only the stages around a key change. The valid bits a
+//    stage finds are those of the stages drawn SF_PREP_SLOTS - 1 before it or earlier (one more stage of lag than with
+//    one stage of lead); the refreshes in between recompute identical pixels.
+__device__ __forceinline__ void sf_publish_recs(const SfDev& D, SfStagePrep* ring, int cur, int lane, int h, bool native) {
+  SfEnvRec& r = ring[cur].env[32 * h + lane];
   if (r.env >= 0 && !(r.core & SF_CORE_SHIP_ALIVE)) {
     const unsigned stamp = __ldcg(&D.expstamp[r.env]);  // both loads in flight together
     const unsigned long long mw = __ldcg(reinterpret_cast<const unsigned long long*>(&D.expo_meta[r.env]));
     const unsigned mx = (unsigned)mw, my = (unsigned)(mw >> 32);
+    const unsigned key = sf_expo_key(r);
     int building = stamp != r.life ? 1 : 0;
-    // second tick of the stage: the ship died in the first one, whose slot builds the sprite for both
-    if (h > 0 && building && !(Tm.env[lane].core & SF_CORE_SHIP_ALIVE) && Tm.env[lane].env == r.env && Tm.env[lane].life == r.life) building = 0;
+    bool refresh = true;
+#pragma unroll 1
+    for (int k = 0; k < SF_PREP_SLOTS * SF_STAGE_TICKS; k++) {
+      const int j = k / SF_STAGE_TICKS, hh = k - j * SF_STAGE_TICKS;
+      if (j == cur && hh >= h) continue;
+      const SfEnvRec& o = ring[j].env[32 * hh + lane];
+      if (o.env != r.env || (o.core & SF_CORE_SHIP_ALIVE)) continue;
+      if (o.life == r.life) building = 0;
+      if (o.life != r.life || sf_expo_key(o) != key) refresh = false;
+    }
     if (!native) {
-      const unsigned key = sf_expo_key(r);
       const bool same = mx == r.life && (my & 0x0FFFFFFFu) == key;
       if (same) { if (!building) building |= (int)(my >> 28) << 4; }
       else atomicExch(reinterpret_cast<unsigned long long*>(&D.expo_meta[r.env]), (unsigned long long)r.life | ((unsigned long long)key << 32));
     }
-    r.building = building;
+    r.building = building | (refresh ? 2 : 0);
   }
   __syncwarp();
 }
 
 // what persists from one group of envs to the next in a persistent block
 struct SfStageState {
-  int stage;      // copy (0 / 1) the next stage is drawn from
-  int prev_used;  // coverage cells the previous stage used in the OTHER copy: zeroed while the next stage is drawn
+  int stage;      // ring slot the next stage is drawn from
+  int prev_used;  // coverage cells the previous stage used: zeroed at the start of the next one
 };
 
-// warp 0: restart the pools of the copy whose stage it has just prepared
-__device__ __forceinline__ void sf_restart_pools(SfTeamSmem& Tm, int lane) {
-  if (lane == 0) { Tm.next_task = 0; Tm.next_patch = 0; Tm.nregions = 0; Tm.cells_used = 0; }
-  __syncwarp();
-}
-
-// warp 0: the first round of a new stage in Tm: up to SF_STAGE_TICKS consecutive ticks starting at tick t (nt of them
-// are left). prep(t, Tm, h) writes the env records of tick t into slots 32h .. 32h + 31 and leaves the SoA state at
-// that tick. The strokes of a tick are gathered from the state before it moves on, so the first tick must fit the
+// warp 0: the first round of a new stage in ring slot sg: up to SF_STAGE_TICKS consecutive ticks starting at tick t (nt
+// of them are left). prep(t, Tm, h) writes the env records of tick t into slots 32h .. 32h + 31 and leaves the SoA state
+// at that tick. The strokes of a tick are gathered from the state before it moves on, so the first tick must fit the
 // round in one piece; if it does not, the stage covers that tick only (and takes several rounds).
 template <class Prep>
-__device__ __forceinline__ void sf_prepare_first_round(const SfDev& D, const SfBlockSmem& B, SfTeamSmem& Tm, int lane, int t, int nt, SfFrameOut out, Prep prep) {
+__device__ __forceinline__ void sf_prepare_first_round(const SfDev& D, SfBlockSmem& B, int sg, int lane, int t, int nt, SfFrameOut out, Prep prep) {
+  SfStagePrep& Tm = B.prep[sg];
   const bool native = out.native != 0;
 #ifdef SF_BARRIER_TIMING
   long long tb_ = clock64();
@@ -1353,7 +1415,7 @@ __device__ __forceinline__ void sf_prepare_first_round(const SfDev& D, const SfB
 #endif
   prep(t, Tm, 0);
   SF_BT(3);
-  sf_publish_recs(D, Tm, lane, 0, native);
+  sf_publish_recs(D, B.prep, sg, lane, 0, native);
   SF_BT(4);
   SfScanState S;
   sf_scan_begin(S);
@@ -1367,7 +1429,7 @@ __device__ __forceinline__ void sf_prepare_first_round(const SfDev& D, const SfB
   if (nt > 1 && !Tm.more) {
     prep(t + 1, Tm, 1);
     SF_BT(3);
-    sf_publish_recs(D, Tm, lane, 1, native);
+    sf_publish_recs(D, B.prep, sg, lane, 1, native);
     SF_BT(4);
     sf_scan_half(Tm, lane, 1, 0, S);   // continues the first tick's scan (the round was not closed: !Tm.more)
     sf_scan_finish(Tm, lane, 0, S);
@@ -1378,16 +1440,17 @@ __device__ __forceinline__ void sf_prepare_first_round(const SfDev& D, const SfB
   }
 #endif
   if (lane == 0) Tm.nticks = nticks;
-  sf_restart_pools(Tm, lane);
+  __syncwarp();
   SF_BT(7);
 }
 
-// One stage drawn by the 15 drawing warps (see the pipeline description above): B1 geometry, B3 passes, base
-// patches, B2 explosion sprite, C windows.
-__device__ __forceinline__ void sf_draw_stage(const SfDev& D, SfBlockSmem& B, SfWarpSmem& W, int lane, const SfFrameOut& out, int sg) {
+// One stage drawn by the 23 drawing warps (see the pipeline description above): B1 geometry, B3 passes, base
+// patches, B2 explosion sprite, C windows. Returns the coverage cells the stage used (zeroed at the start of the next).
+__device__ __forceinline__ int sf_draw_stage(const SfDev& D, SfBlockSmem& B, SfWarpSmem& W, int lane, const SfFrameOut& out, int sg) {
   const int warp = threadIdx.x >> 5;
   const int wi = warp - 1, nw = SF_RENDER_WARPS - 1;  // index among the drawing warps, and their number
-  SfTeamSmem& Tm = sf_team(sg);
+  const SfStagePrep& Tm = B.prep[sg];
+  SfStagePool& P = B.pool;
 #ifdef SF_PHASE_TIMING
   long long t_last_ = clock64(), w_last_ = t_last_;
   const int gwarp = warp;
@@ -1412,9 +1475,9 @@ __device__ __forceinline__ void sf_draw_stage(const SfDev& D, SfBlockSmem& B, Sf
     if (base_issuer) {
       asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
       __syncwarp();
-      if (lane == 0) { __threadfence_block(); *(volatile int*)&Tm.base_ready = 1; }
+      if (lane == 0) { __threadfence_block(); *(volatile int*)&P.base_ready = 1; }
     } else {
-      while (*(volatile int*)&Tm.base_ready == 0) {}
+      while (*(volatile int*)&P.base_ready == 0) {}
     }
     __syncwarp();
     SF_PROF(65);
@@ -1422,7 +1485,7 @@ __device__ __forceinline__ void sf_draw_stage(const SfDev& D, SfBlockSmem& B, Sf
 #pragma unroll 1
     for (;;) {
       int e = 0;
-      if (lane == 0) e = atomicAdd(&Tm.next_patch, 1);
+      if (lane == 0) e = atomicAdd(&P.next_patch, 1);
       e = r0 + __shfl_sync(0xffffffffu, e, 0);
       if (e >= r1) break;
       sf_env_base_patch(D, B, lane, e, out, sg);
@@ -1430,11 +1493,15 @@ __device__ __forceinline__ void sf_draw_stage(const SfDev& D, SfBlockSmem& B, Sf
     SF_PROF(66);
   }
 #ifdef SF_PHASE_TIMING
-  if (lane == 0 && blockIdx.x == 0) { atomicAdd(&sf_dbg_cycles[32 + (gwarp & 15)], (unsigned long long)(clock64() - w_last_)); atomicMax(&Tm.dbg_max_b, (int)(clock64() - w_last_)); }
+  if (lane == 0 && blockIdx.x == 0) { atomicAdd(&sf_dbg_cycles[32 + (gwarp & 15)], (unsigned long long)(clock64() - w_last_)); atomicMax(&P.dbg_max_b, (int)(clock64() - w_last_)); }
 #endif
   SF_WTICK(10);
+  const int used = P.cells_used;  // final since the geometry barrier in sf_phase_strokes
   sf_render_sync();
   SF_TICK(2); SF_WTICK(8);
+  // the counters of B are not touched again in this stage: restart them for the next one (its B1 starts after every
+  // drawing warp has synced on the next stage's full barrier)
+  if (threadIdx.x == 32) { P.nregions = 0; P.cells_used = 0; P.next_patch = 0; P.base_ready = 0; }
   // ---- C: window tasks, handed out first come first served (env tasks first: the big ones) ----
   SF_PROF_RESET();
   if (!out.native) {
@@ -1442,7 +1509,7 @@ __device__ __forceinline__ void sf_draw_stage(const SfDev& D, SfBlockSmem& B, Sf
 #pragma unroll 1
     for (;;) {
       int t = 0;
-      if (lane == 0) t = atomicAdd(&Tm.next_task, 1);
+      if (lane == 0) t = atomicAdd(&P.next_task, 1);
       t = __shfl_sync(0xffffffffu, t, 0);
       if (t >= netask + nst) break;
       SF_PROF(29);
@@ -1453,45 +1520,67 @@ __device__ __forceinline__ void sf_draw_stage(const SfDev& D, SfBlockSmem& B, Sf
     for (int t = wi; t < (r1 - r0) * 12; t += nw) sf_phase_native_tile(D, B, W, lane, r0 + t / 12, t % 12, out, sg);
   }
 #ifdef SF_PHASE_TIMING
-  if (lane == 0 && blockIdx.x == 0) { atomicAdd(&sf_dbg_cycles[48 + (gwarp & 15)], (unsigned long long)(clock64() - w_last_)); atomicMax(&Tm.dbg_max_c, (int)(clock64() - w_last_)); }
+  if (lane == 0 && blockIdx.x == 0) { atomicAdd(&sf_dbg_cycles[48 + (gwarp & 15)], (unsigned long long)(clock64() - w_last_)); atomicMax(&P.dbg_max_c, (int)(clock64() - w_last_)); }
   SF_WTICK(11);
   if (threadIdx.x == 32 && blockIdx.x == 0) {
-    atomicAdd(&sf_dbg_cycles[71], (unsigned long long)Tm.dbg_max_b); atomicAdd(&sf_dbg_cycles[72], (unsigned long long)Tm.dbg_max_c);
+    atomicAdd(&sf_dbg_cycles[71], (unsigned long long)P.dbg_max_b); atomicAdd(&sf_dbg_cycles[72], (unsigned long long)P.dbg_max_c);
     atomicAdd(&sf_dbg_cycles[73], 1ull); atomicAdd(&sf_dbg_cycles[74], (unsigned long long)(Tm.netask + nst)); atomicAdd(&sf_dbg_cycles[75], (unsigned long long)Tm.netask);
     atomicAdd(&sf_dbg_cycles[76], (unsigned long long)(Tm.build_env >= 0));
-    Tm.dbg_max_b = 0; Tm.dbg_max_c = 0;
+    P.dbg_max_b = 0; P.dbg_max_c = 0;
   }
 #endif
+  return used;
 }
 
-// All frames of T consecutive ticks of one group, as two ROLES that run the same stage sequence and meet at one block
-// barrier per stage: sf_stepper_ticks (warp 0) and sf_drawer_ticks (the other warps). prep(t, Tm, h) is executed by
-// warp 0 only and writes the env records of tick t into Tm.env[32h ..] (one env per lane, env = -1: unused); for a
-// rollout it is the step of tick t, which therefore runs while the other warps draw the ticks before it.
-// A STAGE is a round of up to SF_STAGE_TICKS consecutive ticks. Stage s is drawn from copy s & 1 by the drawing warps
-// while warp 0 prepares stage s + 1 in the other copy; ONE block barrier per stage separates them. Nothing of a
-// stage that is being drawn reads the SoA state, so the steps may overwrite it; the strokes of a LATER round of the
-// same stage are gathered (from the state, which still holds the stage's last tick) before the next step.
+// All frames of T consecutive ticks of one group, as two ROLES that run the same stage sequence: sf_stepper_ticks
+// (warp 0) and sf_drawer_ticks (the other warps). prep(t, Tm, h) is executed by warp 0 only and writes the env records
+// of tick t into Tm.env[32h ..] (one env per lane, env = -1: unused); for a rollout it is the step of tick t, which
+// therefore runs while the other warps draw the ticks before it.
+// A STAGE is a round of up to SF_STAGE_TICKS consecutive ticks, prepared in ring slot s % SF_PREP_SLOTS. Warp 0 fills
+// the slots in drawing order and hands each one over at its full barrier; it waits (empty barrier) only when it is
+// SF_PREP_SLOTS stages ahead of the drawing warps, so a slow stage on one side is absorbed by the lead instead of
+// stalling the other side. Nothing of a stage that is being drawn reads the SoA state, so the steps may overwrite it;
+// the strokes of a LATER round of the same stage are gathered (from the state, which still holds the stage's last tick)
+// before the next step.
 // The roles are separate functions on purpose: the rollout kernel calls them out of line, so that each role gets its own
 // register allocation (sharing one loop, the long-lived variables of the drawing warps were spilled around the stepping
 // warp's calls and reloaded inside the drawing code: nvdisasm -g attribution of LDL / STL).
+
+// warp 0: the ring slot of its stage number `stage` (stages prepared by the block so far), once the drawing warps have
+// drawn what the slot held
+__device__ __forceinline__ int sf_stepper_claim(int stage) {
+  const int sg = stage % SF_PREP_SLOTS;
+  SF_TL(4);
+  if (stage >= SF_PREP_SLOTS) sf_stage_empty_wait(sg);
+  SF_TL(5);
+  return sg;
+}
+// warp 0, at the end of the kernel: take the drawing warps' arrivals for the last stages, so that no named barrier is
+// left half arrived
+__device__ __forceinline__ void sf_stepper_drain(int stage) {
+#pragma unroll 1
+  for (int s = max(stage - SF_PREP_SLOTS, 0); s < stage; s++)
+    asm volatile("bar.sync %0, %1;" :: "r"(3 + SF_PREP_SLOTS + s % SF_PREP_SLOTS), "r"(32 * SF_RENDER_WARPS) : "memory");
+}
+
 template <class Prep>
 __device__ __forceinline__ void sf_stepper_ticks(const SfDev& D, SfBlockSmem& B, int lane, bool native, int T, int& stage, Prep prep) {
   SfFrameOut out;
   out.obs = nullptr; out.obs_bytes = 0; out.tick_bytes = 0; out.native = native ? 1 : 0;
-  sf_prepare_first_round(D, B, B.team[stage], lane, 0, T, out, prep);
+  int sg = sf_stepper_claim(stage);
+  sf_prepare_first_round(D, B, sg, lane, 0, T, out, prep);
   SF_TL(3);
   int t = 0;
 #pragma unroll 1
   for (;;) {
-    SF_TL(4);
-    sf_team_sync();  // the stage is prepared; every warp is done with the previous one
-    SF_TL(5);
-    SfTeamSmem& Tm = B.team[stage];
-    SfTeamSmem& Nx = B.team[stage ^ 1];
+    sf_stage_full_arrive(sg);  // the stage is prepared
+    stage++;
+    const SfStagePrep& Tm = B.prep[sg];
     const bool more = Tm.more != 0;            // more env slots in the stage than this round could take?
     const int nticks = Tm.nticks;
-    const bool last = !more && t + nticks >= T;
+    if (!more && t + nticks >= T) break;
+    const int nx = sf_stepper_claim(stage);
+    SfStagePrep& Nx = B.prep[nx];
     if (more) {
 #pragma unroll
       for (int h = 0; h < SF_STAGE_TICKS; h++) Nx.env[32 * h + lane] = Tm.env[32 * h + lane];
@@ -1499,13 +1588,11 @@ __device__ __forceinline__ void sf_stepper_ticks(const SfDev& D, SfBlockSmem& B,
       __syncwarp();
       sf_round_scan(Nx, lane, Tm.r1, SF_GROUP_ENVS * nticks);
       sf_gather_strokes(D, Nx, lane, nticks - 1);  // the slots that are left are of the stage's last tick (see above)
-      sf_restart_pools(Nx, lane);
-    } else if (!last) {
-      sf_prepare_first_round(D, B, Nx, lane, t + nticks, T - (t + nticks), out, prep);
+    } else {
+      sf_prepare_first_round(D, B, nx, lane, t + nticks, T - (t + nticks), out, prep);
+      t += nticks;
     }
-    stage ^= 1;
-    if (!more) t += nticks;
-    if (last) break;
+    sg = nx;
   }
   SF_TL(7);
 }
@@ -1515,23 +1602,25 @@ __device__ __forceinline__ void sf_drawer_ticks(const SfDev& D, SfBlockSmem& B, 
   int t = 0;
 #pragma unroll 1
   for (;;) {
+    const int sg = st.stage;
     SF_TL(4);
-    sf_team_sync();  // the stage is prepared; every warp is done with the previous one
+    sf_stage_full_wait(sg);  // the stage is prepared, and every drawing warp is done with the one before it
     SF_TL(5);
-    SfTeamSmem& Tm = B.team[st.stage];
-    SfTeamSmem& Nx = B.team[st.stage ^ 1];
+    const SfStagePrep& Tm = B.prep[sg];
     const bool more = Tm.more != 0;
     const int nticks = Tm.nticks;
     const bool last = !more && t + nticks >= T;
-    // zero the coverage cells of the stage before this one (the other copy)
+    // the pool is the previous stage's until here: zero the coverage cells it used (before the passes of this stage,
+    // which follow the geometry barrier) and restart the window queue (used after the second barrier)
     {
       const int nz = (st.prev_used + 1) >> 1;
-      for (int k = threadIdx.x - 32; k < nz; k += 32 * (SF_RENDER_WARPS - 1)) reinterpret_cast<unsigned*>(Nx.cells)[k] = 0u;
+      for (int k = threadIdx.x - 32; k < nz; k += 32 * (SF_RENDER_WARPS - 1)) reinterpret_cast<unsigned*>(B.pool.cells)[k] = 0u;
+      if (threadIdx.x == 32) B.pool.next_task = 0;
     }
     out.obs = obs0 + (size_t)t * out.tick_bytes;
-    sf_draw_stage(D, B, W, lane, out, st.stage);
-    st.prev_used = Tm.cells_used;
-    st.stage ^= 1;
+    st.prev_used = sf_draw_stage(D, B, W, lane, out, sg);
+    sf_stage_empty_arrive(sg);  // the slot may be refilled
+    st.stage = sg + 1 == SF_PREP_SLOTS ? 0 : sg + 1;
     if (!more) t += nticks;
     if (last) break;
   }

@@ -26,9 +26,9 @@ blocks = min(148, (n + 31) // 32 if n > 148 * 32 else 147)
 cyc = ms * 1e-3 * 1.965e9
 W = 24
 print(os.path.basename(os.environ.get("SF_B200_LIB", "")), "%s n=%d: launch %.3f ms = %.0f cycles; %.3e steps/s" % (gt, n, ms, cyc, n * T / ms * 1e3))
-print("per drawing warp: stage barrier %.1f %%, drawing-warp barriers %.1f %% of the launch; stepping warp at the stage barrier %.1f %%"
+print("per drawing warp: waiting for a prepared stage (full barriers) %.1f %%, drawing-warp barriers %.1f %% of the launch; stepping warp waiting for a free ring slot (empty barriers) %.1f %%"
       % (100 * v[0] / (blocks * (W - 1)) / cyc, 100 * v[1] / (blocks * (W - 1)) / cyc, 100 * v[2] / blocks / cyc))
-print("stepping warp, share of the launch: steps %.1f %%, memo state %.1f %%, round scans %.1f %%, stroke gathering %.1f %%, pools + base copies %.1f %%"
+print("stepping warp, share of the launch: steps %.1f %%, memo state %.1f %%, round scans %.1f %%, stroke gathering %.1f %%, stage control words %.1f %%"
       % tuple(100 * v[k] / blocks / cyc for k in (3, 4, 5, 6, 7)))
 print("step sections, cycles per tick and block: load %.0f | keys + respawn %.0f | ship %.0f | fortress %.0f | shells %.0f | missiles %.0f | timers + shaping %.0f | outputs + store + record %.0f"
       % tuple(v[k] / blocks / T for k in (8, 9, 10, 11, 12, 13, 14, 15)))
