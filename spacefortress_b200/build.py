@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libsf_b200.so")
 SOURCES = ["sf_kernels.cu", "sf_tables.cpp"]
-HEADERS = ["sf_geom.h", "sf_tables.h", "sf_state.cuh", "sf_step.cuh", "sf_render.cuh", os.path.join("..", "..", "include", "sf_b200.h")]
+HEADERS = ["sf_geom.h", "sf_tables.h", "sf_state.cuh", "sf_probe.cuh", "sf_step.cuh", "sf_render.cuh", os.path.join("..", "..", "include", "sf_b200.h")]
 
 
 def _nvcc():
@@ -30,9 +30,11 @@ def needs_build():
 
 
 def build(force=False, verbose=False, out=None, defs=None):
-    """out / defs: a variant build (tools/: instrumented or experimental -D knobs) beside the product library."""
+    """out / defs: a variant build beside the product library, e.g. a probe of csrc/sf_probe.cuh (defs="-DSF_TIMELINE")."""
     if out is None and not force and not needs_build():
         return LIB
+    if out is not None:
+        os.makedirs(os.path.dirname(os.path.abspath(out)), exist_ok=True)
     cmd = [
         _nvcc(), "-shared", "-o", out or LIB,
         "-gencode", "arch=compute_100a,code=sm_100a",
@@ -43,7 +45,7 @@ def build(force=False, verbose=False, out=None, defs=None):
         "--fmad=false",
         "-Xptxas", "-v" if verbose else "-O3",
         "-I", os.path.join(HERE, "..", "include"),
-    ] + (defs.split() if defs is not None else os.environ.get("SF_NVCC_DEFS", "").split()) + [os.path.join(CSRC, s) for s in SOURCES]
+    ] + (defs or "").split() + [os.path.join(CSRC, s) for s in SOURCES]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if r.returncode != 0:
         raise RuntimeError("nvcc failed:\n%s\n%s" % (r.stdout, r.stderr))

@@ -31,11 +31,7 @@
 #include "sf_step.cuh"
 #include "sf_tables.h"
 
-#define SF_WARPS_PER_BLOCK SF_RENDER_WARPS  // sf_render.cuh: one block per SM
-#define SF_BLOCK (32 * SF_WARPS_PER_BLOCK)
-#ifndef SF_BLOCKS_PER_SM
-#define SF_BLOCKS_PER_SM 1  // resident blocks per SM (each with its own stepping warp, pools and barriers)
-#endif
+#define SF_BLOCK (32 * SF_RENDER_WARPS)  // sf_render.cuh: one block per SM
 
 // ------------------------------------------------------------------------------------------------
 // synthetic policy: stateless counter hash (SURVEY.md §8(d)); same function on host and device
@@ -89,13 +85,6 @@ __device__ __forceinline__ void sf_accumulate_episode(const SfDev& D, int env, S
   int4 st0 = make_int4(0, 0, 0, 0), st1 = st0, st2 = st0;
   if (finished) { sf_flush_stats(D, env, e); st0 = __ldcg(&D.st0[env]); st1 = __ldcg(&D.st1[env]); st2 = __ldcg(&D.st2[env]); }
   sf_accumulate_episode_vals(D.epi, finished, lane, e.q3.w, e.q3.z, e.q3.x, e.q3.y, e.st3.x, st0, st1, st2);
-}
-// The rollout kernel's stepping warp takes the env by REFERENCE instead, out of line: that keeps its SfEnv in local memory
-// (L1) and its register demand low, and with it the register allocation of the whole kernel body — the drawing code
-// inlined next to it then comes out without a single spill (with the by-value call it has ~15 local loads / stores in
-// sf_draw_stage / sf_phase_strokes / sf_env_base_patch and the launch is 5 % slower: tools/gpu_ab.py + nvdisasm -g).
-__device__ __noinline__ void sf_accumulate_episode_ref(const SfDev& D, int env, SfEnv& e, bool finished, int lane) {
-  sf_accumulate_episode(D, env, e, finished, lane);
 }
 
 // the renderer's view of one stepped env (written by the env's lane into the block's record array)
@@ -162,10 +151,7 @@ __device__ __noinline__ void sf_step_group(const SfDev& D, const SfRollArgs& A, 
   SfEnv e;
   bool finished = false;
   unsigned shell_vis = 0;
-#ifdef SF_BARRIER_TIMING
-  unsigned stmask_ = __ballot_sync(0xffffffffu, mine);
-#endif
-  SF_ST_BEGIN();
+  SF_ST_BEGIN(__ballot_sync(0xffffffffu, mine));
   SfStepSmem& SS = sf_block_smem().step;
   const bool first_tick = t == 0, last_tick = t == A.T - 1;
   if (mine) {
@@ -175,17 +161,12 @@ __device__ __noinline__ void sf_step_group(const SfDev& D, const SfRollArgs& A, 
       e.q0 = SS.q0[lane]; e.q1 = SS.q1[lane]; e.q2 = SS.q2[lane]; e.q3 = SS.q3[lane]; e.st3 = SS.st3[lane];
       e.d0 = SS.d0[lane]; e.d1 = SS.d1[lane]; e.d2 = SS.d2[lane];
     }
-#ifdef SF_BARRIER_TIMING
-    if (e.q0.x == 0x7fffffff) e.q0.y = 0;  // (a use of the loaded words: the section ends when they have arrived)
-#endif
+    SF_ST_USE(e.q0.x, e.q0.y);
     SF_ST(8);
     int a = A.actions ? A.actions[(size_t)t * D.n + env]
                       : sf_hash_action(A.action_seed, (unsigned long long)(D.first_global_env + env), (unsigned long long)(A.t0 + t), D.num_actions);
     int km = (A.flags & SF_FLAG_ACTIONS_ARE_KEYMASKS) ? (a & 15) : D.keymask_of_action[min(max(a, 0), D.num_actions - 1)];
     SfStepOut o;
-#ifdef SF_BARRIER_TIMING
-    o.sync_mask = stmask_;
-#endif
     sf_env_step(D, H, env, e, km, autoreset, (A.flags & SF_FLAG_RAW_REWARD) != 0, o);
     size_t oi = (size_t)t * D.n + env;
     if (A.reward) A.reward[oi] = o.reward;
@@ -195,15 +176,9 @@ __device__ __noinline__ void sf_step_group(const SfDev& D, const SfRollArgs& A, 
     finished = o.done && autoreset;
     shell_vis = o.shell_vis;
   }
-#ifdef SF_BARRIER_TIMING
-  ts_ = clock64(); stmask_ = 0xffffffffu;
-#endif
+  SF_ST_RESTART(0xffffffffu);
   if (__any_sync(0xffffffffu, finished)) {
-#ifdef SF_STEP_ENV_BY_REF
-    sf_accumulate_episode_ref(D, env, e, finished, lane);
-#else
     sf_accumulate_episode(D, env, e, finished, lane);
-#endif
     if (finished) { sf_new_game(D, H, env, e); shell_vis = 0; }  // gym_vecenv: the returned obs is the first frame of the new episode
   }
   if (mine) {
@@ -308,7 +283,7 @@ __device__ __noinline__ void sf_block_host_delta(const SfDev& D, const SfRollArg
 // (HOST_DELTA is a second instantiation, used by sf_step_host only: the register allocation of the plain kernel is
 // sensitive to anything that is added to its body, see DESIGN.md 7b.)
 template <bool HOST_DELTA>
-__global__ void __launch_bounds__(SF_BLOCK, SF_BLOCKS_PER_SM) sf_rollout_kernel(const __grid_constant__ SfDev D, const __grid_constant__ SfRollArgs A) {
+__global__ void __launch_bounds__(SF_BLOCK, 1) sf_rollout_kernel(const __grid_constant__ SfDev D, const __grid_constant__ SfRollArgs A) {
   sf_block_smem_init(D.static_image);
   sf_warp_smem_init(sf_my_smem(), threadIdx.x & 31);
   if (threadIdx.x < 32) sf_rollout_stepper(D, A); else sf_rollout_drawer(D, A);
@@ -333,9 +308,6 @@ __global__ void __launch_bounds__(128) sf_step_only_kernel(SfDev D, SfRollArgs A
                         : sf_hash_action(A.action_seed, (unsigned long long)(D.first_global_env + env), (unsigned long long)(A.t0 + t), D.num_actions);
       int km = (A.flags & SF_FLAG_ACTIONS_ARE_KEYMASKS) ? (a & 15) : D.keymask_of_action[min(max(a, 0), D.num_actions - 1)];
       SfStepOut o;
-#ifdef SF_BARRIER_TIMING
-      o.sync_mask = __activemask();
-#endif
       sf_env_step(D, &D.tab->hot, env, e, km, autoreset, (A.flags & SF_FLAG_RAW_REWARD) != 0, o);
       size_t oi = (size_t)t * D.n + env;
       if (A.reward) A.reward[oi] = o.reward;
@@ -354,7 +326,7 @@ __global__ void __launch_bounds__(128) sf_step_only_kernel(SfDev D, SfRollArgs A
 }
 
 // render the current state (Game.draw): the same block-cooperative pipeline without the step
-__global__ void __launch_bounds__(SF_BLOCK, SF_BLOCKS_PER_SM) sf_render_kernel(SfDev D, unsigned char* obs, int flags, const unsigned char* mask, int EB, int ngroups) {
+__global__ void __launch_bounds__(SF_BLOCK, 1) sf_render_kernel(SfDev D, unsigned char* obs, int flags, const unsigned char* mask, int EB, int ngroups) {
   const int lane = threadIdx.x & 31;
   SfBlockSmem& B = sf_block_smem();
   SfWarpSmem& W = sf_my_smem();
@@ -753,7 +725,7 @@ static int fail(int code, const std::string& msg) { g_err = msg; return code; }
 #define CUDA_TRY(x) do { cudaError_t e_ = (x); if (e_ != cudaSuccess) return fail(SF_ERR_CUDA, std::string(#x) + ": " + cudaGetErrorString(e_)); } while (0)
 
 #define SF_MAX_MIRRORS 4
-#define SF_HOST_MAX_SLICES 8
+#define SF_HOST_STEP_SLICES 4  // sf_step_host with whole frames: launches over slices of the slab (see there)
 struct sf_handle {
   SfDev dev;
   int device;
@@ -768,8 +740,7 @@ struct sf_handle {
   size_t staging_obs_bytes;
   SfSched* d_sched;  // sf_rollout_kernel's scheduling state (group hand-out, cost-dealt envs)
   cudaStream_t host_compute, host_copy;  // sf_step_host: kernels of slice k + 1 overlap the device->host copy of slice k
-  cudaEvent_t host_ev[SF_HOST_MAX_SLICES];
-  int host_slices;
+  cudaEvent_t host_ev[SF_HOST_STEP_SLICES];
   // SF_FLAG_HOST_DELTA: device copy of what the caller's page-locked h_obs holds, so that only changed bytes cross PCIe
   struct Mirror { const void* host; unsigned char* d; size_t cap, bytes; unsigned long long used; };
   Mirror mirrors[SF_MAX_MIRRORS];     // one per host buffer (a caller may rotate a few buffers); least recently used goes first
@@ -888,13 +859,13 @@ extern "C" int sf_create(const char* gametype, int action_set, int n_envs, int d
   if ((ce = cudaMemset(h->d_sched, 0, sizeof(SfSched))) != cudaSuccess) return bail("cudaMemset scheduler state", ce);
   if ((ce = cudaMemset(h->slab, 0, h->slab_bytes)) != cudaSuccess) return bail("cudaMemset state slab", ce);
   if ((ce = cudaMemcpy((void*)d.tab, h->h_tab, sizeof(SfTables), cudaMemcpyHostToDevice)) != cudaSuccess) return bail("upload tables", ce);
-  if ((ce = cudaFuncSetAttribute(sf_rollout_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK))) != cudaSuccess) return bail("shared memory opt-in (rollout)", ce);
-  if ((ce = cudaFuncSetAttribute(sf_rollout_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK))) != cudaSuccess) return bail("shared memory opt-in (rollout, host delta)", ce);
-  if ((ce = cudaFuncSetAttribute(sf_render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK))) != cudaSuccess) return bail("shared memory opt-in (render)", ce);
-  if ((ce = cudaFuncSetAttribute(sf_pack_static_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK))) != cudaSuccess) return bail("shared memory opt-in (pack)", ce);
+  if ((ce = cudaFuncSetAttribute(sf_rollout_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS))) != cudaSuccess) return bail("shared memory opt-in (rollout)", ce);
+  if ((ce = cudaFuncSetAttribute(sf_rollout_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS))) != cudaSuccess) return bail("shared memory opt-in (rollout, host delta)", ce);
+  if ((ce = cudaFuncSetAttribute(sf_render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS))) != cudaSuccess) return bail("shared memory opt-in (render)", ce);
+  if ((ce = cudaFuncSetAttribute(sf_pack_static_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS))) != cudaSuccess) return bail("shared memory opt-in (pack)", ce);
   if ((ce = cudaFuncSetAttribute(sf_save_envs_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared)) != cudaSuccess) return bail("shared memory carveout (save envs)", ce);
   if ((ce = cudaFuncSetAttribute(sf_load_envs_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared)) != cudaSuccess) return bail("shared memory carveout (load envs)", ce);
-  sf_pack_static_kernel<<<1, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK)>>>(d, const_cast<unsigned char*>(d.static_image));
+  sf_pack_static_kernel<<<1, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS)>>>(d, const_cast<unsigned char*>(d.static_image));
   if ((ce = cudaGetLastError()) != cudaSuccess) return bail("static image kernel launch", ce);
   // default seeding: every env replays srand(1) — the reference never seeds libc (game.cpp:137-148)
   sf_seed_kernel<<<(d.n + 127) / 128, 128>>>(d, nullptr);
@@ -919,7 +890,7 @@ extern "C" int sf_destroy(sf_handle* h) {
   if (h->d_delta_stats) cudaFree(h->d_delta_stats);
   if (h->host_compute) cudaStreamDestroy(h->host_compute);
   if (h->host_copy) cudaStreamDestroy(h->host_copy);
-  for (int k = 0; k < SF_HOST_MAX_SLICES; k++) if (h->host_ev[k]) cudaEventDestroy(h->host_ev[k]);
+  for (int k = 0; k < SF_HOST_STEP_SLICES; k++) if (h->host_ev[k]) cudaEventDestroy(h->host_ev[k]);
   delete h->h_tab;
   delete h;
   return SF_OK;
@@ -961,9 +932,8 @@ extern "C" int sf_seed(sf_handle* h, const uint32_t* h_seeds, long long first_gl
 // the SMs (4096 envs -> 28 per block, 147 blocks); beyond that a group is a full warp of 32 stepping lanes and
 // the blocks are persistent over their groups.
 static void group_shape(const sf_handle* h, int n, int* EB, int* ngroups, int* blocks) {
-  const int sms = h->num_sms * SF_BLOCKS_PER_SM, teams = sms;
-  int eb = n <= teams * SF_GROUP_ENVS ? (n + teams - 1) / teams : SF_GROUP_ENVS;
-  if (const char* ov = getenv("SF_ENVS_PER_BLOCK")) { int e = atoi(ov); if (e >= 1 && e <= SF_GROUP_ENVS) eb = e; }  // tuning knob
+  const int sms = h->num_sms;  // one block per SM
+  const int eb = n <= sms * SF_GROUP_ENVS ? (n + sms - 1) / sms : SF_GROUP_ENVS;
   *EB = eb;
   *ngroups = (n + eb - 1) / eb;
   *blocks = std::min(*ngroups, sms);
@@ -972,7 +942,7 @@ static void group_shape(const sf_handle* h, int n, int* EB, int* ngroups, int* b
 static int launch_render(sf_handle* h, unsigned char* d_obs, int flags, const unsigned char* d_mask, cudaStream_t st) {
   int EB, ngroups, blocks;
   group_shape(h, h->dev.n, &EB, &ngroups, &blocks);
-  sf_render_kernel<<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK), st>>>(h->dev, d_obs, flags, d_mask, EB, ngroups);
+  sf_render_kernel<<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(h->dev, d_obs, flags, d_mask, EB, ngroups);
   CUDA_TRY(cudaGetLastError());
   return SF_OK;
 }
@@ -1108,8 +1078,8 @@ static int launch_rollout(sf_handle* h, const SfRollArgs& a, cudaStream_t st) {
     int blocks;
     group_shape(h, b.envn, &b.EB, &b.ngroups, &blocks);
     b.sched = (a.env0 == 0 && a.envn == d.n && !a.host_obs) ? h->d_sched : nullptr;  // slices of the slab (sf_step_host), in-kernel delta: static groups
-    if (b.host_obs) sf_rollout_kernel<true><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK), st>>>(d, b);
-    else sf_rollout_kernel<false><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK), st>>>(d, b);
+    if (b.host_obs) sf_rollout_kernel<true><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, b);
+    else sf_rollout_kernel<false><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, b);
   } else {
     sf_step_only_kernel<<<(a.envn + 127) / 128, 128, 0, st>>>(d, a);
   }
@@ -1185,9 +1155,7 @@ static int ensure_staging(sf_handle* h, size_t obs_bytes) {
   if (!h->host_compute) {
     CUDA_TRY(cudaStreamCreateWithFlags(&h->host_compute, cudaStreamNonBlocking));
     CUDA_TRY(cudaStreamCreateWithFlags(&h->host_copy, cudaStreamNonBlocking));
-    for (int k = 0; k < SF_HOST_MAX_SLICES; k++) CUDA_TRY(cudaEventCreateWithFlags(&h->host_ev[k], cudaEventDisableTiming));
-    h->host_slices = 4;
-    if (const char* ov = getenv("SF_HOST_SLICES")) { int v = atoi(ov); if (v >= 1 && v <= SF_HOST_MAX_SLICES) h->host_slices = v; }  // tuning knob
+    for (int k = 0; k < SF_HOST_STEP_SLICES; k++) CUDA_TRY(cudaEventCreateWithFlags(&h->host_ev[k], cudaEventDisableTiming));
     h->delta_lanes = 4;  // 64 bytes: whole host cache lines (no partial-line writes in the host's memory system)
     if (const char* ov = getenv("SF_DELTA_GRANULE")) { int v = atoi(ov); if (v == 16 || v == 32 || v == 64 || v == 128 || v == 256) h->delta_lanes = v / 16; }  // tuning knob
   }
@@ -1221,20 +1189,8 @@ static void* device_alias(const void* host) {
   return at.type == cudaMemoryTypeHost ? at.devicePointer : nullptr;
 }
 
-#ifdef SF_HOST_PROFILE  // tools/: host-side phases of sf_step_host (ns, averaged, printed every 512 calls)
-#include <time.h>
-static double g_hp[8]; static long g_hp_calls; static double g_hp_last;
-static double hp_now() { timespec ts; clock_gettime(CLOCK_MONOTONIC, &ts); return ts.tv_sec * 1e9 + ts.tv_nsec; }
-#define SF_HP(k) do { double t_ = hp_now(); if (k == 0) { g_hp_calls++; } else g_hp[k] += t_ - g_hp_last; g_hp_last = t_; \
-  if (k == 5 && g_hp_calls % 512 == 0) { fprintf(stderr, "sf_step_host phases (us): entry %.1f legacy-sync %.1f aliases %.1f launches %.1f wait %.1f\n", \
-    g_hp[1] / 512e3, g_hp[2] / 512e3, g_hp[3] / 512e3, g_hp[4] / 512e3, g_hp[5] / 512e3); for (double& v : g_hp) v = 0; } } while (0)
-#else
-#define SF_HP(k) do {} while (0)
-#endif
-
 extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_obs, int32_t* h_reward, uint8_t* h_done,
                             uint8_t* h_fortkill, uint32_t* h_events, int flags) {
-  SF_HP(0);
   if (!h || !h_actions) return fail(SF_ERR_INVALID, "handle or actions is NULL");
   CUDA_TRY(cudaSetDevice(h->device));
   size_t n = (size_t)h->dev.n;
@@ -1275,18 +1231,15 @@ extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_o
   }
   const bool delta = want_delta && mir->host == h_obs && mir->bytes == obs_bytes;
   flags &= ~SF_FLAG_HOST_DELTA;
-  SF_HP(1);
   CUDA_TRY(cudaStreamSynchronize(cudaStreamLegacy));  // calls made with stream == NULL (sf_reset, sf_seed ...) come first
-  SF_HP(2);
   // page-locked actions / rewards / dones / kills / events are read and written in place by the kernel
   const int* k_actions = (const int*)device_alias(h_actions);
   int* k_reward = (int*)device_alias(h_reward);
   unsigned char* k_done = (unsigned char*)device_alias(h_done);
   unsigned char* k_kill = (unsigned char*)device_alias(h_fortkill);
   unsigned* k_events = (unsigned*)device_alias(h_events);
-  SF_HP(3);
   if (!k_actions) CUDA_TRY(cudaMemcpyAsync(h->d_actions, h_actions, n * 4, cudaMemcpyHostToDevice, sc));
-  const int slices = (render && !delta && n >= 2048) ? h->host_slices : 1;
+  const int slices = (render && !delta && n >= 2048) ? SF_HOST_STEP_SLICES : 1;
   const bool fused_delta = delta && per % 16 == 0;  // the blocks of the step kernel send their own frames' changes
   for (int k = 0; k < slices; k++) {
     const size_t e0 = n * k / slices, e1 = n * (k + 1) / slices;
@@ -1321,9 +1274,7 @@ extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_o
   if (h_done && !k_done) CUDA_TRY(cudaMemcpyAsync(h_done, h->d_done, n, cudaMemcpyDeviceToHost, sc));
   if (h_fortkill && !k_kill) CUDA_TRY(cudaMemcpyAsync(h_fortkill, h->d_kill, n, cudaMemcpyDeviceToHost, sc));
   if (h_events && !k_events) CUDA_TRY(cudaMemcpyAsync(h_events, h->d_events, n * 4, cudaMemcpyDeviceToHost, sc));
-  SF_HP(4);
   cudaError_t e1 = cudaStreamSynchronize(sc), e2 = (render && !delta) ? cudaStreamSynchronize(sx) : cudaSuccess;
-  SF_HP(5);
   if (e1 != cudaSuccess || e2 != cudaSuccess) {
     for (auto& m : h->mirrors) m.host = nullptr;
     return fail(SF_ERR_CUDA, std::string("sf_step_host: ") + cudaGetErrorString(e1 != cudaSuccess ? e1 : e2));
@@ -1437,32 +1388,6 @@ extern "C" int sf_episode_stats(sf_handle* h, long long* d_out, int reset, void*
   return SF_OK;
 }
 
-#ifdef SF_BARRIER_TIMING
-extern "C" int sf_barrier_cycles(unsigned long long* h_out, int reset) {
-  cudaDeviceSynchronize();
-  cudaMemcpyFromSymbol(h_out, sf_bar_cycles, sizeof(unsigned long long) * 16);
-  if (reset) { unsigned long long z[16] = {0}; cudaMemcpyToSymbol(sf_bar_cycles, z, sizeof(z)); }
-  return SF_OK;
-}
-#endif
-#ifdef SF_TIMELINE
-extern "C" int sf_timeline(unsigned long long* h_out) {  // [160][2][SF_TL_MAX]: (globaltimer ns << 8) | tag; zeroed after the read
-  cudaDeviceSynchronize();
-  cudaMemcpyFromSymbol(h_out, sf_tl, sizeof(unsigned long long) * 160 * 2 * SF_TL_MAX);
-  static unsigned long long z[160 * 2 * SF_TL_MAX];
-  cudaMemcpyToSymbol(sf_tl, z, sizeof(z));
-  return SF_TL_MAX;
-}
-#endif
-#ifdef SF_PHASE_TIMING
-extern "C" int sf_debug_cycles(unsigned long long* h_out, int reset) {
-  cudaDeviceSynchronize();
-  cudaMemcpyFromSymbol(h_out, sf_dbg_cycles, sizeof(unsigned long long) * 96);
-  if (reset) { unsigned long long z[96] = {0}; cudaMemcpyToSymbol(sf_dbg_cycles, z, sizeof(z)); }
-  return SF_OK;
-}
-#endif
-
 extern "C" int sf_set_glyph_masks(sf_handle* h, const uint8_t* h_alpha, const uint8_t* h_slot) {
   if (!h || (!h_alpha) != (!h_slot)) return fail(SF_ERR_INVALID, "handle is NULL, or only one of alpha / slot given");
   SfTables* nt = new SfTables();
@@ -1473,7 +1398,7 @@ extern "C" int sf_set_glyph_masks(sf_handle* h, const uint8_t* h_alpha, const ui
   if (ce == cudaSuccess) ce = cudaMemcpy((void*)h->dev.tab, nt, sizeof(SfTables), cudaMemcpyHostToDevice);
   if (ce == cudaSuccess) ce = cudaMemset(h->dev.expo_meta, 0, sizeof(uint2) * (size_t)h->dev.n_pad);  // cached resampled boxes may hold old digits
   if (ce == cudaSuccess) {
-    sf_pack_static_kernel<<<1, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_WARPS_PER_BLOCK)>>>(h->dev, const_cast<unsigned char*>(h->dev.static_image));
+    sf_pack_static_kernel<<<1, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS)>>>(h->dev, const_cast<unsigned char*>(h->dev.static_image));
     ce = cudaGetLastError();
     if (ce == cudaSuccess) ce = cudaDeviceSynchronize();
   }

@@ -30,10 +30,10 @@
 //    wireframe reaches into it, and from then on copied instead of recomputed (memos, not game state).
 #pragma once
 #include "sf_geom.h"
+#include "sf_probe.cuh"
 #include "sf_state.cuh"
 #include "sf_tables.h"
 
-#define SF_GROUP_ENVS_ 32   // == SF_GROUP_ENVS (defined below)
 #define SF_BATCH_QUADS 32
 #define SF_MAX_GROUPS 256    // (stroke, 8 sub-rows) work groups of one batch: 8 wireframes x <= 30, or 32 one-quad strokes x <= 8
 // A window is the INTER_AREA footprint closure of a box of at most 28x28 native pixels (the explosion sprite):
@@ -49,14 +49,10 @@
 #define SF_SPAN_NONE 0xFFFFFFFFu
 #define SF_QF_IRREGULAR 2    // quad flag: not a 2+2 edge split, test all four edges
 
-#ifndef SF_RENDER_WARPS
 #define SF_RENDER_WARPS 24   // warps per block (one block per SM): warp 0 steps, the others draw; 80 registers per thread
-#endif
 #define SF_FORT_LIST_SMEM 48                     // lit pixels of a fortress sprite kept in shared memory (the sprites have <= 42)
 #define SF_GROUP_ENVS 32                         // envs a block renders per tick: one per lane of the stepping warp
-#ifndef SF_STAGE_TICKS
-#define SF_STAGE_TICKS 2                         // consecutive ticks of the group drawn together in one stage (1 or 2)
-#endif
+#define SF_STAGE_TICKS 2                         // consecutive ticks of the group drawn together in one stage
 #define SF_STAGE_SLOTS (SF_GROUP_ENVS * SF_STAGE_TICKS)  // env slot = 32 * (tick within the stage) + lane of the env
 #define SF_ROUND_STROKES (8 * (SF_RENDER_WARPS - 1))  // strokes pooled per round: one batch of <= 8 per drawing warp (a round takes as many envs of the group as fit)
 // Block-wide pools of a round: one region (bounding box in native pixels + coverage cells) per visible stroke.
@@ -65,10 +61,10 @@
 #define SF_CELLS_SHIP 144
 #define SF_CELLS_MISSILE 49
 #define SF_CELLS_SHELL 49
-#ifndef SF_POOL_CELLS
 #define SF_POOL_CELLS 12288                      // 16-bit coverage cells
-#endif
 #define SF_POOL_REGIONS SF_ROUND_STROKES
+// B1 is latency bound (a batch of 8 strokes takes as long as one of 4), and every batch rounds its last pass of B3 up:
+#define SF_CHUNK_WARPS 12  // about 12 batches per round measured best (22: +1 % more passes; 8: the same)
 
 
 // per-warp shared memory (3.6 KB): the records of the batch being scan-converted; the window being composited
@@ -82,9 +78,6 @@ struct __align__(16) SfWarpSmem {
   int4 srec[SF_BATCH_QUADS];                //  512 B per stroke slot: {x0 | w<<8 | nq<<16 | quad0<<24, top (biased), first cell, s0 | s1<<16}
   unsigned short glist[SF_MAX_GROUPS];      //  512 B slot | k<<5 : sub-rows s0 + 8k .. s0 + 8k + 7 of a stroke
   int ngroups, pad0, pad1, pad2;
-#ifdef SF_PHASE_TIMING
-  long long prof_last, prof_pad;
-#endif
 };
 
 // what the renderer needs to know about one env of the block's group (written by the lane that stepped it)
@@ -138,7 +131,7 @@ struct __align__(16) SfStagePool {
   int4 region[SF_POOL_REGIONS];      // {x0, y0, w | h<<16, first cell | tag<<15 | colour<<16}
   short stroke_region[SF_ROUND_STROKES];  // region of stroke k of the round's list, -1: none
   int next_task, next_patch, nregions, cells_used;  // phase C work queue; base patches handed out; regions / cells opened
-  int base_ready, dbg_max_b, dbg_max_c, padq;       // the round's bulk copies have landed (set by the warp that issued them)
+  int base_ready, padq[3];                          // the round's bulk copies have landed (set by the warp that issued them)
   unsigned short exp_item0[SF_EXP_QUADS];   // build: copies of the y phase's per-quad table entries (SfExpPhase) for the sprite pass
   short exp_qxmin[SF_EXP_QUADS];
   signed char exp_row0[SF_EXP_QUADS];
@@ -152,9 +145,9 @@ struct __align__(16) SfStagePool {
 // with shared memory instead of issuing 7 global loads and 7 global stores per tick into the memory pipeline that the 23
 // drawing warps keep full (measured: 4.1 k + 7.0 k of its 27 k cycles per tick went there).
 struct __align__(16) SfStepSmem {
-  double2 pos[SF_GROUP_ENVS_], vel[SF_GROUP_ENVS_];
-  int4 q0[SF_GROUP_ENVS_], q1[SF_GROUP_ENVS_], q2[SF_GROUP_ENVS_], q3[SF_GROUP_ENVS_], st3[SF_GROUP_ENVS_];
-  unsigned d0[SF_GROUP_ENVS_], d1[SF_GROUP_ENVS_], d2[SF_GROUP_ENVS_];  // pending Stats increments (8-bit fields, flushed every 8 ticks)
+  double2 pos[SF_GROUP_ENVS], vel[SF_GROUP_ENVS];
+  int4 q0[SF_GROUP_ENVS], q1[SF_GROUP_ENVS], q2[SF_GROUP_ENVS], q3[SF_GROUP_ENVS], st3[SF_GROUP_ENVS];
+  unsigned d0[SF_GROUP_ENVS], d1[SF_GROUP_ENVS], d2[SF_GROUP_ENVS];  // pending Stats increments (8-bit fields, flushed every 8 ticks)
 };
 
 // per-block shared memory: copies of the static tables that every window touches, and the teams
@@ -176,9 +169,6 @@ struct __align__(16) SfBlockSmem {
   unsigned colour_white, padc[3];
   unsigned char exp_colour[SF_EXP_STROKES + 3];
   alignas(16) unsigned long long init_mbar, pad_mbar;  // the bulk copy of the static part above signals this mbarrier
-#ifdef SF_TIMELINE
-  int tl_n[4];
-#endif
   int next_group[SF_NEXT_GROUPS];  // rollout kernel: the block's next groups (written by warp 0 ahead of the drawing warps)
   SfStepSmem step;             // rollout kernel: the group's scalar state between ticks
   SfStagePrep prep[SF_PREP_SLOTS];
@@ -197,10 +187,6 @@ extern __shared__ __align__(16) unsigned char sf_smem_raw[];
 __device__ __forceinline__ SfBlockSmem& sf_block_smem() { return *reinterpret_cast<SfBlockSmem*>(sf_smem_raw); }
 __device__ __forceinline__ SfStagePrep& sf_prep(int sg) { return sf_block_smem().prep[sg]; }  // sg: the ring slot of the stage being drawn, handed down in a register
 __device__ __forceinline__ SfStagePool& sf_pool() { return sf_block_smem().pool; }
-#ifdef SF_BARRIER_TIMING  // tools/gpu_barrier_timing.py: cycles the warps spend at the barriers
-__device__ unsigned long long sf_bar_cycles[16];  // [8..15]: sections of the step (SF_ST in sf_step.cuh / sf_step_group); [0] wait for a prepared stage (drawing warps), [1] drawing-warp barriers, [2] wait for a free ring slot (warp 0)
-__device__ __forceinline__ void sf_bar_add(int k, long long t0) { if ((threadIdx.x & 31) == 0) atomicAdd(&sf_bar_cycles[k], (unsigned long long)(clock64() - t0)); }
-#endif
 // Hand-over of ring slot i between the two roles: two named hardware barriers of 768 threads each, full[i] = 3 + i and
 // empty[i] = 3 + SF_PREP_SLOTS + i (bar 0: __syncthreads, bar 2: the drawing warps).
 //  * full[i]: warp 0 ARRIVES when it has written the stage into slot i; the 23 drawing warps SYNC on it before they read it.
@@ -217,79 +203,26 @@ __device__ __forceinline__ void sf_stage_full_arrive(int sg) {  // warp 0
   asm volatile("bar.arrive %0, %1;" :: "r"(3 + sg), "r"(32 * SF_RENDER_WARPS) : "memory");
 }
 __device__ __forceinline__ void sf_stage_full_wait(int sg) {  // drawing warps
-#ifdef SF_BARRIER_TIMING
-  const long long t0 = clock64();
-#endif
+  SF_BT_BEGIN();
   asm volatile("bar.sync %0, %1;" :: "r"(3 + sg), "r"(32 * SF_RENDER_WARPS) : "memory");
-#ifdef SF_BARRIER_TIMING
-  sf_bar_add(0, t0);
-#endif
+  SF_BT(0);
 }
 __device__ __forceinline__ void sf_stage_empty_arrive(int sg) {  // drawing warps
   asm volatile("bar.arrive %0, %1;" :: "r"(3 + SF_PREP_SLOTS + sg), "r"(32 * SF_RENDER_WARPS) : "memory");
 }
 __device__ __forceinline__ void sf_stage_empty_wait(int sg) {  // warp 0
-#ifdef SF_BARRIER_TIMING
-  const long long t0 = clock64();
-#endif
+  SF_BT_BEGIN();
   asm volatile("bar.sync %0, %1;" :: "r"(3 + SF_PREP_SLOTS + sg), "r"(32 * SF_RENDER_WARPS) : "memory");
-#ifdef SF_BARRIER_TIMING
-  sf_bar_add(2, t0);
-#endif
+  SF_BT(2);
 }
 __device__ __forceinline__ void sf_render_sync() {  // the warps that draw: all but warp 0, which steps (named barrier 2)
-#ifdef SF_BARRIER_TIMING
-  const long long t0 = clock64();
-#endif
+  SF_BT_BEGIN();
   asm volatile("bar.sync 2, %0;" :: "r"(32 * (SF_RENDER_WARPS - 1)) : "memory");
-#ifdef SF_BARRIER_TIMING
-  sf_bar_add(1, t0);
-#endif
+  SF_BT(1);
 }
-#ifdef SF_TIMELINE  // tools/gpu_timeline.py: wall-clock marks (globaltimer, ns) of warps 0 and 1 of every block
-#define SF_TL_MAX 96
-__device__ unsigned long long sf_tl[160 * 2 * SF_TL_MAX];
-__device__ __forceinline__ void sf_tl_mark(int tag) {
-  const int warp = threadIdx.x >> 5;
-  if ((threadIdx.x & 31) == 0 && warp < 2 && blockIdx.x < 160) {
-    SfBlockSmem& B = sf_block_smem();
-    const int k = B.tl_n[warp]++;
-    if (k < SF_TL_MAX) {
-      unsigned long long g;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(g));
-      sf_tl[(blockIdx.x * 2 + warp) * SF_TL_MAX + k] = (g << 8) | (unsigned long long)tag;
-    }
-  }
-}
-#define SF_TL(tag) sf_tl_mark(tag)
-#else
-#define SF_TL(tag) ((void)0)
-#endif
 __device__ __forceinline__ SfWarpSmem& sf_warp_smem(int warp) { return reinterpret_cast<SfWarpSmem*>(sf_smem_raw + sizeof(SfBlockSmem))[warp]; }
 __device__ __forceinline__ SfWarpSmem& sf_my_smem() { return sf_warp_smem(threadIdx.x >> 5); }
 #define SF_RENDER_SMEM_BYTES(warps) (sizeof(SfBlockSmem) + sizeof(SfWarpSmem) * (warps))
-
-// debug build (-DSF_PHASE_TIMING): cycles of block 0 per phase / per code section (tools/gpu_phase_timing.py)
-#ifdef SF_PHASE_TIMING
-__device__ unsigned long long sf_dbg_cycles[96];  // 32..47: phase B busy cycles per warp, 48..63: phase C
-__device__ __forceinline__ void sf_prof(int k) {  // time since this warp's previous mark goes to bucket k
-  if ((threadIdx.x & 31) == 0 && blockIdx.x == 0) {
-    SfWarpSmem& W = sf_my_smem();
-    const long long now = clock64();
-    atomicAdd(&sf_dbg_cycles[k], (unsigned long long)(now - W.prof_last));
-    W.prof_last = now;
-  }
-}
-__device__ __forceinline__ void sf_prof_reset() { if ((threadIdx.x & 31) == 0 && blockIdx.x == 0) sf_my_smem().prof_last = clock64(); }
-__device__ __forceinline__ void sf_prof_count(int k, int v) { if ((threadIdx.x & 31) == 0 && blockIdx.x == 0) atomicAdd(&sf_dbg_cycles[k], (unsigned long long)v); }
-#define SF_PROF(k) sf_prof(k)
-#define SF_PROF_RESET() sf_prof_reset()
-#define SF_PROF_COUNT(k, v) sf_prof_count(k, v)
-#else
-#define SF_PROF(k) ((void)0)
-#define SF_PROF_RESET() ((void)0)
-#define SF_PROF_COUNT(k, v) ((void)0)
-#endif
 
 __device__ __forceinline__ int sf_warp_min(int v) {
 #pragma unroll
@@ -339,10 +272,7 @@ __device__ __forceinline__ void sf_block_smem_fill(const SfTables* T) {
 // slower next to the loads and the extra live state cost the drawing code registers: -3 % overall.)
 __device__ __forceinline__ void sf_block_smem_init(const unsigned char* image) {
   SfBlockSmem& B = sf_block_smem();
-#ifdef SF_TIMELINE
-  if ((threadIdx.x & 31) == 0 && (threadIdx.x >> 5) < 2) B.tl_n[threadIdx.x >> 5] = 0;
-  SF_TL(1);
-#endif
+  SF_TL_START();
   const unsigned bar = (unsigned)__cvta_generic_to_shared(&B.init_mbar);
   if (threadIdx.x == 0) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" :: "r"(bar) : "memory");
@@ -645,9 +575,7 @@ __device__ __noinline__ bool sf_composite(const SfTables* T, unsigned char* expc
   const unsigned core = rec.core;
   const int nx0 = SF_WIN_X0(win), ny0 = SF_WIN_Y0(win);
   const int nx1 = nx0 + SF_WIN_W(win), ny1 = ny0 + (int)SF_WIN_H(win);  // exclusive
-  SF_PROF(31);
   sf_patch_init(W, T, lane, win);
-  SF_PROF(22);
   // regions of this env (one per visible stroke, in draw order) that reach into the window
   int sr = -1, tag = SF_TAG_PROJECTILE;
   bool hit = false;
@@ -662,7 +590,6 @@ __device__ __noinline__ bool sf_composite(const SfTables* T, unsigned char* expc
   unsigned rmask = __ballot_sync(0xffffffffu, hit);
   const bool no_wireframe = rmask == 0u;
   const bool first_is_ship = __shfl_sync(0xffffffffu, tag, 0) == SF_TAG_SHIP;
-  SF_PROF(23);
   // ---- ship wireframe | ship explosion (draw.cpp:233-237) ----
   if (core & SF_CORE_SHIP_ALIVE) {
     if ((rmask & 1u) && first_is_ship) { const int s0r = __shfl_sync(0xffffffffu, sr, 0); sf_blend_region(s0r, win); rmask &= ~1u; }
@@ -694,7 +621,6 @@ __device__ __noinline__ bool sf_composite(const SfTables* T, unsigned char* expc
       __syncwarp();
     }
   }
-  SF_PROF(24);
   // ---- fortress wireframe | fortress explosion (draw.cpp:238-242) ----
   {
     const int fst = (core & SF_CORE_FORT_ALIVE) ? (int)((core >> SF_CORE_FANG_SHIFT) & 63u) : 36;
@@ -736,7 +662,6 @@ __device__ __noinline__ bool sf_composite(const SfTables* T, unsigned char* expc
       __syncwarp();
     }
   }
-  SF_PROF(25);
   // ---- missiles, then shells (draw.cpp:243-253): the env's strokes are stored in draw order ----
 #pragma unroll 1
   while (rmask) {
@@ -745,7 +670,6 @@ __device__ __noinline__ bool sf_composite(const SfTables* T, unsigned char* expc
     const int sq = __shfl_sync(0xffffffffu, sr, q);
     sf_blend_region(sq, win);
   }
-  SF_PROF(26);
   // ---- score digits (draw.cpp:160-173,267): "%07d" of (int)mPoints ----
   {
     const int ix0 = max(SF_TEXT_X0, nx0), ix1 = min(SF_TEXT_X0 + SF_TEXT_W, nx1);
@@ -827,10 +751,8 @@ __device__ __forceinline__ bool sf_window_orect(const SfTables* T, unsigned char
   const int win = nx0 | (ny0 << 8) | ((nx1 - nx0 + 1) << 16) | ((ny1 - ny0 + 1) << 24);
   const int orect = j0 | (i0 << 8) | ((j1 - j0 + 1) << 16) | ((i1 - i0 + 1) << 24);
   const bool pure = sf_composite(T, expcache, e, win, sg);
-  SF_PROF(27);
   sf_window_out(win, orect, obs84, pure ? cache : nullptr, corigin);
   __syncwarp();
-  SF_PROF(28);
   return pure && cache;
 }
 
@@ -839,7 +761,6 @@ __device__ __forceinline__ bool sf_window_orect(const SfTables* T, unsigned char
 // Every lane passes the description of ITS slot's stroke. Appends one region per visible stroke and publishes the
 // quads. Returns the region of the lane's slot (-1 invisible).
 __device__ __forceinline__ int sf_wire_geometry(SfWarpSmem& W, int lane, const SfTables* T, int kind, double px, double py, int angle) {
-  SF_PROF(31);
   const int slot = lane >> 2, line = lane & 3;
   SfQuadGeom G;
   G.ymin_g = 1 << 30; G.ymax_g = -(1 << 30); G.xmin = 1 << 30; G.xmax = -(1 << 30); G.split = 0; G.flags = 0;
@@ -868,13 +789,10 @@ __device__ __forceinline__ int sf_wire_geometry(SfWarpSmem& W, int lane, const S
     ymin_g = min(ymin_g, __shfl_xor_sync(0xffffffffu, ymin_g, o)); ymax_g = max(ymax_g, __shfl_xor_sync(0xffffffffu, ymax_g, o));
     xmin = min(xmin, __shfl_xor_sync(0xffffffffu, xmin, o)); xmax = max(xmax, __shfl_xor_sync(0xffffffffu, xmax, o));
   }
-  SF_PROF(16);
   // one region per slot, opened in slot order by the slot's first lane
   int rid = sf_open_regions(lane, line == 0 && kind >= 0, ymin_g, ymax_g, xmin, xmax, sf_block_smem().colour_white, kind == 0 ? SF_TAG_SHIP : SF_TAG_PROJECTILE);
-  SF_PROF(17);
   rid = __shfl_sync(0xffffffffu, rid, lane & ~3);
   sf_publish_quads(W, lane, G, has, rid, line == 0 && kind >= 0, slot, kind >= 0 ? sf_block_smem().wf_nlines[kind] : 0, ymin_g, ymax_g);
-  SF_PROF(18);
   return rid;
 }
 
@@ -1070,9 +988,6 @@ __device__ __forceinline__ void sf_scan_finish(SfStagePrep& Tm, int lane, int r_
     Tm.build_env2 = (Tm.build_env >= 0 && S.build_env2 >= 0 && S.build_env2 < S.r1) ? S.build_env2 : -1;
     // phase B1 hands the strokes out in equal batches of <= 8, one per drawing warp
     // (the last drawing warps get no batch: one of them issues the round's bulk copies instead, see sf_draw_stage)
-#ifndef SF_CHUNK_WARPS  // B1 is latency bound (a batch of 8 strokes takes as long as one of 4), and every batch rounds its last pass of B3 up:
-#define SF_CHUNK_WARPS 12  // about 12 batches per round measured best (22: +1 % more passes; 8: the same)
-#endif
     Tm.chunk = min(max((S.nst + SF_CHUNK_WARPS - 1) / SF_CHUNK_WARPS, 1), 8);
     Tm.netask = S.carry_task;
   }
@@ -1224,10 +1139,8 @@ __device__ __forceinline__ void sf_phase_strokes(const SfDev& D, SfBlockSmem& B,
   // drawing warp down: the geometry batches go to the first warps, so the two overlap.
   const int be = Tm.build_env;
   if (be >= 0) sf_phase_exp_items(D, be, lane, nw - 1 - wi, nw, sg);
-  SF_PROF(21);
   const int s = wi * chunk;
   if (s < nst) {
-    SF_PROF_COUNT(67, 1);
     const int slot = lane >> 2;
     const bool valid = slot < chunk && s + slot < nst;
     const int idx = s + slot;
@@ -1243,7 +1156,6 @@ __device__ __forceinline__ void sf_phase_strokes(const SfDev& D, SfBlockSmem& B,
     if (lane == 0) W.ngroups = 0;
   }
   sf_render_sync();  // every batch is published, the explosion items are done
-  SF_PROF(64);
   // B2, second half: the sprite (its stamp is visible to the stepping warp long before it looks at the next stage). A
   // round takes at most two explosions; they share the item lengths and the pixel masks, one after the other.
   if (be >= 0) {
@@ -1261,14 +1173,12 @@ __device__ __forceinline__ void sf_phase_strokes(const SfDev& D, SfBlockSmem& B,
 #pragma unroll
   for (int o = 1; o < 32; o <<= 1) { int t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
   const int total = __shfl_sync(0xffffffffu, incl, 31);
-  SF_PROF_COUNT(68, total);
 #pragma unroll 1
   for (int g = wi; g < total; g += nw) {
     const int owner = __popc(__ballot_sync(0xffffffffu, incl <= g));  // first warp whose inclusive count exceeds g
     const int first = __shfl_sync(0xffffffffu, incl - mine, owner);
     sf_accumulate_pass(owner + 1, (g - first) << 2);
   }
-  SF_PROF(20);
 }
 
 // phase C task t of this round: env tasks (quarters of explosion boxes, score strips) first, then one per stroke
@@ -1333,14 +1243,6 @@ __device__ __forceinline__ void sf_phase_native_tile(const SfDev& D, SfBlockSmem
   sf_for_rect(lane, pw, ph, [&](int c, int r) { dst[r * SF_NAT_W + c] = W.patch[r * SF_PATCH_STRIDE + c]; });
   __syncwarp();
 }
-
-#ifdef SF_PHASE_TIMING
-#define SF_TICK(k) do { if (threadIdx.x == 32 && blockIdx.x == 0) { long long now_ = clock64(); atomicAdd(&sf_dbg_cycles[k], (unsigned long long)(now_ - t_last_)); t_last_ = now_; } } while (0)
-#define SF_WTICK(k) do { if (lane == 0 && blockIdx.x == 0) { long long now_ = clock64(); atomicAdd(&sf_dbg_cycles[k], (unsigned long long)(now_ - w_last_)); w_last_ = now_; } } while (0)
-#else
-#define SF_TICK(k) ((void)0)
-#define SF_WTICK(k) ((void)0)
-#endif
 
 // warp 0, one env per lane, on the records of tick h of the stage being prepared in ring slot `cur`: a dead ship whose
 // explosion sprite is neither cached nor built by an earlier round gets it built in this round (bit 0); which quarters
@@ -1407,12 +1309,7 @@ template <class Prep>
 __device__ __forceinline__ void sf_prepare_first_round(const SfDev& D, SfBlockSmem& B, int sg, int lane, int t, int nt, SfFrameOut out, Prep prep) {
   SfStagePrep& Tm = B.prep[sg];
   const bool native = out.native != 0;
-#ifdef SF_BARRIER_TIMING
-  long long tb_ = clock64();
-#define SF_BT(k) do { sf_bar_add(k, tb_); tb_ = clock64(); } while (0)
-#else
-#define SF_BT(k) ((void)0)
-#endif
+  SF_BT_BEGIN();
   prep(t, Tm, 0);
   SF_BT(3);
   sf_publish_recs(D, B.prep, sg, lane, 0, native);
@@ -1425,7 +1322,6 @@ __device__ __forceinline__ void sf_prepare_first_round(const SfDev& D, SfBlockSm
   sf_gather_strokes(D, Tm, lane, 0);
   SF_BT(6);
   int nticks = 1;
-#if SF_STAGE_TICKS > 1
   if (nt > 1 && !Tm.more) {
     prep(t + 1, Tm, 1);
     SF_BT(3);
@@ -1438,7 +1334,6 @@ __device__ __forceinline__ void sf_prepare_first_round(const SfDev& D, SfBlockSm
     SF_BT(6);
     nticks = 2;
   }
-#endif
   if (lane == 0) Tm.nticks = nticks;
   __syncwarp();
   SF_BT(7);
@@ -1451,10 +1346,6 @@ __device__ __forceinline__ int sf_draw_stage(const SfDev& D, SfBlockSmem& B, SfW
   const int wi = warp - 1, nw = SF_RENDER_WARPS - 1;  // index among the drawing warps, and their number
   const SfStagePrep& Tm = B.prep[sg];
   SfStagePool& P = B.pool;
-#ifdef SF_PHASE_TIMING
-  long long t_last_ = clock64(), w_last_ = t_last_;
-  const int gwarp = warp;
-#endif
   const int r0 = Tm.r0, r1 = Tm.r1, nst = Tm.nstrokes;
   // ---- B: stroke tasks ----
   // The default observations of the round go out as bulk copies issued by ONE warp, the last drawing warp, one copy per
@@ -1467,9 +1358,7 @@ __device__ __forceinline__ int sf_draw_stage(const SfDev& D, SfBlockSmem& B, SfW
 #pragma unroll 1
     for (int e = r0 + lane; e < r1; e += 32) sf_env_base_issue(B, e, out, sg);
   }
-  SF_PROF_RESET();
   sf_phase_strokes(D, B, W, lane, wi, nw, nst, sg);
-  SF_PROF(69);
   if (!out.native) {
     // the copies were issued a whole phase ago: the issuer's wait returns at once, and so does everybody's look at the flag
     if (base_issuer) {
@@ -1480,7 +1369,6 @@ __device__ __forceinline__ int sf_draw_stage(const SfDev& D, SfBlockSmem& B, SfW
       while (*(volatile int*)&P.base_ready == 0) {}
     }
     __syncwarp();
-    SF_PROF(65);
     // first come first served: the warps leave the passes one pass apart, and a patch is as long as a pass
 #pragma unroll 1
     for (;;) {
@@ -1490,20 +1378,13 @@ __device__ __forceinline__ int sf_draw_stage(const SfDev& D, SfBlockSmem& B, SfW
       if (e >= r1) break;
       sf_env_base_patch(D, B, lane, e, out, sg);
     }
-    SF_PROF(66);
   }
-#ifdef SF_PHASE_TIMING
-  if (lane == 0 && blockIdx.x == 0) { atomicAdd(&sf_dbg_cycles[32 + (gwarp & 15)], (unsigned long long)(clock64() - w_last_)); atomicMax(&P.dbg_max_b, (int)(clock64() - w_last_)); }
-#endif
-  SF_WTICK(10);
   const int used = P.cells_used;  // final since the geometry barrier in sf_phase_strokes
   sf_render_sync();
-  SF_TICK(2); SF_WTICK(8);
   // the counters of B are not touched again in this stage: restart them for the next one (its B1 starts after every
   // drawing warp has synced on the next stage's full barrier)
   if (threadIdx.x == 32) { P.nregions = 0; P.cells_used = 0; P.next_patch = 0; P.base_ready = 0; }
   // ---- C: window tasks, handed out first come first served (env tasks first: the big ones) ----
-  SF_PROF_RESET();
   if (!out.native) {
     const int netask = Tm.netask;
 #pragma unroll 1
@@ -1512,23 +1393,12 @@ __device__ __forceinline__ int sf_draw_stage(const SfDev& D, SfBlockSmem& B, SfW
       if (lane == 0) t = atomicAdd(&P.next_task, 1);
       t = __shfl_sync(0xffffffffu, t, 0);
       if (t >= netask + nst) break;
-      SF_PROF(29);
       sf_phase_window(D, B, W, lane, t, netask, out, sg);
     }
   } else {
 #pragma unroll 1
     for (int t = wi; t < (r1 - r0) * 12; t += nw) sf_phase_native_tile(D, B, W, lane, r0 + t / 12, t % 12, out, sg);
   }
-#ifdef SF_PHASE_TIMING
-  if (lane == 0 && blockIdx.x == 0) { atomicAdd(&sf_dbg_cycles[48 + (gwarp & 15)], (unsigned long long)(clock64() - w_last_)); atomicMax(&P.dbg_max_c, (int)(clock64() - w_last_)); }
-  SF_WTICK(11);
-  if (threadIdx.x == 32 && blockIdx.x == 0) {
-    atomicAdd(&sf_dbg_cycles[71], (unsigned long long)P.dbg_max_b); atomicAdd(&sf_dbg_cycles[72], (unsigned long long)P.dbg_max_c);
-    atomicAdd(&sf_dbg_cycles[73], 1ull); atomicAdd(&sf_dbg_cycles[74], (unsigned long long)(Tm.netask + nst)); atomicAdd(&sf_dbg_cycles[75], (unsigned long long)Tm.netask);
-    atomicAdd(&sf_dbg_cycles[76], (unsigned long long)(Tm.build_env >= 0));
-    P.dbg_max_b = 0; P.dbg_max_c = 0;
-  }
-#endif
   return used;
 }
 

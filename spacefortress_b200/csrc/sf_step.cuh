@@ -8,14 +8,8 @@
 #include "sf_geom.h"
 #include "sf_state.cuh"
 #include "../../include/sf_b200.h"
+#include "sf_probe.cuh"
 
-#ifdef SF_BARRIER_TIMING  // sections of the step, cycles of warp 0 (tools/gpu_barrier_timing.py); sf_bar_add is in sf_render.cuh
-#define SF_ST_BEGIN() long long ts_ = clock64()
-#define SF_ST(k) do { __syncwarp(stmask_); sf_bar_add(k, ts_); ts_ = clock64(); } while (0)   // stmask_: the lanes that step an env
-#else
-#define SF_ST_BEGIN() ((void)0)
-#define SF_ST(k) ((void)0)
-#endif
 #define SF_TICK_MS 34        // ssf_env.py:61
 #define SF_GAME_TIME 180000  // configs.cpp:55,66,78,86
 #define SF_GAME_TICKS 5295   // first tick with mTime >= gameTime (game.cpp:487-489)
@@ -24,9 +18,6 @@ struct SfStepOut {
   int reward;       // shaped (train presets) or raw (test presets) integer reward
   unsigned events;  // SF_EV_*
   bool done, fort_kill;
-#ifdef SF_BARRIER_TIMING
-  unsigned sync_mask;
-#endif
   unsigned shell_vis;  // live shells further than 21 from the fortress after the tick (what draw.cpp:249-250 shows), bit per slot
 };
 
@@ -244,10 +235,7 @@ __device__ __forceinline__ int sf_first_free(unsigned mask, int n) {
 // One SSF_Env.step: keymask -> key events -> stepOneTick(34) -> shaping -> done -> auto-reset.
 __device__ inline void sf_env_step(const SfDev& D, const SfHot* T, int i, SfEnv& e, int keymask, bool autoreset, bool raw_reward, SfStepOut& out) {
   const int np = D.n_pad;
-#ifdef SF_BARRIER_TIMING
-  const unsigned stmask_ = out.sync_mask;
-#endif
-  SF_ST_BEGIN();
+  SF_ST_BEGIN(__activemask());  // the lanes that step an env
   float rew = 0.f;
   unsigned ev = 0;
   unsigned core = (unsigned)e.q0.x;

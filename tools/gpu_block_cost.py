@@ -1,9 +1,13 @@
-"""How well does the state of a block's envs predict the block's time in a T-step launch? (-DSF_TIMELINE build.)
-Least-squares fit of the per-block duration on per-block sums of env features taken BEFORE the launch.
-usage: SF_B200_LIB=build_variants/libsf_tl.so python tools/gpu_block_cost.py [n] [T] [gametype]"""
+"""How well does the state of a block's envs predict the block's time in a T-step launch? (-DSF_TIMELINE probe, built
+here as build_variants/libsf_tl.so.) Least-squares fit of the per-block duration on per-block sums of env features taken
+BEFORE the launch. usage: python tools/gpu_block_cost.py [n] [T] [gametype]"""
 import os, sys, ctypes as C
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+VARIANT = os.path.join(ROOT, "build_variants", "libsf_tl.so")
+os.environ["SF_B200_LIB"] = VARIANT  # read when the package is imported
+from spacefortress_b200 import build
+build.build(out=VARIANT, defs="-DSF_TIMELINE")
 import numpy as np, torch
 from spacefortress_b200 import SFVecEnv, _lib
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 4096

@@ -1,9 +1,14 @@
-"""Wall-clock timeline of the fused rollout (a -DSF_TIMELINE build, built here beforehand as build_variants/libsf_tl.so):
+"""Wall-clock timeline of the fused rollout (-DSF_TIMELINE probe, csrc/sf_probe.cuh; built here as build_variants/libsf_tl.so):
 marks of warp 0 (stepper) and warp 1 (a drawing warp) of every block: kernel entry, tables loaded, first stage prepared,
-arrival at / release from every stage hand-over (warp 0: wait for a free ring slot, warp 1: wait for a prepared stage), end. usage: SF_B200_LIB=build_variants/libsf_tl.so python tools/gpu_timeline.py [n] [T] [gametype]"""
+arrival at / release from every stage hand-over (warp 0: wait for a free ring slot, warp 1: wait for a prepared stage), end.
+usage: python tools/gpu_timeline.py [n] [T] [gametype]"""
 import os, sys, ctypes as C
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+VARIANT = os.path.join(ROOT, "build_variants", "libsf_tl.so")
+os.environ["SF_B200_LIB"] = VARIANT  # read when the package is imported
+from spacefortress_b200 import build
+build.build(out=VARIANT, defs="-DSF_TIMELINE")
 import numpy as np, torch
 from spacefortress_b200 import SFVecEnv, _lib
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 4096
