@@ -117,7 +117,7 @@ struct SfSched {
 };
 
 struct SfRollArgs {
-  int T, EB, ngroups, flags;  // EB = envs per group (<= 32), ngroups = ceil(n / EB)
+  int T, EB, ngroups, flags;  // EB = envs per group (<= 32), ngroups = ceil(n / EB): set by launch_rollout
   const int* actions;  // [T][n] or NULL
   unsigned action_seed;
   long long t0;
@@ -126,13 +126,12 @@ struct SfRollArgs {
   unsigned char* done;
   unsigned char* fortkill;
   unsigned* events;
-  SfSched* sched;      // NULL: static assignment (sf_render_kernel-like contiguous groups, no hand-out)
+  SfSched* sched;      // NULL: static assignment (sf_render_kernel-like contiguous groups, no hand-out); set by launch_rollout
   int env0, envn;      // the envs this launch steps: [env0, env0 + envn) (sf_step_host steps the slab in slices)
   // SF_FLAG_HOST_DELTA (sf_step_host, T == 1): every block ends by sending the changed granules of its own frames
   uint4* host_obs;     // device alias of the caller's page-locked observation buffer, or NULL
   uint4* mirror;       // device copy of what that buffer holds
   unsigned long long* delta_stats;
-  int delta_lanes;     // granule in 16-byte lanes
 };
 
 // ------------------------------------------------------------------------------------------------
@@ -239,45 +238,83 @@ __device__ __forceinline__ void sf_rollout_drawer(const SfDev& D, const SfRollAr
   }
 }
 
-// SF_FLAG_HOST_DELTA inside the kernel: the block compares the frames of its own groups (just written: L2) with the
-// mirror, 16 bytes per thread and four in flight, and stores the granules that differ straight into the host buffer
-// (posted writes across PCIe) and into the mirror. Blocks finish at different times (at T = 1 the median block is done
-// after ~70 % of the launch), so most of this and most of the PCIe traffic hides under the slower blocks; a separate
-// kernel (sf_host_delta_kernel, the fallback for frames that are not a multiple of 16 bytes) would start after the
-// slowest block.
+// ------------------------------------------------------------------------------------------------
+// SF_FLAG_HOST_DELTA (sf_step_host). Between two steps of an env only a few dozen bytes of its frame change (the moving
+// objects and now and then a score digit), so the frames are not copied: `mirror` is the device's copy of what the
+// caller's page-locked buffer holds, the new frames are compared with it, and the granules that differ are stored
+// straight into the host buffer (its device alias: posted writes across PCIe). The host buffer ends up identical to a
+// full copy; the traffic is ~600-1100 B per env-step instead of 7056.
+// ------------------------------------------------------------------------------------------------
+// 64 bytes = a host cache line: the host's memory system sees no partial-line writes (with 8 ranks writing at once up to
+// 19 % faster than 32-byte granules, DESIGN.md 7.4). A variant build may set 16 ... 256 bytes.
+#ifndef SF_DELTA_GRANULE
+#define SF_DELTA_GRANULE 64
+#endif
+#define SF_DELTA_LANES (SF_DELTA_GRANULE / 16)  // 16-byte chunks per granule: neighbouring lanes of one ballot
+static_assert(SF_DELTA_GRANULE == 16 || SF_DELTA_GRANULE == 32 || SF_DELTA_GRANULE == 64 || SF_DELTA_GRANULE == 128 || SF_DELTA_GRANULE == 256,
+              "SF_DELTA_GRANULE must be 16, 32, 64, 128 or 256 bytes (1 to 16 lanes of a warp's ballot)");
+
+// The 16-byte chunks [c0, c1) of the frames, shared by `nthreads` threads (a multiple of 32) of which this is `tid`, with
+// four loads in flight. The loop bound is the same for every lane, so whole warps take part in each ballot. Returns the
+// chunks this thread sent.
+__device__ __forceinline__ unsigned sf_host_delta_range(const uint4* cur, uint4* mirror, uint4* host, size_t c0, size_t c1, unsigned tid, unsigned nthreads) {
+  const unsigned gsh = (threadIdx.x & 31) & ~(unsigned)(SF_DELTA_LANES - 1);
+  unsigned sent = 0;
+#pragma unroll 1
+  for (size_t base = c0; base < c1; base += 4 * nthreads) {
+    uint4 a[4], b[4];
+#pragma unroll
+    for (int u = 0; u < 4; u++) {
+      const size_t i = base + u * nthreads + tid;
+      a[u] = b[u] = make_uint4(0, 0, 0, 0);
+      if (i < c1) { a[u] = __ldcg(cur + i); b[u] = __ldcg(mirror + i); }
+    }
+#pragma unroll
+    for (int u = 0; u < 4; u++) {
+      const size_t i = base + u * nthreads + tid;
+      const bool diff = (a[u].x != b[u].x) | (a[u].y != b[u].y) | (a[u].z != b[u].z) | (a[u].w != b[u].w);
+      const unsigned m = __ballot_sync(0xffffffffu, diff);
+      if (m == 0) continue;
+      if (i < c1 && ((m >> gsh) & ((1u << SF_DELTA_LANES) - 1u))) { host[i] = a[u]; sent++; }  // whole granules
+      if (diff) mirror[i] = a[u];
+    }
+  }
+  return sent;
+}
+
+// stats[0] += the bytes the warp sent (one atomic per warp); stats[1] counts the calls
+__device__ __forceinline__ void sf_host_delta_count(unsigned long long* stats, unsigned sent) {
+  for (int o = 16; o; o >>= 1) sent += __shfl_xor_sync(0xffffffffu, sent, o);
+  if ((threadIdx.x & 31) == 0 && sent) atomicAdd(&stats[0], (unsigned long long)sent * 16u);
+  if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&stats[1], 1ull);
+}
+
+// Inside the step kernel: each block compares the frames of its own groups, still in L2. Blocks finish at different
+// times (at T = 1 the median block is done after ~70 % of the launch), so most of this and most of the PCIe traffic
+// hides under the slower blocks; a separate kernel would start after the slowest block (DESIGN.md 7.4: 110 -> 105 us).
 __device__ __noinline__ void sf_block_host_delta(const SfDev& D, const SfRollArgs& A) {
-  const unsigned lane = threadIdx.x & 31;
-  const unsigned gmask = (1u << A.delta_lanes) - 1u, gsh = lane & ~(unsigned)(A.delta_lanes - 1);
-  const uint4* cur = reinterpret_cast<const uint4*>(A.obs);
   const size_t per16 = (size_t)(84 * 84) / 16;
   unsigned sent = 0;
 #pragma unroll 1
   for (int group = blockIdx.x; group < A.ngroups; group += gridDim.x) {
     const int env_lo = A.env0 + group * A.EB, env_hi = min(env_lo + A.EB, A.env0 + A.envn);
-    const size_t c1 = (size_t)env_hi * per16;
-#pragma unroll 1
-    for (size_t base = (size_t)env_lo * per16; base < c1; base += 4 * SF_BLOCK) {
-      uint4 a[4], b[4];
-#pragma unroll
-      for (int u = 0; u < 4; u++) {
-        const size_t i = base + u * SF_BLOCK + threadIdx.x;
-        a[u] = b[u] = make_uint4(0, 0, 0, 0);
-        if (i < c1) { a[u] = __ldcg(cur + i); b[u] = __ldcg(A.mirror + i); }
-      }
-#pragma unroll
-      for (int u = 0; u < 4; u++) {
-        const size_t i = base + u * SF_BLOCK + threadIdx.x;
-        const bool diff = (a[u].x != b[u].x) | (a[u].y != b[u].y) | (a[u].z != b[u].z) | (a[u].w != b[u].w);
-        const unsigned m = __ballot_sync(0xffffffffu, diff);
-        if (m == 0) continue;
-        if (i < c1 && ((m >> gsh) & gmask)) { A.host_obs[i] = a[u]; sent++; }
-        if (diff) A.mirror[i] = a[u];
-      }
-    }
+    sent += sf_host_delta_range(reinterpret_cast<const uint4*>(A.obs), A.mirror, A.host_obs, (size_t)env_lo * per16, (size_t)env_hi * per16,
+                                threadIdx.x, SF_BLOCK);
   }
-  for (int o = 16; o; o >>= 1) sent += __shfl_xor_sync(0xffffffffu, sent, o);
-  if (lane == 0 && sent) atomicAdd(&A.delta_stats[0], (unsigned long long)sent * 16u);
-  if (blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(&A.delta_stats[1], 1ull);
+  sf_host_delta_count(A.delta_stats, sent);
+}
+
+// The separate kernel, over the whole buffer: the only one for frames that are not a multiple of 16 bytes (native 92x90,
+// 8280 B per env). The last (bytes % 16) bytes go every time.
+__global__ void __launch_bounds__(256) sf_host_delta_kernel(const uint4* __restrict__ cur, uint4* __restrict__ mirror, uint4* __restrict__ host,
+                                                            size_t n16, int tail, unsigned long long* stats) {
+  const unsigned sent = sf_host_delta_range(cur, mirror, host, 0, n16, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
+  if (tail && blockIdx.x == 0 && threadIdx.x < (unsigned)tail) {
+    const size_t o = n16 * 16 + threadIdx.x;
+    const unsigned char v = reinterpret_cast<const unsigned char*>(cur)[o];
+    reinterpret_cast<unsigned char*>(host)[o] = v; reinterpret_cast<unsigned char*>(mirror)[o] = v;
+  }
+  sf_host_delta_count(stats, sent);
 }
 
 // (HOST_DELTA is a second instantiation, used by sf_step_host only: the register allocation of the plain kernel is
@@ -742,12 +779,34 @@ struct sf_handle {
   cudaStream_t host_compute, host_copy;  // sf_step_host: kernels of slice k + 1 overlap the device->host copy of slice k
   cudaEvent_t host_ev[SF_HOST_STEP_SLICES];
   // SF_FLAG_HOST_DELTA: device copy of what the caller's page-locked h_obs holds, so that only changed bytes cross PCIe
-  struct Mirror { const void* host; unsigned char* d; size_t cap, bytes; unsigned long long used; };
+  struct Mirror { const void* host; unsigned char* d; size_t cap, bytes; unsigned long long used; };  // host: the buffer it describes, or NULL
   Mirror mirrors[SF_MAX_MIRRORS];     // one per host buffer (a caller may rotate a few buffers); least recently used goes first
   unsigned long long mirror_clock;
   unsigned long long* d_delta_stats;  // [0] observation bytes written to the host by delta calls, [1] delta calls
   unsigned long long full_calls;      // calls that sent whole frames (first call, new buffer, flag absent)
-  int delta_lanes;                    // granule of the delta updates in 16-byte lanes (4; SF_DELTA_GRANULE = 16 ... 256 bytes overrides)
+
+  // The mirror of host buffer `host`, with room for `bytes`: its own entry, else a free one, else the least recently used
+  // one. An entry that is taken over or grown describes no buffer until whole frames have been copied into it.
+  int mirror_for(const void* host, size_t bytes, Mirror** out) {
+    Mirror* mir = nullptr;
+    for (auto& m : mirrors) if (m.host == host) mir = &m;
+    if (!mir) {
+      for (auto& m : mirrors) if (!mir || (mir->host && (!m.host || m.used < mir->used))) mir = &m;
+      mir->host = nullptr;
+    }
+    if (bytes > mir->cap) {
+      if (mir->d) { cudaFree(mir->d); mir->d = nullptr; mir->cap = 0; }
+      mir->host = nullptr;
+      CUDA_TRY(cudaMalloc(&mir->d, bytes));
+      mir->cap = bytes;
+    }
+    mir->used = ++mirror_clock;
+    *out = mir;
+    return SF_OK;
+  }
+  void forget_mirrors(const void* host) {  // NULL: every buffer; the device memory is kept for the next buffer
+    for (auto& m : mirrors) if (m.host == host || !host) m.host = nullptr;
+  }
 };
 
 extern "C" const char* sf_last_error(void) { return g_err.c_str(); }
@@ -1070,16 +1129,16 @@ extern "C" int sf_render(sf_handle* h, uint8_t* d_obs, int flags, void* stream) 
   return launch_render(h, d_obs, flags, nullptr, (cudaStream_t)stream);
 }
 
-static int launch_rollout(sf_handle* h, const SfRollArgs& a, cudaStream_t st) {
+// The launch shape (EB, ngroups, sched) is derived here; callers set the other fields.
+static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st) {
   const SfDev& d = h->dev;
   bool render = (a.flags & SF_FLAG_RENDER) && a.obs;
   if (render) {
-    SfRollArgs b = a;
     int blocks;
-    group_shape(h, b.envn, &b.EB, &b.ngroups, &blocks);
-    b.sched = (a.env0 == 0 && a.envn == d.n && !a.host_obs) ? h->d_sched : nullptr;  // slices of the slab (sf_step_host), in-kernel delta: static groups
-    if (b.host_obs) sf_rollout_kernel<true><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, b);
-    else sf_rollout_kernel<false><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, b);
+    group_shape(h, a.envn, &a.EB, &a.ngroups, &blocks);
+    a.sched = (a.env0 == 0 && a.envn == d.n && !a.host_obs) ? h->d_sched : nullptr;  // slices of the slab (sf_step_host), in-kernel delta: static groups
+    if (a.host_obs) sf_rollout_kernel<true><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
+    else sf_rollout_kernel<false><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
   } else {
     sf_step_only_kernel<<<(a.envn + 127) / 128, 128, 0, st>>>(d, a);
   }
@@ -1092,8 +1151,8 @@ extern "C" int sf_step(sf_handle* h, const int32_t* d_actions, uint8_t* d_obs, i
   if (!h || !d_actions) return fail(SF_ERR_INVALID, "handle or actions is NULL");
   CUDA_TRY(cudaSetDevice(h->device));
   SfRollArgs a = {};
-  a.T = 1; a.EB = 1; a.ngroups = 0; a.flags = flags; a.actions = d_actions; a.action_seed = 0; a.t0 = 0;
-  a.obs = d_obs; a.reward = d_reward; a.done = d_done; a.fortkill = d_fortkill; a.events = d_events; a.sched = nullptr; a.env0 = 0; a.envn = h->dev.n;
+  a.T = 1; a.flags = flags; a.actions = d_actions;
+  a.obs = d_obs; a.reward = d_reward; a.done = d_done; a.fortkill = d_fortkill; a.events = d_events; a.envn = h->dev.n;
   return launch_rollout(h, a, (cudaStream_t)stream);
 }
 
@@ -1102,52 +1161,13 @@ extern "C" int sf_rollout(sf_handle* h, int T, const int32_t* d_actions, uint32_
   if (!h || T <= 0) return fail(SF_ERR_INVALID, "handle is NULL or T <= 0");
   CUDA_TRY(cudaSetDevice(h->device));
   SfRollArgs a = {};
-  a.T = T; a.EB = 1; a.ngroups = 0; a.flags = flags; a.actions = d_actions; a.action_seed = action_seed; a.t0 = t0;
-  a.obs = d_obs; a.reward = d_reward; a.done = d_done; a.fortkill = d_fortkill; a.events = nullptr; a.sched = nullptr; a.env0 = 0; a.envn = h->dev.n;
+  a.T = T; a.flags = flags; a.actions = d_actions; a.action_seed = action_seed; a.t0 = t0;
+  a.obs = d_obs; a.reward = d_reward; a.done = d_done; a.fortkill = d_fortkill; a.envn = h->dev.n;
   return launch_rollout(h, a, (cudaStream_t)stream);
 }
 
 extern "C" int sf_synthetic_action(uint32_t action_seed, long long global_env, long long t, int num_actions) {
   return sf_hash_action(action_seed, (unsigned long long)global_env, (unsigned long long)t, num_actions);
-}
-
-// SF_FLAG_HOST_DELTA. Between two steps of an env only a few dozen bytes of its frame change (the moving objects and
-// now and then a score digit), so the frames are not copied: `mirror` is the device's copy of what the caller's
-// page-locked buffer holds, and this kernel compares the new frames with it 16 bytes per thread and stores, straight
-// into the host buffer (its device alias: posted writes across PCIe), the granules (64 bytes: a host cache line) that differ. The host buffer
-// ends up identical to a full copy; the traffic is ~600-1100 B per env-step instead of 7056.
-template <int LANES>  // lanes (of 16 bytes) per granule
-__global__ void __launch_bounds__(256) sf_host_delta_kernel(const uint4* __restrict__ cur, uint4* __restrict__ mirror, uint4* __restrict__ host,
-                                                             size_t n16, int tail, unsigned long long* stats) {
-  __shared__ unsigned block_sent;
-  if (threadIdx.x == 0) block_sent = 0;
-  __syncthreads();
-  const unsigned lane = threadIdx.x & 31;
-  const size_t stride = (size_t)gridDim.x * blockDim.x;
-  const size_t n16_warp = (n16 + 31) & ~(size_t)31;  // whole warps stay in the loop for the ballot
-  unsigned sent = 0;
-  for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n16_warp; i += stride) {
-    const bool in = i < n16;
-    uint4 a = make_uint4(0, 0, 0, 0), b = a;
-    if (in) { a = __ldcg(cur + i); b = __ldcg(mirror + i); }
-    const bool diff = (a.x != b.x) | (a.y != b.y) | (a.z != b.z) | (a.w != b.w);
-    const unsigned m = __ballot_sync(0xffffffffu, diff);
-    if (m == 0) continue;
-    if (in && ((m >> (lane & ~(unsigned)(LANES - 1))) & ((1u << LANES) - 1u))) { host[i] = a; sent++; }  // whole granules
-    if (diff) mirror[i] = a;
-  }
-  if (tail && blockIdx.x == 0 && threadIdx.x < (unsigned)tail) {  // the last (bytes % 16) bytes go every time
-    const size_t o = n16 * 16 + threadIdx.x;
-    const unsigned char v = reinterpret_cast<const unsigned char*>(cur)[o];
-    reinterpret_cast<unsigned char*>(host)[o] = v; reinterpret_cast<unsigned char*>(mirror)[o] = v;
-  }
-  for (int o = 16; o; o >>= 1) sent += __shfl_xor_sync(0xffffffffu, sent, o);
-  if (lane == 0 && sent) atomicAdd(&block_sent, sent);
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    if (block_sent) atomicAdd(&stats[0], (unsigned long long)block_sent * 16u);
-    if (blockIdx.x == 0) atomicAdd(&stats[1], 1ull);
-  }
 }
 
 static int ensure_staging(sf_handle* h, size_t obs_bytes) {
@@ -1156,8 +1176,6 @@ static int ensure_staging(sf_handle* h, size_t obs_bytes) {
     CUDA_TRY(cudaStreamCreateWithFlags(&h->host_compute, cudaStreamNonBlocking));
     CUDA_TRY(cudaStreamCreateWithFlags(&h->host_copy, cudaStreamNonBlocking));
     for (int k = 0; k < SF_HOST_STEP_SLICES; k++) CUDA_TRY(cudaEventCreateWithFlags(&h->host_ev[k], cudaEventDisableTiming));
-    h->delta_lanes = 4;  // 64 bytes: whole host cache lines (no partial-line writes in the host's memory system)
-    if (const char* ov = getenv("SF_DELTA_GRANULE")) { int v = atoi(ov); if (v == 16 || v == 32 || v == 64 || v == 128 || v == 256) h->delta_lanes = v / 16; }  // tuning knob
   }
   if (!h->d_actions) {
     CUDA_TRY(cudaMalloc(&h->d_actions, n * 4)); CUDA_TRY(cudaMalloc(&h->d_reward, n * 4));
@@ -1193,44 +1211,33 @@ extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_o
                             uint8_t* h_fortkill, uint32_t* h_events, int flags) {
   if (!h || !h_actions) return fail(SF_ERR_INVALID, "handle or actions is NULL");
   CUDA_TRY(cudaSetDevice(h->device));
-  size_t n = (size_t)h->dev.n;
-  size_t per = (flags & SF_FLAG_NATIVE_OBS) ? (size_t)SF_NAT_H * SF_NAT_W : (size_t)84 * 84;
-  bool render = (flags & SF_FLAG_RENDER) && h_obs;
-  int rc = ensure_staging(h, render ? n * per : 0);
+  const size_t n = (size_t)h->dev.n;
+  const size_t per = (flags & SF_FLAG_NATIVE_OBS) ? (size_t)SF_NAT_H * SF_NAT_W : (size_t)84 * 84, obs_bytes = n * per;
+  const bool render = (flags & SF_FLAG_RENDER) && h_obs;
+  int rc = ensure_staging(h, render ? obs_bytes : 0);
   if (rc) return rc;
   // Synchronous, on the handle's own streams. Whole-frame mode: the slab is stepped in slices of consecutive envs, the
   // kernel of slice k + 1 runs while the frames of slice k cross PCIe (one cudaMemcpyAsync per buffer and slice), so only
-  // the first slice's kernel is exposed. Delta mode: one launch, no copies (see sf_block_host_delta). Work the caller has queued on OTHER streams for this handle must be complete (the Python
-  // wrapper synchronises its stream first); everything queued here is complete on return.
+  // the first slice's kernel is exposed. Delta mode: one launch, no copies (see sf_block_host_delta). Work the caller has
+  // queued on OTHER streams for this handle must be complete (the Python wrapper synchronises its stream first);
+  // everything queued here is complete on return.
   cudaStream_t sc = h->host_compute, sx = h->host_copy;
   // SF_FLAG_HOST_DELTA: h_obs is page-locked and still holds what the previous call with this flag wrote there
   uint4* host_alias = nullptr;
   sf_handle::Mirror* mir = nullptr;
-  const size_t obs_bytes = n * per;
   const bool want_delta = render && (flags & SF_FLAG_HOST_DELTA);
   if (want_delta) {
     host_alias = reinterpret_cast<uint4*>(device_alias(h_obs));
     if (!host_alias) return fail(SF_ERR_INVALID, "SF_FLAG_HOST_DELTA needs a page-locked h_obs (sf_host_alloc, cudaHostAlloc, cudaHostRegister)");
     if (((uintptr_t)h_obs | (uintptr_t)host_alias) & 15) return fail(SF_ERR_INVALID, "SF_FLAG_HOST_DELTA needs a 16-byte aligned h_obs");
-    for (auto& m : h->mirrors) if (m.host == h_obs) mir = &m;
-    if (!mir) {  // a buffer seen for the first time: a free entry, else the least recently used one
-      for (auto& m : h->mirrors) if (!mir || (mir->host && (!m.host || m.used < mir->used))) mir = &m;
-      mir->host = nullptr;
-    }
-    if (obs_bytes > mir->cap) {
-      if (mir->d) { cudaFree(mir->d); mir->d = nullptr; mir->cap = 0; }
-      mir->host = nullptr;
-      CUDA_TRY(cudaMalloc(&mir->d, obs_bytes));
-      mir->cap = obs_bytes;
-    }
-    mir->used = ++h->mirror_clock;
+    if ((rc = h->mirror_for(h_obs, obs_bytes, &mir))) return rc;
     if (!h->d_delta_stats) {
       CUDA_TRY(cudaMalloc(&h->d_delta_stats, 16));
       CUDA_TRY(cudaMemset(h->d_delta_stats, 0, 16));
     }
   }
   const bool delta = want_delta && mir->host == h_obs && mir->bytes == obs_bytes;
-  flags &= ~SF_FLAG_HOST_DELTA;
+  const bool fused_delta = delta && per % 16 == 0;  // the blocks of the step kernel send their own frames' changes
   CUDA_TRY(cudaStreamSynchronize(cudaStreamLegacy));  // calls made with stream == NULL (sf_reset, sf_seed ...) come first
   // page-locked actions / rewards / dones / kills / events are read and written in place by the kernel
   const int* k_actions = (const int*)device_alias(h_actions);
@@ -1239,17 +1246,17 @@ extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_o
   unsigned char* k_kill = (unsigned char*)device_alias(h_fortkill);
   unsigned* k_events = (unsigned*)device_alias(h_events);
   if (!k_actions) CUDA_TRY(cudaMemcpyAsync(h->d_actions, h_actions, n * 4, cudaMemcpyHostToDevice, sc));
+  flags &= ~SF_FLAG_HOST_DELTA;
+  SfRollArgs a = {};
+  a.T = 1; a.flags = render ? flags : (flags & ~SF_FLAG_RENDER);
+  a.actions = k_actions ? k_actions : h->d_actions;
+  a.obs = render ? h->d_obs : nullptr; a.reward = k_reward ? k_reward : h->d_reward; a.done = k_done ? k_done : h->d_done;
+  a.fortkill = k_kill ? k_kill : h->d_kill; a.events = k_events ? k_events : h->d_events;
+  if (fused_delta) { a.host_obs = host_alias; a.mirror = reinterpret_cast<uint4*>(mir->d); a.delta_stats = h->d_delta_stats; }
   const int slices = (render && !delta && n >= 2048) ? SF_HOST_STEP_SLICES : 1;
-  const bool fused_delta = delta && per % 16 == 0;  // the blocks of the step kernel send their own frames' changes
   for (int k = 0; k < slices; k++) {
     const size_t e0 = n * k / slices, e1 = n * (k + 1) / slices;
-    SfRollArgs a = {};
-    a.T = 1; a.EB = 1; a.ngroups = 0; a.flags = render ? flags : (flags & ~SF_FLAG_RENDER); a.action_seed = 0; a.t0 = 0;
-    a.actions = k_actions ? k_actions : h->d_actions;
-    a.obs = render ? h->d_obs : nullptr; a.reward = k_reward ? k_reward : h->d_reward; a.done = k_done ? k_done : h->d_done;
-    a.fortkill = k_kill ? k_kill : h->d_kill; a.events = k_events ? k_events : h->d_events; a.sched = nullptr;
     a.env0 = (int)e0; a.envn = (int)(e1 - e0);
-    if (fused_delta) { a.host_obs = host_alias; a.mirror = reinterpret_cast<uint4*>(mir->d); a.delta_stats = h->d_delta_stats; a.delta_lanes = h->delta_lanes; }
     rc = launch_rollout(h, a, sc);
     if (rc) { cudaStreamSynchronize(sc); cudaStreamSynchronize(sx); return rc; }
     if (render && !delta) {
@@ -1261,9 +1268,8 @@ extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_o
   if (delta && !fused_delta) {
     const size_t n16 = obs_bytes / 16;
     const int blocks = (int)std::min<size_t>((n16 + 255) / 256, (size_t)h->num_sms * 8);
-    auto kern = h->delta_lanes == 1 ? sf_host_delta_kernel<1> : (h->delta_lanes >= 4 ? sf_host_delta_kernel<4> : sf_host_delta_kernel<2>);
-    kern<<<std::max(blocks, 1), 256, 0, sc>>>(reinterpret_cast<const uint4*>(h->d_obs), reinterpret_cast<uint4*>(mir->d), host_alias,
-                                              n16, (int)(obs_bytes & 15), h->d_delta_stats);
+    sf_host_delta_kernel<<<std::max(blocks, 1), 256, 0, sc>>>(reinterpret_cast<const uint4*>(h->d_obs), reinterpret_cast<uint4*>(mir->d), host_alias,
+                                                              n16, (int)(obs_bytes & 15), h->d_delta_stats);
     CUDA_TRY(cudaGetLastError());
   } else if (want_delta) {  // whole frames went out: from here on the mirror describes this buffer
     CUDA_TRY(cudaMemcpyAsync(mir->d, h->d_obs, obs_bytes, cudaMemcpyDeviceToDevice, sc));
@@ -1276,7 +1282,7 @@ extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_o
   if (h_events && !k_events) CUDA_TRY(cudaMemcpyAsync(h_events, h->d_events, n * 4, cudaMemcpyDeviceToHost, sc));
   cudaError_t e1 = cudaStreamSynchronize(sc), e2 = (render && !delta) ? cudaStreamSynchronize(sx) : cudaSuccess;
   if (e1 != cudaSuccess || e2 != cudaSuccess) {
-    for (auto& m : h->mirrors) m.host = nullptr;
+    h->forget_mirrors(nullptr);
     return fail(SF_ERR_CUDA, std::string("sf_step_host: ") + cudaGetErrorString(e1 != cudaSuccess ? e1 : e2));
   }
   return SF_OK;
@@ -1284,7 +1290,7 @@ extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_o
 
 extern "C" int sf_host_forget(sf_handle* h, const void* h_obs) {
   if (!h) return fail(SF_ERR_INVALID, "handle is NULL");
-  for (auto& m : h->mirrors) if (m.host == h_obs || !h_obs) m.host = nullptr;  // the device memory is kept for the next buffer
+  h->forget_mirrors(h_obs);
   return SF_OK;
 }
 

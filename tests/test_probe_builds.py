@@ -1,12 +1,13 @@
-"""CPU: the probe builds of csrc/sf_probe.cuh still compile, each exports its reader, and the product library exports
-neither (the probes are build variants, never part of the product)."""
+"""CPU: the variant builds the tools make still compile. Each probe of csrc/sf_probe.cuh exports its reader and the
+product library exports neither (the probes are build variants, never part of the product); a build with another
+granule of the host-buffer delta updates exports the whole C-ABI."""
 import ctypes as C
 import os
 from concurrent.futures import ThreadPoolExecutor
 
 import pytest
 
-from spacefortress_b200 import build
+from spacefortress_b200 import _lib, build
 
 PROBES = {"-DSF_BARRIER_TIMING": "sf_barrier_cycles", "-DSF_TIMELINE": "sf_timeline"}
 
@@ -33,3 +34,15 @@ def test_probe_variants_build_and_export_their_readers(nvcc, tmp_path):
     product = C.CDLL(build.build())
     for name in PROBES.values():
         assert not hasattr(product, name), name
+
+
+def test_delta_granule_is_a_build_define(nvcc, tmp_path):
+    """The granule of the host-buffer delta updates is fixed when the library is built: a variant with another granule
+    (tools/gpu_host_step_ranks.py) compiles and exports the whole C-ABI, and the product library has no run-time knob
+    that names it."""
+    out = str(tmp_path / "libsf_granule32.so")
+    build.build(out=out, defs="-DSF_DELTA_GRANULE=32")
+    L = C.CDLL(out)
+    assert [s for s in _lib.EXPORTED_SYMBOLS if not hasattr(L, s)] == []
+    with open(build.build(), "rb") as f:
+        assert b"SF_DELTA_GRANULE" not in f.read()

@@ -1,5 +1,6 @@
 """Where the time of one host-buffer step (SFVecEnv.step(np.ndarray) -> sf_step_host) goes: the Python wrapper, the C call,
-and (run it under `ncu --metrics gpu__time_duration.sum`) the two kernels. usage: python tools/gpu_host_step_breakdown.py [n] [steps]"""
+a state-only C call and the device path's kernel. `native`: 92x90 frames, whose delta updates take the separate kernel.
+usage: python tools/gpu_host_step_breakdown.py [n] [steps] [native]"""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np, torch
@@ -7,8 +8,9 @@ from spacefortress_b200 import SFVecEnv, _lib
 
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 4096
 steps = int(sys.argv[2]) if len(sys.argv) > 2 else 300
+native = sys.argv[3:4] == ["native"]
 for gt in ("autoturn", "youturn"):
-    env = SFVecEnv(gt, num_envs=n, device=0)
+    env = SFVecEnv(gt, num_envs=n, device=0, native_obs=native)
     env.reset()
     env.rollout(400, want=("reward",), action_seed=7)
     torch.cuda.synchronize()
@@ -39,12 +41,12 @@ for gt in ("autoturn", "youturn"):
     for t in range(steps):
         env.step(a_dev[5 + t])
     e1.record(); torch.cuda.synchronize()
-    print("%s n=%d: wrapper %.1f us/step (%.1f M env-steps/s), C call %.1f us, state-only C call %.1f us, device-path kernel %.1f us, obs bytes/env-step %.0f"
-          % (gt, n, 1e6 * t_wrap, n / t_wrap / 1e6, 1e6 * t_call, 1e6 * t_state, 1e3 * e0.elapsed_time(e1) / steps, (s1[0] - s0[0]) / steps / n), flush=True)
+    print("%s%s n=%d: wrapper %.1f us/step (%.1f M env-steps/s), C call %.1f us, state-only C call %.1f us, device-path kernel %.1f us, obs bytes/env-step %.0f"
+          % (gt, " native" if native else "", n, 1e6 * t_wrap, n / t_wrap / 1e6, 1e6 * t_call, 1e6 * t_state, 1e3 * e0.elapsed_time(e1) / steps, (s1[0] - s0[0]) / steps / n), flush=True)
     env.close()
     for mode, what in (("ring", "SubprocVecEnv look-alike's default: fresh read-only arrays from a rotation of page-locked buffers"),
                        (True, "private writable copies every step")):
-        lit = SFVecEnv(gt, num_envs=n, device=0, copy_outputs=mode)
+        lit = SFVecEnv(gt, num_envs=n, device=0, native_obs=native, copy_outputs=mode)
         lit.reset()
         for t in range(5):
             o, r, d, i = lit.step(acts[t])   # (bound like in the loop below: the ring's second buffer is allocated here)
