@@ -10,10 +10,12 @@
 //                               Groups beyond the first 148 are handed out first come first served (SfSched); between
 //                               the ticks of a launch the group's scalars stay in shared memory (SfStepSmem); the static
 //                               tables arrive as one bulk copy of a per-handle image (sf_pack_static_kernel).
+//                               Three instantiations (SfRollMode): step, step with host delta (sf_step_host), and draw
+//                               (sf_render, sf_reset: warp 0 loads the current state instead of stepping it).
 //   sf_step_only_kernel         state-only variant (render off), one env per thread.
 //   sf_features_kernel          the feature observation types of ssf_env.py:95-157, one env per thread.
 //   sf_policy_input_kernel      4-frame stack -> the policy's first-layer input (bf16 or fp32, space-to-depth NHWC).
-//   sf_reset_kernel / sf_seed_kernel / sf_render_kernel / sf_get_state_kernel / sf_set_state_kernel / sf_pack_static_kernel
+//   sf_reset_kernel / sf_seed_kernel / sf_get_state_kernel / sf_set_state_kernel / sf_pack_static_kernel
 #include <cuda_runtime.h>
 #include <stdio.h>
 #include <stdlib.h>
@@ -126,13 +128,31 @@ struct SfRollArgs {
   unsigned char* done;
   unsigned char* fortkill;
   unsigned* events;
-  SfSched* sched;      // NULL: static assignment (sf_render_kernel-like contiguous groups, no hand-out); set by launch_rollout
+  SfSched* sched;      // NULL: static assignment (block b owns groups b, b + gridDim.x, ...; no hand-out); set by launch_rollout
   int env0, envn;      // the envs this launch steps: [env0, env0 + envn) (sf_step_host steps the slab in slices)
   // SF_FLAG_HOST_DELTA (sf_step_host, T == 1): every block ends by sending the changed granules of its own frames
   uint4* host_obs;     // device alias of the caller's page-locked observation buffer, or NULL
   uint4* mirror;       // device copy of what that buffer holds
   unsigned long long* delta_stats;
+  const unsigned char* draw_mask;  // SF_ROLL_DRAW: the envs to draw (NULL: all); the others' frames are not written
 };
+enum SfRollMode { SF_ROLL_STEP, SF_ROLL_STEP_HOST_DELTA, SF_ROLL_DRAW };
+// ticks per group, for both roles of a launch: a draw is the one frame of the current state
+template <int MODE>
+__device__ __forceinline__ int sf_roll_ticks(const SfRollArgs& A) { return MODE == SF_ROLL_DRAW ? 1 : A.T; }
+
+// one tick of one env (both step kernels; H: the step's tables): its action, the step, the step's outputs
+__device__ __forceinline__ void sf_tick_env(const SfDev& D, const SfHot* H, const SfRollArgs& A, int env, int t, bool autoreset, SfEnv& e, SfStepOut& o) {
+  int a = A.actions ? A.actions[(size_t)t * D.n + env]
+                    : sf_hash_action(A.action_seed, (unsigned long long)(D.first_global_env + env), (unsigned long long)(A.t0 + t), D.num_actions);
+  int km = (A.flags & SF_FLAG_ACTIONS_ARE_KEYMASKS) ? (a & 15) : D.keymask_of_action[min(max(a, 0), D.num_actions - 1)];
+  sf_env_step(D, H, env, e, km, autoreset, (A.flags & SF_FLAG_RAW_REWARD) != 0, o);
+  size_t oi = (size_t)t * D.n + env;
+  if (A.reward) A.reward[oi] = o.reward;
+  if (A.done) A.done[oi] = o.done;
+  if (A.fortkill) A.fortkill[oi] = o.fort_kill;
+  if (A.events) A.events[oi] = o.events;
+}
 
 // ------------------------------------------------------------------------------------------------
 // fused step + render
@@ -162,16 +182,8 @@ __device__ __noinline__ void sf_step_group(const SfDev& D, const SfRollArgs& A, 
     }
     SF_ST_USE(e.q0.x, e.q0.y);
     SF_ST(8);
-    int a = A.actions ? A.actions[(size_t)t * D.n + env]
-                      : sf_hash_action(A.action_seed, (unsigned long long)(D.first_global_env + env), (unsigned long long)(A.t0 + t), D.num_actions);
-    int km = (A.flags & SF_FLAG_ACTIONS_ARE_KEYMASKS) ? (a & 15) : D.keymask_of_action[min(max(a, 0), D.num_actions - 1)];
     SfStepOut o;
-    sf_env_step(D, H, env, e, km, autoreset, (A.flags & SF_FLAG_RAW_REWARD) != 0, o);
-    size_t oi = (size_t)t * D.n + env;
-    if (A.reward) A.reward[oi] = o.reward;
-    if (A.done) A.done[oi] = o.done;
-    if (A.fortkill) A.fortkill[oi] = o.fort_kill;
-    if (A.events) A.events[oi] = o.events;
+    sf_tick_env(D, H, A, env, t, autoreset, e, o);
     finished = o.done && autoreset;
     shell_vis = o.shell_vis;
   }
@@ -194,6 +206,18 @@ __device__ __noinline__ void sf_step_group(const SfDev& D, const SfRollArgs& A, 
   SF_ST(15);
 }
 
+// SF_ROLL_DRAW (Game.draw of the current state): the group's records without a step (warp 0, one env per lane)
+__device__ __forceinline__ void sf_load_group(const SfDev& D, const SfRollArgs& A, int group, SfEnvRec* recs) {
+  const int lane = threadIdx.x & 31;
+  const int env = A.env0 + group * A.EB + lane;
+  const bool mine = lane < A.EB && env < A.env0 + A.envn && (!A.draw_mask || A.draw_mask[env]);
+  if (mine) {
+    SfEnv e;
+    sf_load_env(D, env, e);
+    sf_make_env_rec(e, env, sf_visible_shells(D, env, (unsigned)e.q0.y), recs[lane]);
+  } else recs[lane].env = -1;
+  __syncwarp();
+}
 
 // The two roles of the rollout kernel, out of line (separate register allocations, see sf_stepper_ticks). Both walk the
 // same sequence of groups: the block's first group is blockIdx.x, further ones are handed out first come first served
@@ -201,7 +225,8 @@ __device__ __noinline__ void sf_step_group(const SfDev& D, const SfRollArgs& A, 
 // and leaves it in shared memory (a ring indexed by the group count, SF_NEXT_GROUPS); the other warps read it when they
 // are done with the current group, many barriers later. The steps of the next ticks (warp 0) run while the other warps
 // draw the ticks before them, across groups too.
-__device__ __noinline__ void sf_rollout_stepper(const SfDev& D, const SfRollArgs& A) {
+template <int MODE>
+__device__ __forceinline__ void sf_stepper_role(const SfDev& D, const SfRollArgs& A) {
   const int lane = threadIdx.x & 31;
   SfBlockSmem& B = sf_block_smem();
   const bool native = (A.flags & SF_FLAG_NATIVE_OBS) != 0;
@@ -209,7 +234,10 @@ __device__ __noinline__ void sf_rollout_stepper(const SfDev& D, const SfRollArgs
 #pragma unroll 1
   for (int k = 0; group < A.ngroups; k = (k + 1) % SF_NEXT_GROUPS) {
     if (lane == 0) B.next_group[k] = A.sched ? (int)gridDim.x + atomicAdd(&A.sched->next_group, 1) : group + (int)gridDim.x;
-    sf_stepper_ticks(D, B, lane, native, A.T, stage, [&](int t, SfStagePrep& Tm, int h) { sf_step_group(D, A, group, t, &Tm.env[32 * h]); });
+    sf_stepper_ticks(D, B, lane, native, sf_roll_ticks<MODE>(A), stage, [&](int t, SfStagePrep& Tm, int h) {
+      if constexpr (MODE == SF_ROLL_DRAW) sf_load_group(D, A, group, Tm.env);
+      else sf_step_group(D, A, group, t, &Tm.env[32 * h]);
+    });
     group = B.next_group[k];
   }
   sf_stepper_drain(stage);
@@ -219,6 +247,13 @@ __device__ __noinline__ void sf_rollout_stepper(const SfDev& D, const SfRollArgs
     if (atomicAdd(&A.sched->done, 1) == (int)gridDim.x - 1) { A.sched->next_group = 0; A.sched->done = 0; __threadfence(); }
   }
 }
+// The step modes call the stepping warp's role out of line. The draw mode inlines it: its short preparation is all of
+// warp 0's work, and out of line it reaches D and A through references to the kernel parameters (generic loads instead
+// of constant-bank loads), which made a draw 1-2.5 % slower (DESIGN.md 4.1).
+template <int MODE>
+__device__ __noinline__ void sf_rollout_stepper(const SfDev& D, const SfRollArgs& A) { sf_stepper_role<MODE>(D, A); }
+
+template <int MODE>
 __device__ __forceinline__ void sf_rollout_drawer(const SfDev& D, const SfRollArgs& A) {
   const int lane = threadIdx.x & 31;
   SfBlockSmem& B = sf_block_smem();
@@ -227,13 +262,13 @@ __device__ __forceinline__ void sf_rollout_drawer(const SfDev& D, const SfRollAr
   out.native = (A.flags & SF_FLAG_NATIVE_OBS) ? 1 : 0;
   out.obs_bytes = out.native ? (size_t)SF_NAT_H * SF_NAT_W : (size_t)84 * 84;
   out.obs = A.obs;
-  out.tick_bytes = (size_t)D.n * out.obs_bytes;
+  out.tick_bytes = MODE == SF_ROLL_DRAW ? 0 : (size_t)D.n * out.obs_bytes;
   SfStageState st;
   st.stage = 0; st.prev_used = 0;
   int group = blockIdx.x;
 #pragma unroll 1
   for (int k = 0; group < A.ngroups; k = (k + 1) % SF_NEXT_GROUPS) {
-    sf_drawer_ticks(D, B, W, lane, out, A.T, st);
+    sf_drawer_ticks(D, B, W, lane, out, sf_roll_ticks<MODE>(A), st);
     group = B.next_group[k];
   }
 }
@@ -317,14 +352,17 @@ __global__ void __launch_bounds__(256) sf_host_delta_kernel(const uint4* __restr
   sf_host_delta_count(stats, sent);
 }
 
-// (HOST_DELTA is a second instantiation, used by sf_step_host only: the register allocation of the plain kernel is
-// sensitive to anything that is added to its body, see DESIGN.md 7b.)
-template <bool HOST_DELTA>
+// (SF_ROLL_STEP_HOST_DELTA is a separate instantiation, used by sf_step_host only: the register allocation of the plain
+// kernel is sensitive to anything that is added to its body, see DESIGN.md 7b. SF_ROLL_DRAW runs T = 1 with static groups.)
+template <int MODE>
 __global__ void __launch_bounds__(SF_BLOCK, 1) sf_rollout_kernel(const __grid_constant__ SfDev D, const __grid_constant__ SfRollArgs A) {
   sf_block_smem_init(D.static_image);
   sf_warp_smem_init(sf_my_smem(), threadIdx.x & 31);
-  if (threadIdx.x < 32) sf_rollout_stepper(D, A); else sf_rollout_drawer(D, A);
-  if (HOST_DELTA) {
+  if (threadIdx.x < 32) {
+    if constexpr (MODE == SF_ROLL_DRAW) sf_stepper_role<MODE>(D, A);
+    else sf_rollout_stepper<MODE>(D, A);
+  } else sf_rollout_drawer<MODE>(D, A);
+  if (MODE == SF_ROLL_STEP_HOST_DELTA) {
     __syncthreads();  // every frame of this block's groups is written (the bulk copies were waited for before the patches)
     sf_block_host_delta(D, A);
   }
@@ -341,16 +379,8 @@ __global__ void __launch_bounds__(128) sf_step_only_kernel(SfDev D, SfRollArgs A
   for (int t = 0; t < A.T; t++) {
     bool finished = false;
     if (mine) {
-      int a = A.actions ? A.actions[(size_t)t * D.n + env]
-                        : sf_hash_action(A.action_seed, (unsigned long long)(D.first_global_env + env), (unsigned long long)(A.t0 + t), D.num_actions);
-      int km = (A.flags & SF_FLAG_ACTIONS_ARE_KEYMASKS) ? (a & 15) : D.keymask_of_action[min(max(a, 0), D.num_actions - 1)];
       SfStepOut o;
-      sf_env_step(D, &D.tab->hot, env, e, km, autoreset, (A.flags & SF_FLAG_RAW_REWARD) != 0, o);
-      size_t oi = (size_t)t * D.n + env;
-      if (A.reward) A.reward[oi] = o.reward;
-      if (A.done) A.done[oi] = o.done;
-      if (A.fortkill) A.fortkill[oi] = o.fort_kill;
-      if (A.events) A.events[oi] = o.events;
+      sf_tick_env(D, &D.tab->hot, A, env, t, autoreset, e, o);
       finished = o.done && autoreset;
     }
     if (__any_sync(0xffffffffu, finished)) {
@@ -362,42 +392,6 @@ __global__ void __launch_bounds__(128) sf_step_only_kernel(SfDev D, SfRollArgs A
   if (mine) sf_store_env(D, env, e);
 }
 
-// render the current state (Game.draw): the same block-cooperative pipeline without the step
-__global__ void __launch_bounds__(SF_BLOCK, 1) sf_render_kernel(SfDev D, unsigned char* obs, int flags, const unsigned char* mask, int EB, int ngroups) {
-  const int lane = threadIdx.x & 31;
-  SfBlockSmem& B = sf_block_smem();
-  SfWarpSmem& W = sf_my_smem();
-  sf_block_smem_init(D.static_image);
-  sf_warp_smem_init(W, lane);
-  const bool native = (flags & SF_FLAG_NATIVE_OBS) != 0;
-  if (threadIdx.x < 32) {
-    int stage = 0;
-#pragma unroll 1
-    for (int group = blockIdx.x; group < ngroups; group += gridDim.x)
-      sf_stepper_ticks(D, B, lane, native, 1, stage, [&](int, SfStagePrep& Tm, int) {
-        const int env = group * EB + lane;
-        const bool mine = lane < EB && env < D.n && (!mask || mask[env]);
-        if (mine) {
-          SfEnv e;
-          sf_load_env(D, env, e);
-          sf_make_env_rec(e, env, sf_visible_shells(D, env, (unsigned)e.q0.y), Tm.env[lane]);
-        } else Tm.env[lane].env = -1;
-        __syncwarp();
-      });
-    sf_stepper_drain(stage);
-  } else {
-    SfFrameOut out;
-    out.native = native ? 1 : 0;
-    out.obs_bytes = out.native ? (size_t)SF_NAT_H * SF_NAT_W : (size_t)84 * 84;
-    out.obs = obs;
-    out.tick_bytes = 0;
-    SfStageState st;
-    st.stage = 0; st.prev_used = 0;
-#pragma unroll 1
-    for (int group = blockIdx.x; group < ngroups; group += gridDim.x) sf_drawer_ticks(D, B, W, lane, out, 1, st);
-  }
-}
-
 // once per handle (and after sf_set_glyph_masks): the static part of SfBlockSmem, built from the tables, as an image in
 // global memory that the rendering kernels fetch with one bulk copy
 __global__ void __launch_bounds__(SF_BLOCK) sf_pack_static_kernel(SfDev D, unsigned char* image) {
@@ -407,14 +401,22 @@ __global__ void __launch_bounds__(SF_BLOCK) sf_pack_static_kernel(SfDev D, unsig
   for (int k = threadIdx.x; k < (int)(SF_STATIC_BYTES / 16); k += blockDim.x) reinterpret_cast<int4*>(image)[k] = src[k];
 }
 
+// For a state that was not reached by stepping the env (new seed, forced record, loaded blob). The env's render caches
+// (explosion sprite, resampled box) are keyed by the ship's life: the rand() calls consumed at its spawn + 1. That key
+// names a life only along one rand() stream followed step by step: after a new seed the counter restarts, and a forced or
+// loaded state may place a dead ship anywhere at a count that a life of this env's old state also had.
+__device__ __forceinline__ void sf_forget_render_caches(const SfDev& D, int env) {
+  D.expstamp[env] = 0;
+  D.expo_meta[env] = make_uint2(0u, 0u);
+}
+
 __global__ void sf_seed_kernel(SfDev D, const unsigned* seeds) {
   const int env = blockIdx.x * blockDim.x + threadIdx.x;
   if (env >= D.n) return;
   SfEnv e;
   sf_load_env(D, env, e);
   sf_srand(D, env, e, seeds ? seeds[env] : 1u);
-  D.expstamp[env] = 0;  // the rand() call counter restarts: no cached explosion belongs to a life of the new stream
-  D.expo_meta[env] = make_uint2(0u, 0u);
+  sf_forget_render_caches(D, env);
   sf_store_env(D, env, e);
 }
 
@@ -601,8 +603,7 @@ __global__ void sf_set_state_kernel(SfDev D, int first, int count, const sf_stat
     D.svel[(size_t)s * D.n_pad + i] = make_double2(r.shell_vx[s], r.shell_vy[s]);
     D.sang[(size_t)s * D.n_pad + i] = r.shell_angle[s];
   }
-  D.expstamp[i] = 0;  // a forced state may place a dead ship anywhere
-  D.expo_meta[i] = make_uint2(0u, 0u);
+  sf_forget_render_caches(D, i);
   sf_store_env(D, i, e);
 }
 
@@ -691,8 +692,7 @@ __global__ void __launch_bounds__(32) sf_save_envs_kernel(SfDev D, int gametype,
 }
 
 // Rows with a bad header or target index are skipped and counted into *rejected (one atomic per warp). Writes only the
-// live missile and shell slots (the others are never read), and resets the env's render caches: a cached explosion is
-// keyed by the rand() calls consumed at the ship's spawn, which envs of equal seeds reach at different positions.
+// live missile and shell slots (the others are never read), and resets the env's render caches.
 __global__ void __launch_bounds__(32) sf_load_envs_kernel(SfDev D, int gametype, const int4* __restrict__ blob, const int* __restrict__ idx, int count,
                                                           int* rejected) {
   __shared__ int4 tile[32 * SF_BLOB_PITCH];
@@ -747,8 +747,7 @@ __global__ void __launch_bounds__(32) sf_load_envs_kernel(SfDev D, int gametype,
       const unsigned* rng = reinterpret_cast<const unsigned*>(rb + SF_BO_RNG);
 #pragma unroll
       for (int w = 0; w < SF_RNG_WORDS; w++) D.rng[w * np + i] = rng[w];
-      D.expstamp[i] = 0;
-      D.expo_meta[i] = make_uint2(0u, 0u);
+      sf_forget_render_caches(D, i);
     }
     __syncwarp();  // the tile is reused
   }
@@ -918,9 +917,9 @@ extern "C" int sf_create(const char* gametype, int action_set, int n_envs, int d
   if ((ce = cudaMemset(h->d_sched, 0, sizeof(SfSched))) != cudaSuccess) return bail("cudaMemset scheduler state", ce);
   if ((ce = cudaMemset(h->slab, 0, h->slab_bytes)) != cudaSuccess) return bail("cudaMemset state slab", ce);
   if ((ce = cudaMemcpy((void*)d.tab, h->h_tab, sizeof(SfTables), cudaMemcpyHostToDevice)) != cudaSuccess) return bail("upload tables", ce);
-  if ((ce = cudaFuncSetAttribute(sf_rollout_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS))) != cudaSuccess) return bail("shared memory opt-in (rollout)", ce);
-  if ((ce = cudaFuncSetAttribute(sf_rollout_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS))) != cudaSuccess) return bail("shared memory opt-in (rollout, host delta)", ce);
-  if ((ce = cudaFuncSetAttribute(sf_render_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS))) != cudaSuccess) return bail("shared memory opt-in (render)", ce);
+  if ((ce = cudaFuncSetAttribute(sf_rollout_kernel<SF_ROLL_STEP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS))) != cudaSuccess) return bail("shared memory opt-in (rollout)", ce);
+  if ((ce = cudaFuncSetAttribute(sf_rollout_kernel<SF_ROLL_STEP_HOST_DELTA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS))) != cudaSuccess) return bail("shared memory opt-in (rollout, host delta)", ce);
+  if ((ce = cudaFuncSetAttribute(sf_rollout_kernel<SF_ROLL_DRAW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS))) != cudaSuccess) return bail("shared memory opt-in (rollout, draw)", ce);
   if ((ce = cudaFuncSetAttribute(sf_pack_static_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS))) != cudaSuccess) return bail("shared memory opt-in (pack)", ce);
   if ((ce = cudaFuncSetAttribute(sf_save_envs_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared)) != cudaSuccess) return bail("shared memory carveout (save envs)", ce);
   if ((ce = cudaFuncSetAttribute(sf_load_envs_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared)) != cudaSuccess) return bail("shared memory carveout (load envs)", ce);
@@ -998,10 +997,22 @@ static void group_shape(const sf_handle* h, int n, int* EB, int* ngroups, int* b
   *blocks = std::min(*ngroups, sms);
 }
 
-static int launch_render(sf_handle* h, unsigned char* d_obs, int flags, const unsigned char* d_mask, cudaStream_t st) {
-  int EB, ngroups, blocks;
-  group_shape(h, h->dev.n, &EB, &ngroups, &blocks);
-  sf_render_kernel<<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(h->dev, d_obs, flags, d_mask, EB, ngroups);
+// The launch shape (EB, ngroups, sched) and the instantiation are chosen here; callers set the other fields.
+static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st, bool draw = false) {
+  const SfDev& d = h->dev;
+  bool render = (a.flags & SF_FLAG_RENDER) && a.obs;
+  if (render) {
+    int blocks;
+    group_shape(h, a.envn, &a.EB, &a.ngroups, &blocks);
+    // the hand-out counters serve full-slab steps only; draws, slices of the slab (sf_step_host) and in-kernel delta
+    // launches take static groups
+    a.sched = (!draw && a.env0 == 0 && a.envn == d.n && !a.host_obs) ? h->d_sched : nullptr;
+    if (draw) sf_rollout_kernel<SF_ROLL_DRAW><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
+    else if (a.host_obs) sf_rollout_kernel<SF_ROLL_STEP_HOST_DELTA><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
+    else sf_rollout_kernel<SF_ROLL_STEP><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
+  } else {
+    sf_step_only_kernel<<<(a.envn + 127) / 128, 128, 0, st>>>(d, a);
+  }
   CUDA_TRY(cudaGetLastError());
   return SF_OK;
 }
@@ -1119,31 +1130,18 @@ extern "C" int sf_reset(sf_handle* h, const uint8_t* d_mask, int clear_prev_vlne
   cudaStream_t st = (cudaStream_t)stream;
   sf_reset_kernel<<<(h->dev.n + 127) / 128, 128, 0, st>>>(h->dev, d_mask, clear_prev_vlner);
   CUDA_TRY(cudaGetLastError());
-  if (d_obs) return launch_render(h, d_obs, flags, d_mask, st);
-  return SF_OK;
+  if (!d_obs) return SF_OK;
+  SfRollArgs a = {};
+  a.T = 1; a.obs = d_obs; a.flags = flags | SF_FLAG_RENDER; a.envn = h->dev.n; a.draw_mask = d_mask;
+  return launch_rollout(h, a, st, true);
 }
 
 extern "C" int sf_render(sf_handle* h, uint8_t* d_obs, int flags, void* stream) {
   if (!h || !d_obs) return fail(SF_ERR_INVALID, "handle or obs is NULL");
   CUDA_TRY(cudaSetDevice(h->device));
-  return launch_render(h, d_obs, flags, nullptr, (cudaStream_t)stream);
-}
-
-// The launch shape (EB, ngroups, sched) is derived here; callers set the other fields.
-static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st) {
-  const SfDev& d = h->dev;
-  bool render = (a.flags & SF_FLAG_RENDER) && a.obs;
-  if (render) {
-    int blocks;
-    group_shape(h, a.envn, &a.EB, &a.ngroups, &blocks);
-    a.sched = (a.env0 == 0 && a.envn == d.n && !a.host_obs) ? h->d_sched : nullptr;  // slices of the slab (sf_step_host), in-kernel delta: static groups
-    if (a.host_obs) sf_rollout_kernel<true><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
-    else sf_rollout_kernel<false><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
-  } else {
-    sf_step_only_kernel<<<(a.envn + 127) / 128, 128, 0, st>>>(d, a);
-  }
-  CUDA_TRY(cudaGetLastError());
-  return SF_OK;
+  SfRollArgs a = {};
+  a.T = 1; a.obs = d_obs; a.flags = flags | SF_FLAG_RENDER; a.envn = h->dev.n;
+  return launch_rollout(h, a, (cudaStream_t)stream, true);
 }
 
 extern "C" int sf_step(sf_handle* h, const int32_t* d_actions, uint8_t* d_obs, int32_t* d_reward, uint8_t* d_done,

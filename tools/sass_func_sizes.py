@@ -1,11 +1,11 @@
 """Instructions and local-memory accesses (LDL / STL: spills, by-reference structs) of a kernel per SOURCE function, from
 the line markers of `nvdisasm -g` — no GPU needed. With two libraries: only the functions that differ (A/B of a build).
-usage: python tools/sass_func_sizes.py libA.so [libB.so] [--kernel sf_rollout_kernelILb0]"""
+usage: python tools/sass_func_sizes.py libA.so [libB.so] [--kernel sf_rollout_kernelILi0]"""
 import os, re, subprocess, sys, tempfile
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SRC = os.path.join(ROOT, "spacefortress_b200", "csrc")
 args = [a for a in sys.argv[1:] if not a.startswith("--")]
-kernel = sys.argv[sys.argv.index("--kernel") + 1] if "--kernel" in sys.argv else "sf_rollout_kernelILb0"
+kernel = sys.argv[sys.argv.index("--kernel") + 1] if "--kernel" in sys.argv else "sf_rollout_kernelILi0"
 args = [a for a in args if a != kernel]
 
 def marks_of(fn):
