@@ -71,7 +71,8 @@ enum {
   SF_FLAG_HOST_DELTA = 32   /* sf_step_host only: h_obs is page-locked and unchanged since the previous call (see sf_step_host) */
 };
 
-/* observation types of SSF_Env (ssf_env.py:51): the image is sf_step's d_obs; the other three are sf_features */
+/* observation types of SSF_Env (ssf_env.py:51): the image is sf_step's d_obs; the other three are sf_features of the
+ * current state, or the per-step rows of sf_rollout_features / sf_step_host_features */
 enum { SF_OBS_IMAGE = 0, SF_OBS_FEATURES = 1, SF_OBS_NORMALIZED_FEATURES = 2, SF_OBS_MONITORS = 3 };
 
 /* Per-env state record for get/set (teacher forcing, checkpointing, getters). Same members as the
@@ -233,6 +234,23 @@ int sf_policy_input_f32(const uint8_t* d_frames, long long frame_stride_bytes, i
 int sf_num_features(const sf_handle* h, int obs_type);
 int sf_features(sf_handle* h, int obs_type, float* d_out, void* stream);
 int sf_features_f64(sf_handle* h, int obs_type, double* d_out, void* stream);
+
+/* Feature observations as outputs of the step (render off), from the state-only kernel that steps the envs: no second
+ * launch, and no frames. Row t of an env is bit for bit what sf_features (float32) returns after tick t: the state after
+ * the tick, the first state of the new episode after an auto-reset, the finished state under SF_FLAG_NO_AUTORESET.
+ * obs_type: SF_OBS_FEATURES, SF_OBS_NORMALIZED_FEATURES or SF_OBS_MONITORS. SF_FLAG_RENDER, SF_FLAG_NATIVE_OBS,
+ * SF_FLAG_HOST_DELTA, a bad obs_type or a NULL features pointer -> SF_ERR_INVALID.
+ * sf_rollout_features: T consecutive steps in ONE launch with feature observations instead of frames. d_features float32
+ * [T][n][sf_num_features(h, obs_type)], row t = the features after tick t (auto-reset included); the other outputs as in
+ * sf_rollout plus d_events [T][n] (any may be NULL); d_actions NULL = the synthetic stream. T <= 0 -> SF_ERR_INVALID. */
+int sf_rollout_features(sf_handle* h, int obs_type, int T, const int32_t* d_actions, uint32_t action_seed, long long t0,
+                        float* d_features, int32_t* d_reward, uint8_t* d_done, uint8_t* d_fortkill, uint32_t* d_events,
+                        int flags, void* stream);
+/* sf_step_host with feature rows [n][F] into h_features. If h_features is page-locked, the kernel writes the rows in place
+ * through its device alias, like the small per-env arrays; otherwise a device buffer is copied back. Same ordering rules
+ * as sf_step_host. */
+int sf_step_host_features(sf_handle* h, int obs_type, const int32_t* h_actions, float* h_features, int32_t* h_reward,
+                          uint8_t* h_done, uint8_t* h_fortkill, uint32_t* h_events, int flags);
 
 /* Score digits (drawScore, draw.cpp:160-173) are font dependent: the reference asks fontconfig for "monospace" bold and
  * draws whatever face the machine has. The built-in digits are a 7-segment face on the same metrics. Where a real cairo and

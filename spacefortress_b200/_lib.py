@@ -103,6 +103,9 @@ _PROTOTYPES = {
     "sf_num_features": (C.c_int, [C.c_void_p, C.c_int]),
     "sf_features": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
     "sf_features_f64": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]),
+    "sf_rollout_features": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_uint32, C.c_longlong, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
+    "sf_step_host_features": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "sf_set_glyph_masks": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "sf_background": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "sf_host_static_frame": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),

@@ -12,8 +12,9 @@
 //                               tables arrive as one bulk copy of a per-handle image (sf_pack_static_kernel).
 //                               Three instantiations (SfRollMode): step, step with host delta (sf_step_host), and draw
 //                               (sf_render, sf_reset: warp 0 loads the current state instead of stepping it).
-//   sf_step_only_kernel         state-only variant (render off), one env per thread.
-//   sf_features_kernel          the feature observation types of ssf_env.py:95-157, one env per thread.
+//   sf_step_only_kernel         state-only variant (render off), one env per thread; <true> also writes a feature row per
+//                               env and tick (sf_rollout_features, sf_step_host_features).
+//   sf_features_kernel          the feature observation types of ssf_env.py:95-157 of the current state, one env per thread.
 //   sf_policy_input_kernel      4-frame stack -> the policy's first-layer input (bf16 or fp32, space-to-depth NHWC).
 //   sf_reset_kernel / sf_seed_kernel / sf_get_state_kernel / sf_set_state_kernel / sf_pack_static_kernel
 #include <cuda_runtime.h>
@@ -135,6 +136,13 @@ struct SfRollArgs {
   uint4* mirror;       // device copy of what that buffer holds
   unsigned long long* delta_stats;
   const unsigned char* draw_mask;  // SF_ROLL_DRAW: the envs to draw (NULL: all); the others' frames are not written
+};
+// The feature rows of sf_rollout_features / sf_step_host_features: float32 [T][n][cols], row t = the state after tick t. A
+// parameter of the state-only kernel of its own: SfRollArgs is 128 bytes, and with these members appended the compiler
+// gave the kernel without feature rows 80 registers instead of 72 (different code from the same source).
+struct SfFeatArgs {
+  float* out;      // NULL: no feature rows
+  int kind, cols;  // SF_OBS_FEATURES / SF_OBS_NORMALIZED_FEATURES / SF_OBS_MONITORS, sf_feature_cols
 };
 enum SfRollMode { SF_ROLL_STEP, SF_ROLL_STEP_HOST_DELTA, SF_ROLL_DRAW };
 // ticks per group, for both roles of a launch: a draw is the one frame of the current state
@@ -368,30 +376,6 @@ __global__ void __launch_bounds__(SF_BLOCK, 1) sf_rollout_kernel(const __grid_co
   }
 }
 
-// state-only: one env per thread
-__global__ void __launch_bounds__(128) sf_step_only_kernel(SfDev D, SfRollArgs A) {
-  const int env = A.env0 + blockIdx.x * blockDim.x + threadIdx.x;
-  const int lane = threadIdx.x & 31;
-  const bool mine = env < A.env0 + A.envn;
-  const bool autoreset = !(A.flags & SF_FLAG_NO_AUTORESET);
-  SfEnv e;
-  if (mine) sf_load_env(D, env, e);
-  for (int t = 0; t < A.T; t++) {
-    bool finished = false;
-    if (mine) {
-      SfStepOut o;
-      sf_tick_env(D, &D.tab->hot, A, env, t, autoreset, e, o);
-      finished = o.done && autoreset;
-    }
-    if (__any_sync(0xffffffffu, finished)) {
-      sf_accumulate_episode(D, env, e, finished, lane);
-      if (finished) sf_new_game(D, &D.tab->hot, env, e);
-    }
-    if (mine && (t & 7) == 7) sf_flush_stats(D, env, e);  // the pending increments are 8-bit fields
-  }
-  if (mine) sf_store_env(D, env, e);
-}
-
 // once per handle (and after sf_set_glyph_masks): the static part of SfBlockSmem, built from the tables, as an image in
 // global memory that the rendering kernels fetch with one bulk copy
 __global__ void __launch_bounds__(SF_BLOCK) sf_pack_static_kernel(SfDev D, unsigned char* image) {
@@ -441,15 +425,19 @@ __global__ void sf_reset_kernel(SfDev D, const unsigned char* mask, int clear_pr
 
 
 // ------------------------------------------------------------------------------------------------
-// feature observations (ssf_env.py:95-157) from the state, one thread per env
+// feature observations (ssf_env.py:95-157), one thread per env: of the current state (sf_features_kernel) or of the
+// state after every tick (sf_step_only_kernel<true>)
 // ------------------------------------------------------------------------------------------------
+// columns of a row: 15 + the key timers (4 youturn, 2 autoturn) for features / normalized-features, 10 for monitors
+__host__ __device__ inline int sf_feature_cols(int autoturn, int kind) { return kind == SF_OBS_MONITORS ? 10 : 15 + (autoturn ? 2 : 4); }
+
 // computeExtra (game.cpp:282-312). The reference evaluates it inside updateShip while the ship is alive and keeps the
 // values while it is dead; position, velocity and heading are frozen while dead, so evaluating it from the current
 // state gives the same numbers. Before the first tick of a Game the reference's mExtra is uninitialised memory; the
 // test harness zero-fills the Game, and so does this (tick 0 -> 0, 0, 0). fdist keeps the bug of the reference (Q11:
 // the y term is ship.y - ship.y).
 struct SfExtra { double vdir, aim, ndist; };
-__device__ inline SfExtra sf_compute_extra(const SfEnv& e) {
+__device__ __forceinline__ SfExtra sf_compute_extra(const SfEnv& e) {
   SfExtra x;
   x.vdir = 0.0; x.aim = 0.0; x.ndist = 0.0;
   if (e.q3.z == 0) return x;
@@ -478,12 +466,11 @@ __device__ __forceinline__ double sf_pymod360(double v) {  // Python's float `v 
   return m;
 }
 
+// The one definition of a feature row: o[0 .. sf_feature_cols) <- the observation `kind` of state e. Inline: it reads the
+// env's registers through a reference (see sf_accumulate_episode_vals). Each value is stored as soon as it is computed,
+// so the stepping kernel holds no row of doubles.
 template <class OutT>
-__global__ void sf_features_kernel(SfDev D, int kind, OutT* out) {
-  const int env = blockIdx.x * blockDim.x + threadIdx.x;
-  if (env >= D.n) return;
-  SfEnv e;
-  sf_load_env(D, env, e);
+__device__ __forceinline__ void sf_feature_row(const SfEnv& e, bool autoturn, int kind, OutT* o) {
   const SfExtra x = sf_compute_extra(e);
   const unsigned core = (unsigned)e.q0.x;
   const double alive = (core & SF_CORE_SHIP_ALIVE) ? 1.0 : 0.0, falive = (core & SF_CORE_FORT_ALIVE) ? 1.0 : 0.0;
@@ -491,32 +478,92 @@ __global__ void sf_features_kernel(SfDev D, int kind, OutT* out) {
   const double kill_window = (vuln > 10 && e.q1.y < 250) ? 1.0 : 0.0;   // vulnerability_timer < fortressVulnerabilityTime
   const int nm = __popc((unsigned)e.q0.y & SF_PMASK_MISSILES), ns = __popc(((unsigned)e.q0.y >> SF_PMASK_SHELL_SHIFT) & 0xFu);
   const double fang = 10.0 * (double)((core >> SF_CORE_FANG_SHIFT) & 63u), sang = (double)(core & SF_CORE_ANGLE_MASK);
-  const int nt = D.autoturn ? 2 : 4;
-  double f[19];
-  int nf;
   if (kind == SF_OBS_MONITORS) {          // ssf_env.py:96-108
-    nf = 10;
-    f[0] = nm > 0 ? 0.5 : -0.5; f[1] = falive != 0.0 ? 0.5 : -0.5; f[2] = vuln > 10 ? 0.5 : -0.5; f[3] = kill_window != 0.0 ? 0.5 : -0.5;
-    f[4] = x.aim < 3 ? 0.5 : -0.5; f[5] = x.aim > 3 ? 0.5 : -0.5;
-    f[6] = x.ndist > .75 ? 0.5 : -0.5; f[7] = x.ndist > .25 ? 0.5 : -0.5; f[8] = x.ndist < -.25 ? 0.5 : -0.5; f[9] = x.ndist < -.75 ? 0.5 : -0.5;
+    auto put = [&](int k, bool on) { o[k] = (OutT)(on ? 0.5 : -0.5); };
+    put(0, nm > 0); put(1, falive != 0.0); put(2, vuln > 10); put(3, kill_window != 0.0);
+    put(4, x.aim < 3); put(5, x.aim > 3);
+    put(6, x.ndist > .75); put(7, x.ndist > .25); put(8, x.ndist < -.25); put(9, x.ndist < -.75);
   } else if (kind == SF_OBS_NORMALIZED_FEATURES) {  // ssf_env.py:109-133 (sic: max(vulnerability, 10)); np.clip(f, -1, 1)
-    nf = 15 + nt;
-    f[0] = alive; f[1] = SF_DDIV(e.pos.x, 90.0); f[2] = SF_DDIV(e.pos.y, 92.0); f[3] = SF_DDIV(e.vel.x, 10.0); f[4] = SF_DDIV(e.vel.y, 10.0);
-    f[5] = SF_DDIV(sang, 360.0); f[6] = SF_DDIV(x.aim, 180.0); f[7] = SF_DDIV(sf_pymod360(x.vdir), 360.0); f[8] = x.ndist;
-    f[9] = falive; f[10] = SF_DDIV(fang, 360.0); f[11] = SF_DDIV((double)max(vuln, 10), 10.0); f[12] = kill_window;
-    f[13] = SF_DDIV((double)nm, 20.0); f[14] = SF_DDIV((double)ns, 20.0);
+    auto put = [&](int k, double v) { o[k] = (OutT)sf_clip1(v); };
+    put(0, alive); put(1, SF_DDIV(e.pos.x, 90.0)); put(2, SF_DDIV(e.pos.y, 92.0)); put(3, SF_DDIV(e.vel.x, 10.0)); put(4, SF_DDIV(e.vel.y, 10.0));
+    put(5, SF_DDIV(sang, 360.0)); put(6, SF_DDIV(x.aim, 180.0)); put(7, SF_DDIV(sf_pymod360(x.vdir), 360.0)); put(8, x.ndist);
+    put(9, falive); put(10, SF_DDIV(fang, 360.0)); put(11, SF_DDIV((double)max(vuln, 10), 10.0)); put(12, kill_window);
+    put(13, SF_DDIV((double)nm, 20.0)); put(14, SF_DDIV((double)ns, 20.0));
     const double max_ticks = 5294.0;  // np.floor(180000 / 34), ssf_env.py:166
-    f[15] = SF_DDIV((double)e.q2.x, max_ticks); f[16] = SF_DDIV((double)e.q2.y, max_ticks);
-    f[17] = SF_DDIV((double)e.q2.z, max_ticks); f[18] = SF_DDIV((double)e.q2.w, max_ticks);
-    for (int k = 0; k < 19; k++) f[k] = sf_clip1(f[k]);
+    put(15, SF_DDIV((double)e.q2.x, max_ticks)); put(16, SF_DDIV((double)e.q2.y, max_ticks));
+    if (!autoturn) { put(17, SF_DDIV((double)e.q2.z, max_ticks)); put(18, SF_DDIV((double)e.q2.w, max_ticks)); }
   } else {                               // 'features', ssf_env.py:134-157
-    nf = 15 + nt;
-    f[0] = alive; f[1] = e.pos.x; f[2] = e.pos.y; f[3] = e.vel.x; f[4] = e.vel.y; f[5] = sang; f[6] = x.aim; f[7] = x.vdir; f[8] = x.ndist;
-    f[9] = falive; f[10] = fang; f[11] = (double)vuln; f[12] = kill_window; f[13] = (double)nm; f[14] = (double)ns;
-    f[15] = (double)e.q2.x; f[16] = (double)e.q2.y; f[17] = (double)e.q2.z; f[18] = (double)e.q2.w;
+    auto put = [&](int k, double v) { o[k] = (OutT)v; };
+    put(0, alive); put(1, e.pos.x); put(2, e.pos.y); put(3, e.vel.x); put(4, e.vel.y); put(5, sang); put(6, x.aim); put(7, x.vdir); put(8, x.ndist);
+    put(9, falive); put(10, fang); put(11, (double)vuln); put(12, kill_window); put(13, (double)nm); put(14, (double)ns);
+    put(15, (double)e.q2.x); put(16, (double)e.q2.y);
+    if (!autoturn) { put(17, (double)e.q2.z); put(18, (double)e.q2.w); }
   }
-  OutT* o = out + (size_t)env * nf;
-  for (int k = 0; k < nf; k++) o[k] = (OutT)f[k];
+}
+
+template <class OutT>
+__global__ void sf_features_kernel(SfDev D, int kind, OutT* out) {
+  const int env = blockIdx.x * blockDim.x + threadIdx.x;
+  if (env >= D.n) return;
+  SfEnv e;
+  sf_load_env(D, env, e);
+  sf_feature_row(e, D.autoturn != 0, kind, out + (size_t)env * sf_feature_cols(D.autoturn, kind));
+}
+
+// out[0, len) <- S[pre, pre + len), by all threads of the block. S is 16-byte aligned and pre = (out / 4) % 4, so out[j] and
+// S[pre + j] have the same address mod 16: the 16-byte chunks go out as 16-byte stores, consecutive threads on consecutive
+// chunks, and the at most 3 floats at either end as 4-byte stores.
+__device__ __forceinline__ void sf_store_span(float* out, const float* S, int pre, int len) {
+  const int s1 = pre + len;
+  const int v0 = min((pre + 3) & ~3, s1), v1 = max(s1 & ~3, v0);  // [v0, v1): the whole chunks
+  for (int s = v0 + 4 * (int)threadIdx.x; s < v1; s += 4 * (int)blockDim.x)
+    *reinterpret_cast<float4*>(out + (s - pre)) = *reinterpret_cast<const float4*>(S + s);
+  const int k = threadIdx.x;
+  if (k < v0 - pre) out[k] = S[pre + k];
+  else if (k >= 4 && k - 4 < s1 - v1) out[v1 - pre + k - 4] = S[v1 + k - 4];
+}
+
+// ------------------------------------------------------------------------------------------------
+// state-only step (render off): one env per thread
+// ------------------------------------------------------------------------------------------------
+// FEAT: every tick also writes the feature row of each env's state after the tick (auto-reset included). In one tick the
+// rows of a block's envs are one contiguous span of the output: they are staged in shared memory (two buffers, so one
+// barrier per tick) and leave as consecutive stores across each warp. One thread storing its own row would scatter
+// 4-byte stores 4 * nfeat bytes apart: in HBM, and across PCIe where sf_step_host_features writes straight into a
+// page-locked host buffer (~1.7 ns per scattered store, profiles/r02_pcie_write_probe.txt).
+#define SF_STEP_ONLY_BLOCK 128
+template <bool FEAT>
+__global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_only_kernel(SfDev D, SfRollArgs A, SfFeatArgs F) {
+  const int env = A.env0 + blockIdx.x * blockDim.x + threadIdx.x;
+  const int lane = threadIdx.x & 31;
+  const bool mine = env < A.env0 + A.envn;
+  const bool autoreset = !(A.flags & SF_FLAG_NO_AUTORESET);
+  SfEnv e;
+  if (mine) sf_load_env(D, env, e);
+  for (int t = 0; t < A.T; t++) {
+    bool finished = false;
+    if (mine) {
+      SfStepOut o;
+      sf_tick_env(D, &D.tab->hot, A, env, t, autoreset, e, o);
+      finished = o.done && autoreset;
+    }
+    if (__any_sync(0xffffffffu, finished)) {
+      sf_accumulate_episode(D, env, e, finished, lane);
+      if (finished) sf_new_game(D, &D.tab->hot, env, e);
+    }
+    if (mine && (t & 7) == 7) sf_flush_stats(D, env, e);  // the pending increments are 8-bit fields
+    if constexpr (FEAT) {
+      __shared__ __align__(16) float rows[2][SF_STEP_ONLY_BLOCK * 19 + 4];  // + 3: the span's offset within 16 bytes
+      float* R = rows[t & 1];
+      const int b0 = A.env0 + blockIdx.x * SF_STEP_ONLY_BLOCK;
+      float* span = F.out + ((size_t)t * D.n + b0) * F.cols;
+      const int pre = (int)(((uintptr_t)span >> 2) & 3);
+      if (mine) sf_feature_row(e, D.autoturn != 0, F.kind, R + pre + threadIdx.x * F.cols);
+      __syncthreads();
+      sf_store_span(span, R, pre, min(SF_STEP_ONLY_BLOCK, A.env0 + A.envn - b0) * F.cols);
+    }
+  }
+  if (mine) sf_store_env(D, env, e);
 }
 
 // ---- state records (AoS <-> SoA), one thread per env ----
@@ -997,8 +1044,9 @@ static void group_shape(const sf_handle* h, int n, int* EB, int* ngroups, int* b
   *blocks = std::min(*ngroups, sms);
 }
 
-// The launch shape (EB, ngroups, sched) and the instantiation are chosen here; callers set the other fields.
-static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st, bool draw = false) {
+// The launch shape (EB, ngroups, sched) and the instantiation are chosen here; callers set the other fields. f: feature
+// rows (render off only).
+static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st, bool draw = false, SfFeatArgs f = {}) {
   const SfDev& d = h->dev;
   bool render = (a.flags & SF_FLAG_RENDER) && a.obs;
   if (render) {
@@ -1011,7 +1059,9 @@ static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st, bool draw
     else if (a.host_obs) sf_rollout_kernel<SF_ROLL_STEP_HOST_DELTA><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
     else sf_rollout_kernel<SF_ROLL_STEP><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
   } else {
-    sf_step_only_kernel<<<(a.envn + 127) / 128, 128, 0, st>>>(d, a);
+    const int blocks = (a.envn + SF_STEP_ONLY_BLOCK - 1) / SF_STEP_ONLY_BLOCK;
+    if (f.out) sf_step_only_kernel<true><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, a, f);
+    else sf_step_only_kernel<false><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, a, f);
   }
   CUDA_TRY(cudaGetLastError());
   return SF_OK;
@@ -1092,9 +1142,8 @@ extern "C" int sf_policy_input_f32(const uint8_t* d_frames, long long frame_stri
 
 extern "C" int sf_num_features(const sf_handle* h, int obs_type) {
   if (!h) return -1;
-  if (obs_type == SF_OBS_MONITORS) return 10;
-  if (obs_type == SF_OBS_FEATURES || obs_type == SF_OBS_NORMALIZED_FEATURES) return 15 + (h->dev.autoturn ? 2 : 4);
-  return -1;
+  if (obs_type != SF_OBS_FEATURES && obs_type != SF_OBS_NORMALIZED_FEATURES && obs_type != SF_OBS_MONITORS) return -1;
+  return sf_feature_cols(h->dev.autoturn, obs_type);
 }
 static int features_common(sf_handle* h, int obs_type, void* d_out, bool f64, void* stream) {
   if (!h || !d_out) return fail(SF_ERR_INVALID, "handle or out is NULL");
@@ -1164,6 +1213,28 @@ extern "C" int sf_rollout(sf_handle* h, int T, const int32_t* d_actions, uint32_
   return launch_rollout(h, a, (cudaStream_t)stream);
 }
 
+// the checks both feature steps share; *nf = the row width
+static int feature_step_args(const sf_handle* h, int obs_type, const float* features, int flags, int* nf) {
+  if (!h || !features) return fail(SF_ERR_INVALID, "handle or features is NULL");
+  if ((*nf = sf_num_features(h, obs_type)) < 0) return fail(SF_ERR_INVALID, "obs_type must be SF_OBS_FEATURES, SF_OBS_NORMALIZED_FEATURES or SF_OBS_MONITORS");
+  if (flags & (SF_FLAG_RENDER | SF_FLAG_NATIVE_OBS | SF_FLAG_HOST_DELTA))
+    return fail(SF_ERR_INVALID, "a feature step draws no frames: SF_FLAG_RENDER, SF_FLAG_NATIVE_OBS and SF_FLAG_HOST_DELTA are invalid");
+  return SF_OK;
+}
+
+extern "C" int sf_rollout_features(sf_handle* h, int obs_type, int T, const int32_t* d_actions, uint32_t action_seed, long long t0,
+                                   float* d_features, int32_t* d_reward, uint8_t* d_done, uint8_t* d_fortkill, uint32_t* d_events,
+                                   int flags, void* stream) {
+  int nf;
+  if (int rc = feature_step_args(h, obs_type, d_features, flags, &nf)) return rc;
+  if (T <= 0) return fail(SF_ERR_INVALID, "T <= 0");
+  CUDA_TRY(cudaSetDevice(h->device));
+  SfRollArgs a = {};
+  a.T = T; a.flags = flags; a.actions = d_actions; a.action_seed = action_seed; a.t0 = t0;
+  a.reward = d_reward; a.done = d_done; a.fortkill = d_fortkill; a.events = d_events; a.envn = h->dev.n;
+  return launch_rollout(h, a, (cudaStream_t)stream, false, SfFeatArgs{d_features, obs_type, nf});
+}
+
 extern "C" int sf_synthetic_action(uint32_t action_seed, long long global_env, long long t, int num_actions) {
   return sf_hash_action(action_seed, (unsigned long long)global_env, (unsigned long long)t, num_actions);
 }
@@ -1205,14 +1276,18 @@ static void* device_alias(const void* host) {
   return at.type == cudaMemoryTypeHost ? at.devicePointer : nullptr;
 }
 
-extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_obs, int32_t* h_reward, uint8_t* h_done,
-                            uint8_t* h_fortkill, uint32_t* h_events, int flags) {
+// sf_step_host and sf_step_host_features. h_feat (frames off): feature rows of kind feat_kind, nfeat floats each.
+static int step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_obs, float* h_feat, int feat_kind, int nfeat, int32_t* h_reward,
+                     uint8_t* h_done, uint8_t* h_fortkill, uint32_t* h_events, int flags) {
   if (!h || !h_actions) return fail(SF_ERR_INVALID, "handle or actions is NULL");
   CUDA_TRY(cudaSetDevice(h->device));
   const size_t n = (size_t)h->dev.n;
   const size_t per = (flags & SF_FLAG_NATIVE_OBS) ? (size_t)SF_NAT_H * SF_NAT_W : (size_t)84 * 84, obs_bytes = n * per;
   const bool render = (flags & SF_FLAG_RENDER) && h_obs;
-  int rc = ensure_staging(h, render ? obs_bytes : 0);
+  // page-locked feature rows are written in place like the small arrays below; pageable ones go through the obs staging
+  float* k_feat = (float*)device_alias(h_feat);
+  const size_t feat_bytes = n * nfeat * sizeof(float);
+  int rc = ensure_staging(h, render ? obs_bytes : (h_feat && !k_feat) ? feat_bytes : 0);
   if (rc) return rc;
   // Synchronous, on the handle's own streams. Whole-frame mode: the slab is stepped in slices of consecutive envs, the
   // kernel of slice k + 1 runs while the frames of slice k cross PCIe (one cudaMemcpyAsync per buffer and slice), so only
@@ -1251,11 +1326,12 @@ extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_o
   a.obs = render ? h->d_obs : nullptr; a.reward = k_reward ? k_reward : h->d_reward; a.done = k_done ? k_done : h->d_done;
   a.fortkill = k_kill ? k_kill : h->d_kill; a.events = k_events ? k_events : h->d_events;
   if (fused_delta) { a.host_obs = host_alias; a.mirror = reinterpret_cast<uint4*>(mir->d); a.delta_stats = h->d_delta_stats; }
+  const SfFeatArgs f = {h_feat ? (k_feat ? k_feat : reinterpret_cast<float*>(h->d_obs)) : nullptr, feat_kind, nfeat};
   const int slices = (render && !delta && n >= 2048) ? SF_HOST_STEP_SLICES : 1;
   for (int k = 0; k < slices; k++) {
     const size_t e0 = n * k / slices, e1 = n * (k + 1) / slices;
     a.env0 = (int)e0; a.envn = (int)(e1 - e0);
-    rc = launch_rollout(h, a, sc);
+    rc = launch_rollout(h, a, sc, false, f);
     if (rc) { cudaStreamSynchronize(sc); cudaStreamSynchronize(sx); return rc; }
     if (render && !delta) {
       CUDA_TRY(cudaEventRecord(h->host_ev[k], sc));
@@ -1274,6 +1350,7 @@ extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_o
     mir->host = h_obs; mir->bytes = obs_bytes;
   }
   if (render && !delta) h->full_calls++;
+  if (h_feat && !k_feat) CUDA_TRY(cudaMemcpyAsync(h_feat, h->d_obs, feat_bytes, cudaMemcpyDeviceToHost, sc));
   if (h_reward && !k_reward) CUDA_TRY(cudaMemcpyAsync(h_reward, h->d_reward, n * 4, cudaMemcpyDeviceToHost, sc));
   if (h_done && !k_done) CUDA_TRY(cudaMemcpyAsync(h_done, h->d_done, n, cudaMemcpyDeviceToHost, sc));
   if (h_fortkill && !k_kill) CUDA_TRY(cudaMemcpyAsync(h_fortkill, h->d_kill, n, cudaMemcpyDeviceToHost, sc));
@@ -1284,6 +1361,18 @@ extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_o
     return fail(SF_ERR_CUDA, std::string("sf_step_host: ") + cudaGetErrorString(e1 != cudaSuccess ? e1 : e2));
   }
   return SF_OK;
+}
+
+extern "C" int sf_step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_obs, int32_t* h_reward, uint8_t* h_done,
+                            uint8_t* h_fortkill, uint32_t* h_events, int flags) {
+  return step_host(h, h_actions, h_obs, nullptr, 0, 0, h_reward, h_done, h_fortkill, h_events, flags);
+}
+
+extern "C" int sf_step_host_features(sf_handle* h, int obs_type, const int32_t* h_actions, float* h_features, int32_t* h_reward,
+                                     uint8_t* h_done, uint8_t* h_fortkill, uint32_t* h_events, int flags) {
+  int nf;
+  if (int rc = feature_step_args(h, obs_type, h_features, flags, &nf)) return rc;
+  return step_host(h, h_actions, nullptr, h_features, obs_type, nf, h_reward, h_done, h_fortkill, h_events, flags);
 }
 
 extern "C" int sf_host_forget(sf_handle* h, const void* h_obs) {

@@ -10,6 +10,9 @@ but all N envs live in one SoA slab on one GPU and one kernel launch advances th
 * ``step(torch.Tensor on cuda)`` -> torch CUDA tensors, no host round trip (sf_step).
 * ``rollout(T, actions=None)`` -> T steps in one launch (sf_rollout), time-major outputs.
 
+With ``obs_type`` 'features' / 'normalized-features' / 'monitors' the observation of every step is a feature row written
+by the same state-only kernel that steps the envs (sf_step_host_features, sf_rollout_features).
+
 Auto-reset follows gym_vecenv's worker loop: when an env is done its returned observation is the first
 frame of the next episode; reward/done/info belong to the terminal step.
 """
@@ -53,7 +56,9 @@ class SFVecEnv(object):
         buffers, each updated in place by the GPU (host_delta), and a buffer is reused only when nobody holds a
         reference to the array that was handed out (or to a view / torch.from_numpy tensor of it), so an observation
         a caller keeps is never overwritten; those arrays are read-only (in-place edits would corrupt the next update). obs_type: 'image' (default), or 'features' / 'normalized-features' / 'monitors' (ssf_env.py:95-157):
-        step() / reset() then return the [N, F] float32 feature matrix computed on the device (sf_features).
+        step() / reset() then return the [N, F] float32 feature matrix computed on the device: reset() reads the new
+        state (sf_features), step() and rollout() get the rows from the kernel that steps the envs (sf_step_host_features,
+        sf_rollout_features), one launch per step or rollout.
         host_delta (numpy path): the frames reach the page-locked observation buffer as SF_FLAG_HOST_DELTA updates (only
         the bytes that changed since the previous step cross PCIe; the buffer's contents are those of a full copy). The
         views step() returns are then read-only, because the next update builds on them. False: whole frames every step."""
@@ -119,13 +124,18 @@ class SFVecEnv(object):
         if self._np is None:
             n = self.num_envs
             self._np = {}
-            for k, shape, dt in (("obs", (n,) + (self.obs_shape if self.obs_type == "image" else (1,)), np.uint8), ("reward", (n,), np.int32), ("done", (n,), np.uint8),
+            obs_dt = np.uint8 if self.obs_type == "image" else np.float32  # features: the kernel writes the rows in place
+            for k, shape, dt in (("obs", (n,) + self.obs_shape, obs_dt), ("reward", (n,), np.int32), ("done", (n,), np.uint8),
                                  ("kill", (n,), np.uint8), ("events", (n,), np.uint32), ("actions", (n,), np.int32)):
                 self._np[k] = _lib.pinned_array(shape, dt)  # page-locked: D2H lands directly in what step() returns
             self._np_ptr = {k: C.c_void_p(v.ctypes.data) for k, v in self._np.items()}  # (building these per step costs ~10 us)
             self._obs_ro = self._np["obs"].view()  # what step() hands out under host_delta: the next update builds on its contents
             self._obs_ro.flags.writeable = False
         return self._np
+
+    def _feature_flags(self):
+        """the step flags for the feature steps, which draw no frames"""
+        return self._flags & ~(_lib.FLAG_RENDER | _lib.FLAG_NATIVE_OBS)
 
     def _stream_ptr(self):
         torch = _torch()
@@ -196,11 +206,15 @@ class SFVecEnv(object):
             self._device_work = False
         p = self._np_ptr
         ring = self._ring_buffer() if (self.copy_outputs == "ring" and self.render_on and self.host_delta) else None
-        _lib.check(self.L.sf_step_host(self.h, p["actions"], (ring[3] if ring else p["obs"]) if self.render_on else None, p["reward"], p["done"], p["kill"], p["events"],
-                                       self._flags | (_lib.FLAG_HOST_DELTA if self.host_delta and self.render_on else 0)))
+        if self.obs_type != "image":  # the step kernel writes the feature rows into the page-locked buffer
+            _lib.check(self.L.sf_step_host_features(self.h, _lib.OBS_TYPES[self.obs_type], p["actions"], p["obs"], p["reward"], p["done"],
+                                                    p["kill"], p["events"], self._feature_flags()))
+        else:
+            _lib.check(self.L.sf_step_host(self.h, p["actions"], (ring[3] if ring else p["obs"]) if self.render_on else None, p["reward"], p["done"], p["kill"], p["events"],
+                                           self._flags | (_lib.FLAG_HOST_DELTA if self.host_delta and self.render_on else 0)))
         self._t += 1
         if self.obs_type != "image":
-            obs = self.features(to_numpy=True)
+            obs = b["obs"].copy()  # a new array every step, as gym_vecenv gives
         elif not self.render_on:
             obs = None
         elif ring:
@@ -240,6 +254,14 @@ class SFVecEnv(object):
         torch = _torch()
         b = self._torch_bufs()
         a = actions.to(device=self._device(), dtype=torch.int32).reshape(self.num_envs).contiguous()
+        if self.obs_type != "image":  # one launch: the step kernel writes the feature rows (a new tensor every step)
+            obs = torch.empty((self.num_envs,) + self.obs_shape, dtype=torch.float32, device=self._device())
+            _lib.check(self.L.sf_rollout_features(
+                self.h, _lib.OBS_TYPES[self.obs_type], 1, C.c_void_p(a.data_ptr()), 0, int(self._t), C.c_void_p(obs.data_ptr()),
+                C.c_void_p(b["reward"].data_ptr()), C.c_void_p(b["done"].data_ptr()), C.c_void_p(b["kill"].data_ptr()),
+                C.c_void_p(b["events"].data_ptr()), self._feature_flags(), self._stream_ptr()))
+            self._t += 1
+            return obs, b["reward"], b["done"].bool(), b["kill"].bool()
         if out_obs is not None:
             assert out_obs.is_contiguous() and out_obs.dtype == torch.uint8 and out_obs.numel() == b["obs"].numel()
             b = dict(b, obs=out_obs)
@@ -248,7 +270,7 @@ class SFVecEnv(object):
             C.c_void_p(b["reward"].data_ptr()), C.c_void_p(b["done"].data_ptr()), C.c_void_p(b["kill"].data_ptr()),
             C.c_void_p(b["events"].data_ptr()), self._flags, self._stream_ptr()))
         self._t += 1
-        obs = b["obs"] if self.render_on else (self.features() if self.obs_type != "image" else None)
+        obs = b["obs"] if self.render_on else None
         return obs, b["reward"], b["done"].bool(), b["kill"].bool()
 
     def host_delta_stats(self):
@@ -270,14 +292,16 @@ class SFVecEnv(object):
 
     def rollout(self, T, actions=None, action_seed=0, out=None, want=("obs", "reward", "done", "kill")):
         """T steps in one launch. actions: int32 CUDA tensor [T,N] or None for the synthetic counter-hash
-        policy. Returns a dict of time-major CUDA tensors."""
+        policy. Returns a dict of time-major CUDA tensors. With obs_type != 'image', "obs" is float32 [T, N, F]: row t
+        holds the features after step t (auto-reset included), written by the kernel that steps the envs."""
         torch = _torch()
         dev = self._device()
         n = self.num_envs
+        features = self.obs_type != "image"
         if out is None:
             out = {}
-            if "obs" in want and self.render_on:
-                out["obs"] = torch.empty((T, n) + self.obs_shape, dtype=torch.uint8, device=dev)
+            if "obs" in want and (self.render_on or features):
+                out["obs"] = torch.empty((T, n) + self.obs_shape, dtype=torch.float32 if features else torch.uint8, device=dev)
             if "reward" in want:
                 out["reward"] = torch.empty((T, n), dtype=torch.int32, device=dev)
             if "done" in want:
@@ -291,9 +315,16 @@ class SFVecEnv(object):
 
         def p(k):
             return C.c_void_p(out[k].data_ptr()) if k in out else None
-        flags = self._flags if "obs" in out else (self._flags & ~_lib.FLAG_RENDER)
-        _lib.check(self.L.sf_rollout(self.h, int(T), aptr, int(action_seed), int(self._t), p("obs"), p("reward"), p("done"),
-                                     p("kill"), flags, self._stream_ptr()))
+        if features and "obs" in out:
+            o = out["obs"]
+            if o.dtype != torch.float32 or not o.is_contiguous() or o.numel() != T * n * self.num_features:
+                raise ValueError("out['obs'] must be a contiguous float32 tensor of shape %r" % ((T, n) + self.obs_shape,))
+            _lib.check(self.L.sf_rollout_features(self.h, _lib.OBS_TYPES[self.obs_type], int(T), aptr, int(action_seed), int(self._t),
+                                                  p("obs"), p("reward"), p("done"), p("kill"), None, self._feature_flags(), self._stream_ptr()))
+        else:
+            flags = self._flags if "obs" in out else (self._flags & ~_lib.FLAG_RENDER)
+            _lib.check(self.L.sf_rollout(self.h, int(T), aptr, int(action_seed), int(self._t), p("obs"), p("reward"), p("done"),
+                                         p("kill"), flags, self._stream_ptr()))
         self._t += T
         return out
 
