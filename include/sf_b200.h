@@ -145,6 +145,29 @@ int sf_rollout(sf_handle* h, int T, const int32_t* d_actions, uint32_t action_se
                int32_t* d_reward, uint8_t* d_done, uint8_t* d_fortkill, int flags, void* stream);
 int sf_synthetic_action(uint32_t action_seed, long long global_env, long long t, int num_actions);
 
+/* Extension: action repeat (gym `frameskip`, EnvPool `frame_skip`, the MaxAndSkip wrapper without the max). With repeat
+ * k, one agent step of an env with action a is what this loop around SSF_Env gives inside the gym_vecenv worker:
+ *     R = 0; kill = False; ev = 0
+ *     for j in range(k):
+ *         obs, r, done, kill_j = env.step(a)     # key events, stepOneTick(34), shaping, prev_vlner: per tick as always
+ *         R += r; kill |= kill_j; ev |= events_j
+ *         if done: break                         # the repeat stops on the tick the episode ends
+ *     (auto-reset at that tick)
+ * reward = the int32 sum of the executed ticks' rewards (raw rewards under SF_FLAG_RAW_REWARD); done and fort_kill = set
+ * by any executed tick; events = the OR of their bits (SF_EV_EPISODE_RESET included). The observation (frame or feature
+ * row) is that of the state after the agent step, the first state of the new episode after an auto-reset: bit for bit
+ * what sf_render / sf_features (float32) return then. Under SF_FLAG_NO_AUTORESET the repeat stops at done as well and
+ * the env stays finished. SF_FLAG_ACTIONS_ARE_KEYMASKS repeats the key mask. The synthetic stream is hash(action_seed,
+ * global_env, t0 + t) with t the agent step: all k ticks of a step use the same action.
+ * The setting belongs to the handle (default 1, which is the plain one-tick step) and applies to every later call of
+ * sf_step, sf_rollout, sf_step_host, sf_rollout_features and sf_step_host_features, whose T counts agent steps.
+ * sf_reset, sf_render, sf_features, the env blobs and sf_episode_stats do not depend on it (episode lengths stay in
+ * ticks; a blob row does not hold it). k < 1 or k > SF_MAX_ACTION_REPEAT (one episode) -> SF_ERR_INVALID, setting
+ * unchanged. sf_action_repeat returns the setting, -1 for a NULL handle. */
+#define SF_MAX_ACTION_REPEAT 5295
+int sf_set_action_repeat(sf_handle* h, int k);
+int sf_action_repeat(const sf_handle* h);
+
 /* Render the current state without stepping (Game.draw + gray + resize). */
 int sf_render(sf_handle* h, uint8_t* d_obs, int flags, void* stream);
 

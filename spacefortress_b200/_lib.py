@@ -24,6 +24,7 @@ FLAG_RENDER, FLAG_NO_AUTORESET, FLAG_ACTIONS_ARE_KEYMASKS, FLAG_NATIVE_OBS, FLAG
 
 ENV_BLOB_BYTES = 832  # SF_ENV_BLOB_BYTES: one env's complete game state as one row (sf_save_envs / sf_load_envs)
 ENV_BLOB_VERSION = 1  # SF_ENV_BLOB_VERSION
+MAX_ACTION_REPEAT = 5295  # SF_MAX_ACTION_REPEAT: ticks per agent step at most (one episode)
 
 OBS_TYPES = {"image": 0, "features": 1, "normalized-features": 2, "monitors": 3}  # ssf_env.py:51
 
@@ -89,6 +90,8 @@ _PROTOTYPES = {
     "sf_step": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "sf_rollout": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p, C.c_uint32, C.c_longlong, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "sf_synthetic_action": (C.c_int, [C.c_uint32, C.c_longlong, C.c_longlong, C.c_int]),
+    "sf_set_action_repeat": (C.c_int, [C.c_void_p, C.c_int]),
+    "sf_action_repeat": (C.c_int, [C.c_void_p]),
     "sf_render": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "sf_step_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "sf_host_delta_stats": (C.c_int, [C.c_void_p, C.c_void_p]),

@@ -14,6 +14,8 @@
 //                               (sf_render, sf_reset: warp 0 loads the current state instead of stepping it).
 //   sf_step_only_kernel         state-only variant (render off), one env per thread; <true> also writes a feature row per
 //                               env and tick (sf_rollout_features, sf_step_host_features).
+//   sf_step_repeat_kernel       action repeat (sf_set_action_repeat, k > 1): the state-only step with up to k ticks of one
+//                               action per agent step; with frames each agent step is followed by a SF_ROLL_DRAW launch.
 //   sf_features_kernel          the feature observation types of ssf_env.py:95-157 of the current state, one env per thread.
 //   sf_policy_input_kernel      4-frame stack -> the policy's first-layer input (bf16 or fp32, space-to-depth NHWC).
 //   sf_reset_kernel / sf_seed_kernel / sf_get_state_kernel / sf_set_state_kernel / sf_pack_static_kernel
@@ -149,17 +151,25 @@ enum SfRollMode { SF_ROLL_STEP, SF_ROLL_STEP_HOST_DELTA, SF_ROLL_DRAW };
 template <int MODE>
 __device__ __forceinline__ int sf_roll_ticks(const SfRollArgs& A) { return MODE == SF_ROLL_DRAW ? 1 : A.T; }
 
-// one tick of one env (both step kernels; H: the step's tables): its action, the step, the step's outputs
-__device__ __forceinline__ void sf_tick_env(const SfDev& D, const SfHot* H, const SfRollArgs& A, int env, int t, bool autoreset, SfEnv& e, SfStepOut& o) {
+// the key mask of an env's action at step t: given actions or the synthetic stream
+__device__ __forceinline__ int sf_step_keys(const SfDev& D, const SfRollArgs& A, int env, int t) {
   int a = A.actions ? A.actions[(size_t)t * D.n + env]
                     : sf_hash_action(A.action_seed, (unsigned long long)(D.first_global_env + env), (unsigned long long)(A.t0 + t), D.num_actions);
-  int km = (A.flags & SF_FLAG_ACTIONS_ARE_KEYMASKS) ? (a & 15) : D.keymask_of_action[min(max(a, 0), D.num_actions - 1)];
-  sf_env_step(D, H, env, e, km, autoreset, (A.flags & SF_FLAG_RAW_REWARD) != 0, o);
+  return (A.flags & SF_FLAG_ACTIONS_ARE_KEYMASKS) ? (a & 15) : D.keymask_of_action[min(max(a, 0), D.num_actions - 1)];
+}
+// a step's outputs at index t
+__device__ __forceinline__ void sf_store_step_out(const SfDev& D, const SfRollArgs& A, int env, int t, const SfStepOut& o) {
   size_t oi = (size_t)t * D.n + env;
   if (A.reward) A.reward[oi] = o.reward;
   if (A.done) A.done[oi] = o.done;
   if (A.fortkill) A.fortkill[oi] = o.fort_kill;
   if (A.events) A.events[oi] = o.events;
+}
+// one tick of one env (both step kernels; H: the step's tables): its action, the step, the step's outputs
+__device__ __forceinline__ void sf_tick_env(const SfDev& D, const SfHot* H, const SfRollArgs& A, int env, int t, bool autoreset, SfEnv& e, SfStepOut& o) {
+  const int km = sf_step_keys(D, A, env, t);
+  sf_env_step(D, H, env, e, km, autoreset, (A.flags & SF_FLAG_RAW_REWARD) != 0, o);
+  sf_store_step_out(D, A, env, t, o);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -526,12 +536,24 @@ __device__ __forceinline__ void sf_store_span(float* out, const float* S, int pr
 // ------------------------------------------------------------------------------------------------
 // state-only step (render off): one env per thread
 // ------------------------------------------------------------------------------------------------
-// FEAT: every tick also writes the feature row of each env's state after the tick (auto-reset included). In one tick the
-// rows of a block's envs are one contiguous span of the output: they are staged in shared memory (two buffers, so one
-// barrier per tick) and leave as consecutive stores across each warp. One thread storing its own row would scatter
-// 4-byte stores 4 * nfeat bytes apart: in HBM, and across PCIe where sf_step_host_features writes straight into a
-// page-locked host buffer (~1.7 ns per scattered store, profiles/r02_pcie_write_probe.txt).
 #define SF_STEP_ONLY_BLOCK 128
+// The feature rows of step t (both state-only step kernels, all threads of the block): each env's row of its state e.
+// In one step the rows of a block's envs are one contiguous span of the output: they are staged in shared memory (two
+// buffers, so one barrier per step) and leave as consecutive stores across each warp. One thread storing its own row
+// would scatter 4-byte stores 4 * nfeat bytes apart: in HBM, and across PCIe where sf_step_host_features writes straight
+// into a page-locked host buffer (~1.7 ns per scattered store, profiles/r02_pcie_write_probe.txt).
+__device__ __forceinline__ void sf_feature_rows(const SfDev& D, const SfRollArgs& A, const SfFeatArgs& F, const SfEnv& e, bool mine, int t) {
+  __shared__ __align__(16) float rows[2][SF_STEP_ONLY_BLOCK * 19 + 4];  // + 3: the span's offset within 16 bytes
+  float* R = rows[t & 1];
+  const int b0 = A.env0 + blockIdx.x * SF_STEP_ONLY_BLOCK;
+  float* span = F.out + ((size_t)t * D.n + b0) * F.cols;
+  const int pre = (int)(((uintptr_t)span >> 2) & 3);
+  if (mine) sf_feature_row(e, D.autoturn != 0, F.kind, R + pre + threadIdx.x * F.cols);
+  __syncthreads();
+  sf_store_span(span, R, pre, min(SF_STEP_ONLY_BLOCK, A.env0 + A.envn - b0) * F.cols);
+}
+
+// FEAT: every tick also writes the feature row of each env's state after the tick (auto-reset included, sf_feature_rows).
 template <bool FEAT>
 __global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_only_kernel(SfDev D, SfRollArgs A, SfFeatArgs F) {
   const int env = A.env0 + blockIdx.x * blockDim.x + threadIdx.x;
@@ -552,16 +574,53 @@ __global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_only_kernel(SfDev 
       if (finished) sf_new_game(D, &D.tab->hot, env, e);
     }
     if (mine && (t & 7) == 7) sf_flush_stats(D, env, e);  // the pending increments are 8-bit fields
-    if constexpr (FEAT) {
-      __shared__ __align__(16) float rows[2][SF_STEP_ONLY_BLOCK * 19 + 4];  // + 3: the span's offset within 16 bytes
-      float* R = rows[t & 1];
-      const int b0 = A.env0 + blockIdx.x * SF_STEP_ONLY_BLOCK;
-      float* span = F.out + ((size_t)t * D.n + b0) * F.cols;
-      const int pre = (int)(((uintptr_t)span >> 2) & 3);
-      if (mine) sf_feature_row(e, D.autoturn != 0, F.kind, R + pre + threadIdx.x * F.cols);
-      __syncthreads();
-      sf_store_span(span, R, pre, min(SF_STEP_ONLY_BLOCK, A.env0 + A.envn - b0) * F.cols);
+    if constexpr (FEAT) sf_feature_rows(D, A, F, e, mine, t);
+  }
+  if (mine) sf_store_env(D, env, e);
+}
+
+// ------------------------------------------------------------------------------------------------
+// action repeat (sf_set_action_repeat, k > 1): the state-only step, up to k ticks per agent step
+// ------------------------------------------------------------------------------------------------
+// Agent step t of an env ticks with the one key mask of its action until k ticks have run or one of them ends the
+// episode (gym's `frameskip`); index t of the outputs holds the sum of those ticks' rewards and the OR of their done, kill
+// and event bits, and FEAT's row t is the state after the agent step. The k iterations are warp-uniform (the loop ends
+// early only when no lane of the warp is still ticking), and a lane whose agent step is over just stops ticking: every
+// lane reaches the __any_sync of the episode accumulation. The pending Stats increments are 8-bit fields: they are
+// flushed every 8 iterations, that is every 8 ticks at most, whatever k is. A kernel of its own, with k a parameter:
+// sf_step_only_kernel keeps its code.
+template <bool FEAT>
+__global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDev D, SfRollArgs A, SfFeatArgs F, int repeat) {
+  const int env = A.env0 + blockIdx.x * blockDim.x + threadIdx.x;
+  const int lane = threadIdx.x & 31;
+  const bool mine = env < A.env0 + A.envn;
+  const bool autoreset = !(A.flags & SF_FLAG_NO_AUTORESET), raw = (A.flags & SF_FLAG_RAW_REWARD) != 0;
+  const SfHot* H = &D.tab->hot;
+  SfEnv e;
+  if (mine) sf_load_env(D, env, e);
+  int tick = 0;  // iterations run by this warp (the Stats flush cadence)
+  for (int t = 0; t < A.T; t++) {
+    const int km = mine ? sf_step_keys(D, A, env, t) : 0;
+    SfStepOut acc;
+    acc.reward = 0; acc.events = 0u; acc.done = false; acc.fort_kill = false;
+    bool ticking = mine;
+    for (int j = 0; j < repeat && __any_sync(0xffffffffu, ticking); j++, tick++) {
+      bool finished = false;
+      if (ticking) {
+        SfStepOut o;
+        sf_env_step(D, H, env, e, km, autoreset, raw, o);
+        acc.reward += o.reward; acc.events |= o.events; acc.fort_kill |= o.fort_kill;
+        acc.done = o.done; ticking = !o.done;
+        finished = o.done && autoreset;
+      }
+      if (__any_sync(0xffffffffu, finished)) {
+        sf_accumulate_episode(D, env, e, finished, lane);
+        if (finished) sf_new_game(D, H, env, e);
+      }
+      if (mine && (tick & 7) == 7) sf_flush_stats(D, env, e);
     }
+    if (mine) sf_store_step_out(D, A, env, t, acc);
+    if constexpr (FEAT) sf_feature_rows(D, A, F, e, mine, t);
   }
   if (mine) sf_store_env(D, env, e);
 }
@@ -815,6 +874,7 @@ struct sf_handle {
   int action_set;
   int gametype;  // 0 youturn 1 autoturn 2 test-youturn 3 test-autoturn
   int num_sms;
+  int action_repeat;  // ticks per agent step of every stepping entry point (sf_set_action_repeat), 1 by default
   void* slab;
   size_t slab_bytes;
   SfTables* h_tab;
@@ -938,6 +998,7 @@ extern "C" int sf_create(const char* gametype, int action_set, int n_envs, int d
   sf_handle* h = new sf_handle();
   memset(h, 0, sizeof(*h));
   h->device = device; h->num_sms = num_sms > 0 ? num_sms : 148; h->action_set = action_set; h->gametype = gt;
+  h->action_repeat = 1;
   SfDev& d = h->dev;
   d.n = n_envs; d.n_pad = (n_envs + 31) & ~31;
   d.autoturn = (gt == 1 || gt == 3);
@@ -1045,10 +1106,38 @@ static void group_shape(const sf_handle* h, int n, int* EB, int* ngroups, int* b
 }
 
 // The launch shape (EB, ngroups, sched) and the instantiation are chosen here; callers set the other fields. f: feature
-// rows (render off only).
+// rows (render off only). a.T counts agent steps.
 static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st, bool draw = false, SfFeatArgs f = {}) {
   const SfDev& d = h->dev;
   bool render = (a.flags & SF_FLAG_RENDER) && a.obs;
+  if (!draw && h->action_repeat > 1) {
+    // Action repeat: the state-only repeat kernel runs the ticks. Without frames it takes all T agent steps in one launch.
+    // With frames every agent step is two launches on `st`: the repeat kernel for that step (T = 1), then a draw of the
+    // state it left into the step's frame slot. (The fused kernel's stepping warp is its critical side already: k ticks
+    // per drawn tick would make it the bottleneck; DESIGN.md 4.6.)
+    const int blocks = (a.envn + SF_STEP_ONLY_BLOCK - 1) / SF_STEP_ONLY_BLOCK;
+    SfRollArgs s = a;
+    s.flags &= ~SF_FLAG_RENDER; s.obs = nullptr; s.host_obs = nullptr; s.mirror = nullptr; s.delta_stats = nullptr;
+    if (render) s.T = 1;
+    const size_t n = (size_t)d.n, per = (a.flags & SF_FLAG_NATIVE_OBS) ? (size_t)SF_NAT_H * SF_NAT_W : (size_t)84 * 84;
+    for (int t = 0; t < (render ? a.T : 1); t++) {
+      if (render) {  // agent step t alone: its slot of every time-major array
+        const size_t o = (size_t)t * n;
+        s.actions = a.actions ? a.actions + o : nullptr; s.t0 = a.t0 + t;
+        s.reward = a.reward ? a.reward + o : nullptr; s.done = a.done ? a.done + o : nullptr;
+        s.fortkill = a.fortkill ? a.fortkill + o : nullptr; s.events = a.events ? a.events + o : nullptr;
+      }
+      if (f.out) sf_step_repeat_kernel<true><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, h->action_repeat);
+      else sf_step_repeat_kernel<false><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, h->action_repeat);
+      CUDA_TRY(cudaGetLastError());
+      if (render) {
+        SfRollArgs r = {};
+        r.T = 1; r.obs = a.obs + (size_t)t * n * per; r.flags = a.flags; r.env0 = a.env0; r.envn = a.envn;
+        if (int rc = launch_rollout(h, r, st, true)) return rc;
+      }
+    }
+    return SF_OK;
+  }
   if (render) {
     int blocks;
     group_shape(h, a.envn, &a.EB, &a.ngroups, &blocks);
@@ -1235,6 +1324,14 @@ extern "C" int sf_rollout_features(sf_handle* h, int obs_type, int T, const int3
   return launch_rollout(h, a, (cudaStream_t)stream, false, SfFeatArgs{d_features, obs_type, nf});
 }
 
+extern "C" int sf_set_action_repeat(sf_handle* h, int k) {
+  if (!h) return fail(SF_ERR_INVALID, "handle is NULL");
+  if (k < 1 || k > SF_MAX_ACTION_REPEAT) return fail(SF_ERR_INVALID, "action repeat must be in [1, " + std::to_string(SF_MAX_ACTION_REPEAT) + "]");
+  h->action_repeat = k;
+  return SF_OK;
+}
+extern "C" int sf_action_repeat(const sf_handle* h) { return h ? h->action_repeat : -1; }
+
 extern "C" int sf_synthetic_action(uint32_t action_seed, long long global_env, long long t, int num_actions) {
   return sf_hash_action(action_seed, (unsigned long long)global_env, (unsigned long long)t, num_actions);
 }
@@ -1310,7 +1407,8 @@ static int step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_obs, flo
     }
   }
   const bool delta = want_delta && mir->host == h_obs && mir->bytes == obs_bytes;
-  const bool fused_delta = delta && per % 16 == 0;  // the blocks of the step kernel send their own frames' changes
+  // the blocks of the step kernel send their own frames' changes (with action repeat the frames come from a draw launch)
+  const bool fused_delta = delta && per % 16 == 0 && h->action_repeat == 1;
   CUDA_TRY(cudaStreamSynchronize(cudaStreamLegacy));  // calls made with stream == NULL (sf_reset, sf_seed ...) come first
   // page-locked actions / rewards / dones / kills / events are read and written in place by the kernel
   const int* k_actions = (const int*)device_alias(h_actions);

@@ -48,7 +48,7 @@ def _torch():
 class SFVecEnv(object):
     def __init__(self, env_id="SpaceFortress-youturn-image-v0", num_envs=16, device=0, action_set=1, seeds=None,
                  render=True, native_obs=False, autoreset=True, first_global_env=0, copy_outputs=False, obs_type="image",
-                 host_delta=True):
+                 host_delta=True, action_repeat=1):
         """copy_outputs (numpy path): False = step() returns views of the env's page-locked output buffers, which the
         next step() overwrites, and `infos` as a bool ndarray (the fast path); True = fresh arrays every step and
         `infos` as a tuple of N bools, exactly what gym_vecenv's np.stack returns; "ring" (SubprocVecEnv / DummyVecEnv
@@ -61,7 +61,11 @@ class SFVecEnv(object):
         sf_rollout_features), one launch per step or rollout.
         host_delta (numpy path): the frames reach the page-locked observation buffer as SF_FLAG_HOST_DELTA updates (only
         the bytes that changed since the previous step cross PCIe; the buffer's contents are those of a full copy). The
-        views step() returns are then read-only, because the next update builds on them. False: whole frames every step."""
+        views step() returns are then read-only, because the next update builds on them. False: whole frames every step.
+        action_repeat: game ticks per agent step (gym's `frameskip`, sf_set_action_repeat): every step() and each of the T
+        steps of rollout(T) repeats its action for up to action_repeat ticks, stopping at the tick an episode ends; the
+        reward is the sum over those ticks, done / infos / events are set by any of them, and the observation is that of
+        the state after the last one. 1 (default) is the plain one-tick step."""
         self.L = _lib.lib()
         self.gametype = _gametype(env_id)
         self.num_envs = int(num_envs)
@@ -81,6 +85,13 @@ class SFVecEnv(object):
         h = C.c_void_p()
         _lib.check(self.L.sf_create(self.gametype.encode(), int(action_set), self.num_envs, self.device_index, C.byref(h)))
         self.h = h
+        self.action_repeat = int(action_repeat)
+        rc = self.L.sf_set_action_repeat(self.h, self.action_repeat)
+        if rc != _lib.SF_OK:
+            msg = self.L.sf_last_error()
+            self.L.sf_destroy(self.h)
+            self.h = None
+            raise ValueError("action_repeat must be in [1, %d]: %s" % (_lib.MAX_ACTION_REPEAT, msg.decode() if msg else "?"))
         self.num_actions = self.L.sf_num_actions(self.h)
         self.action_space = Discrete(self.num_actions)
         self.obs_shape = (1, _lib.NATIVE_H, _lib.NATIVE_W) if native_obs else (1, _lib.OBS_H, _lib.OBS_W)
