@@ -3,66 +3,25 @@ inputs. Bars (BASELINE.json north_star): integer state / events / episode bounda
 kinematics <= 1e-5 relative per step when teacher-forced (observed: bit-exact except shells, which carry the
 device cos/sin); frames >= 99.9 % identical pixels with max |delta| <= 2 (observed: bit-exact)."""
 import ctypes as C
-import json
 import os
 
 import numpy as np
 import pytest
 
 from conftest import scripted_kill_policy
+from gpu_helpers import END_TICK, GAMETYPES, assert_frame_close, assert_state_close, make, stagger, to_oracle_record, torch_cuda
 from oracle.oracle import OracleEnv, Record, draw_native, draw_obs
 
 pytestmark = pytest.mark.gpu
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-GAMETYPES = ["youturn", "autoturn", "test-youturn", "test-autoturn"]
-FLOAT_REL_TOL = 1e-5  # north_star: continuous kinematics within 1e-5 relative per step
-FRAME_MATCH_FRACTION = 0.999
-FRAME_MAX_DELTA = 2
-
-
-def torch_cuda():
-    import torch
-    if not torch.cuda.is_available():
-        pytest.skip("no CUDA device")
-    return torch
-
-
-def make(gametype, n, **kw):
-    torch_cuda()
-    from spacefortress_b200 import SFVecEnv
-    return SFVecEnv(gametype, num_envs=n, device=0, **kw)
-
-
-def to_oracle_record(g):
-    r = Record()
-    C.memmove(C.byref(r), C.byref(g), C.sizeof(Record))
-    return r
-
-
-def assert_state_close(o, g, ctx):
-    assert o.int_state() == to_oracle_record(g).int_state(), ctx
-    assert list(o.stats) == list(g.stats), ctx
-    fo, fg = o.float_state(), to_oracle_record(g).float_state()
-    for k in fo:
-        a, b = np.atleast_1d(np.array(fo[k], dtype=np.float64)), np.atleast_1d(np.array(fg[k], dtype=np.float64))
-        if k.startswith("shell_"):
-            assert np.all(np.abs(a - b) <= FLOAT_REL_TOL * np.maximum(1.0, np.abs(a))), (ctx, k, a, b)
-        else:
-            assert np.array_equal(a, b), (ctx, k, a, b)  # everything not touched by device cos/sin is bit-exact
-
-
-def assert_frame_close(expected, got, ctx):
-    d = np.abs(expected.astype(np.int32) - got.astype(np.int32))
-    assert d.max() <= FRAME_MAX_DELTA, (ctx, int(d.max()))
-    assert (d == 0).mean() >= FRAME_MATCH_FRACTION, (ctx, float((d == 0).mean()))
 
 
 @pytest.mark.parametrize("gametype", GAMETYPES)
 def test_free_running_trace_parity(gametype):
     n, T = 48, 700
     seeds = np.arange(1, n + 1)
-    env = make(gametype, n, seeds=seeds)
+    env = make(gametype, n, seeds=seeds, reset=False)
     obs = env.reset()
     orc = [OracleEnv(gametype, int(s)) for s in seeds]
     for i in range(n):
@@ -90,7 +49,6 @@ def test_config1_youturn_single_env_10k_steps_with_frames():
     torch = torch_cuda()
     T = 10000
     env = make("youturn", 1)
-    env.reset()
     o = OracleEnv("youturn", 1)
     rng = np.random.RandomState(2)
     actions = rng.randint(0, 5, size=(T, 1)).astype(np.int32)
@@ -116,8 +74,8 @@ def test_golden_fixtures_replayed_on_gpu():
     for name in ("youturn", "autoturn", "test-youturn", "test-autoturn", "autoturn_kill"):
         z = np.load(os.path.join(GOLD, "trace_%s.npz" % name))
         gametype = "autoturn" if name == "autoturn_kill" else name
-        from spacefortress_b200 import SFVecEnv, _lib
-        env = SFVecEnv(gametype, num_envs=1, device=0, render=False)
+        from spacefortress_b200 import _lib
+        env = make(gametype, 1, render=False, reset=False)
         env._flags |= _lib.FLAG_ACTIONS_ARE_KEYMASKS
         env.reset()
         T = len(z["keymask"])
@@ -136,7 +94,7 @@ def test_golden_fixtures_replayed_on_gpu():
 
 
 def test_kill_path_and_events():
-    env = make("autoturn", 4, render=False)
+    env = make("autoturn", 4, render=False, reset=False)
     from spacefortress_b200 import _lib
     env._flags |= _lib.FLAG_ACTIONS_ARE_KEYMASKS
     env.reset()
@@ -159,7 +117,7 @@ def test_teacher_forced_single_steps():
     """load state -> one step -> compare (kinematics tolerance 1e-5 relative, ints exact)."""
     n = 64
     for gametype in ("youturn", "autoturn"):
-        env = make(gametype, n, render=False)
+        env = make(gametype, n, render=False, reset=False)
         from spacefortress_b200 import _lib
         env._flags |= _lib.FLAG_ACTIONS_ARE_KEYMASKS
         env.reset()
@@ -198,7 +156,6 @@ def test_frames_from_crafted_states():
     all vulnerability bar states."""
     n = 40
     env = make("youturn", n)
-    env.reset()
     rng = np.random.RandomState(4)
     recs = []
     for i in range(n):
@@ -237,7 +194,6 @@ def test_explosion_all_phases_and_box_cache():
     and resampled-box memo paths and must give the same frames."""
     n = 512
     env = make("autoturn", n)
-    env.reset()
     rng = np.random.RandomState(11)
     recs = []
     for i in range(n):
@@ -269,7 +225,7 @@ def test_explosion_all_phases_and_box_cache():
 def test_rollout_equals_stepwise_and_synthetic_stream():
     torch = torch_cuda()
     n, T = 96, 64
-    a = make("youturn", n); b = make("youturn", n)
+    a = make("youturn", n, reset=False); b = make("youturn", n, reset=False)
     a.reset(); b.reset()
     acts = a.synthetic_actions(T, action_seed=5)
     out = a.rollout(T, action_seed=5)  # device-side hash policy
@@ -305,7 +261,7 @@ def test_rollout_with_many_strokes_and_odd_lengths_equals_stepwise():
             r.shell_vx[s] = 6 * np.cos(np.deg2rad(ang)); r.shell_vy[s] = 6 * np.sin(np.deg2rad(ang))
         recs.append(to_gpu_record(r))
     for T in (1, 2, 5, 8):
-        a = make("youturn", n); b = make("youturn", n)
+        a = make("youturn", n, reset=False); b = make("youturn", n, reset=False)
         a.reset(); b.reset()
         a.set_state(recs); b.set_state(recs)
         acts = a.synthetic_actions(T, action_seed=9)
@@ -317,7 +273,7 @@ def test_rollout_with_many_strokes_and_odd_lengths_equals_stepwise():
         assert bytes(a.get_state()) == bytes(b.get_state())
         a.close(); b.close()
     # and the first frames against the oracle
-    a = make("youturn", n); a.reset(); a.set_state(recs)
+    a = make("youturn", n); a.set_state(recs)
     obs = a.render_frames(native=False)
     for i in range(0, n, 7):
         assert_frame_close(draw_obs(to_oracle_record(recs[i])), obs[i], ("crowded", i))
@@ -330,7 +286,7 @@ def test_soak_fused_rollout_equals_single_steps_many_envs():
     drawing warps, or between two stages, would show up as a sporadic mismatch). tools/gpu_soak.py runs longer."""
     torch = torch_cuda()
     n, T = 4096, 64
-    a = make("autoturn", n); b = make("autoturn", n)
+    a = make("autoturn", n, reset=False); b = make("autoturn", n, reset=False)
     a.reset(to_numpy=False); b.reset(to_numpy=False)
     g = torch.Generator(device="cuda"); g.manual_seed(3)
     for chunk in range(3):
@@ -349,9 +305,9 @@ def test_shard_invariance_two_slabs_equal_one():
     episode statistics add up."""
     n, T = 64, 150
     seeds = np.arange(1, n + 1)
-    whole = make("autoturn", n, seeds=seeds)
-    lo = make("autoturn", n // 2, seeds=seeds[:n // 2], first_global_env=0)
-    hi = make("autoturn", n // 2, seeds=seeds[n // 2:], first_global_env=n // 2)
+    whole = make("autoturn", n, seeds=seeds, reset=False)
+    lo = make("autoturn", n // 2, seeds=seeds[:n // 2], first_global_env=0, reset=False)
+    hi = make("autoturn", n // 2, seeds=seeds[n // 2:], first_global_env=n // 2, reset=False)
     for e in (whole, lo, hi):
         e.reset()
     ow = whole.rollout(T, action_seed=9); ol = lo.rollout(T, action_seed=9); oh = hi.rollout(T, action_seed=9)
@@ -369,7 +325,6 @@ def test_auto_reset_and_episode_stats():
     torch = torch_cuda()
     n = 8
     env = make("autoturn", n, seeds=np.arange(1, n + 1))
-    env.reset()
     orc = [OracleEnv("autoturn", s) for s in range(1, n + 1)]
     T = 5295
     acts = env.synthetic_actions(T, action_seed=1)
@@ -406,11 +361,8 @@ def test_staggered_episode_ends_auto_reset_and_stats():
     the episode statistics must equal the oracle's, step by step."""
     torch = torch_cuda()
     n, T = 24, 48
-    rng = np.random.RandomState(3)
-    ticks = (5295 - 1 - rng.randint(0, 40, size=n)).astype(np.int32)
     env = make("youturn", n, seeds=np.arange(1, n + 1))
-    env.reset()
-    env.set_ticks(ticks)
+    ticks = stagger(env, 1 + np.random.RandomState(3).randint(0, 40, size=n))
     orc = [OracleEnv("youturn", s) for s in range(1, n + 1)]
     for i in range(n):
         r = orc[i].get_state(); r.tick = int(ticks[i]); r.time = int(ticks[i]) * 34; orc[i].set_state(r)
@@ -423,7 +375,7 @@ def test_staggered_episode_ends_auto_reset_and_stats():
             r, d, k, _ = orc[i].step(orc[i].keymask(int(acts[t, i])))
             assert r == int(rew[t, i]) and bool(d) == bool(done[t, i]), (i, t)
             if d:
-                assert t == 5295 - 1 - int(ticks[i]), (i, t)
+                assert t == END_TICK - 1 - int(ticks[i]), (i, t)
                 episodes += 1; sum_len += orc[i].get_state().tick
                 orc[i].reset()
             if d or t % 11 == 0:
@@ -484,7 +436,7 @@ def test_policy_input_kernel_matches_the_torch_stack(dtype):
     tol = 0.06 if dtype == "bf16" else 2e-3
     tf = (torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32)
     torch.backends.cudnn.allow_tf32 = False; torch.backends.cuda.matmul.allow_tf32 = False
-    env = make("youturn", n)
+    env = make("youturn", n, reset=False)
     policy = SFGRUPolicy(env.num_actions).cuda().eval().to(dt)
     ro = OnDeviceRollout(env, policy, num_steps=6)
     assert ro.fused_input
@@ -512,14 +464,12 @@ def test_on_device_rollout_frame_stack_matches_reference_loop():
     """OnDeviceRollout (config 3 plumbing): the 4-frame window over the single-frame buffer equals the
     reference's running `current_obs` (rl/train.py:51-56,92-97: zero the stack on done, shift, append)."""
     torch = torch_cuda()
-    from spacefortress_b200 import SFVecEnv
     from spacefortress_b200.rollout import OnDeviceRollout, SFGRUPolicy
     n, T = 6, 24
-    env = SFVecEnv("youturn", num_envs=n, device=0)
-    env.reset()
+    env = make("youturn", n)
     recs = env.get_state()
     for i in range(n):  # stagger the episode ends so that dones fall inside the rollout
-        recs[i].tick = 5295 - 3 - 2 * i
+        recs[i].tick = END_TICK - 3 - 2 * i
         recs[i].time = recs[i].tick * 34
     env.set_state(recs)
     torch.manual_seed(0)
@@ -559,7 +509,6 @@ def test_graphed_rollout_equals_the_eager_one():
     """OnDeviceRollout(graph=True) replays one CUDA graph per step index: with a deterministic policy it produces the
     same actions, frames, rewards and values as the eager loop, over two consecutive rollouts (history carry-over)."""
     torch = torch_cuda()
-    from spacefortress_b200 import SFVecEnv
     from spacefortress_b200.rollout import OnDeviceRollout, SFGRUPolicy
 
     class Greedy(SFGRUPolicy):
@@ -569,7 +518,7 @@ def test_graphed_rollout_equals_the_eager_one():
     n, T = 96, 6
     outs = []
     for graph in (False, True):
-        env = SFVecEnv("youturn", num_envs=n, device=0)
+        env = make("youturn", n, reset=False)
         torch.manual_seed(3)
         ro = OnDeviceRollout(env, Greedy(env.num_actions).cuda().eval(), num_steps=T, graph=graph)
         got = []
@@ -590,7 +539,7 @@ def test_ppo_update_on_an_on_device_rollout():
     from spacefortress_b200.rollout import OnDeviceRollout, SFGRUPolicy
     from spacefortress_b200.ppo import PPOLearner
     n, T = 64, 8
-    env = make("youturn", n)
+    env = make("youturn", n, reset=False)
     policy = SFGRUPolicy(env.num_actions).cuda()
     ro = OnDeviceRollout(env, policy, num_steps=T)
     ro.collect()

@@ -1,10 +1,10 @@
 """GPU (-m gpu): sf_reset with an env mask. The Python layer always resets every env, so this calls the C-ABI directly.
 A masked-in env starts a new game and its first frame is drawn; a masked-out env keeps its state and its frame bytes are
 not written. The batch is large enough that blocks own more than one group of envs."""
-import ctypes as C
-
 import numpy as np
 import pytest
+
+from gpu_helpers import torch_cuda, vp
 
 pytestmark = pytest.mark.gpu
 
@@ -13,9 +13,7 @@ SENTINEL = 0xA5
 
 @pytest.mark.parametrize("native", [False, True])
 def test_reset_mask_draws_only_masked_envs(native):
-    import torch
-    if not torch.cuda.is_available():
-        pytest.skip("no CUDA device")
+    torch = torch_cuda()
     from spacefortress_b200 import SFVecEnv, _lib
     n = 5000  # > 148 SMs x 32 envs: more groups than blocks
     env = SFVecEnv("youturn", num_envs=n, device=0, native_obs=native)
@@ -32,8 +30,7 @@ def test_reset_mask_draws_only_masked_envs(native):
         h, w = (_lib.NATIVE_H, _lib.NATIVE_W) if native else (_lib.OBS_H, _lib.OBS_W)
         obs = torch.full((n, h, w), SENTINEL, dtype=torch.uint8, device="cuda")
         flags = _lib.FLAG_NATIVE_OBS if native else 0
-        _lib.check(env.L.sf_reset(env.h, C.c_void_p(d_mask.data_ptr()), 1, C.c_void_p(obs.data_ptr()), flags,
-                                  C.c_void_p(torch.cuda.current_stream().cuda_stream)))
+        _lib.check(env.L.sf_reset(env.h, vp(d_mask), 1, vp(obs), flags, torch.cuda.current_stream().cuda_stream))
         torch.cuda.synchronize()
         got = obs.cpu().numpy()
         ref = env.render_frames(native=native)

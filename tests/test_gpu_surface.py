@@ -6,16 +6,10 @@ episode statistics)."""
 import numpy as np
 import pytest
 
+from gpu_helpers import END_TICK, stagger, to_oracle_record, torch_cuda
 from oracle.oracle import OracleEnv, RefEnv, ref_available
 
 pytestmark = pytest.mark.gpu
-
-
-def torch_cuda():
-    import torch
-    if not torch.cuda.is_available():
-        pytest.skip("no CUDA device")
-    return torch
 
 
 def oracle_features(o, kind, youturn):
@@ -247,11 +241,10 @@ def test_host_delta_updates_equal_whole_frame_copies(gametype, native, n):
     from spacefortress_b200 import SFVecEnv
     a = SFVecEnv(gametype, num_envs=n, device=0, native_obs=native)                      # delta
     b = SFVecEnv(gametype, num_envs=n, device=0, native_obs=native, host_delta=False)    # whole frames
-    ticks = (5295 - 1 - (np.arange(n) % 37)).astype(np.int32)
     rng = np.random.RandomState(3)
     for e in (a, b):
         e.reset()
-        e.set_ticks(ticks)
+        stagger(e, 1 + np.arange(n) % 37)
     per = a.obs_shape[1] * a.obs_shape[2]
     resets = 0
     for t in range(60):
@@ -422,7 +415,7 @@ def test_config5_episode_stats_equal_host_sums():
     env = SFVecEnv("youturn", num_envs=n, device=0)
     env.reset(to_numpy=False)
     rng = np.random.RandomState(0)
-    ticks = rng.randint(5295 - T - 8, 5295, size=n).astype(np.int32)   # most envs finish inside the rollout
+    ticks = rng.randint(END_TICK - T - 8, END_TICK, size=n).astype(np.int32)   # most envs finish inside the rollout
     env.set_ticks(ticks)
     env.episode_stats(reset=True)
     out = env.rollout(T, action_seed=2)
@@ -443,7 +436,7 @@ def test_config5_episode_stats_equal_host_sums():
     assert st["sum_return"] == int(ret.sum())
     assert st["sum_return_sq"] == int((ret * ret).sum())
     assert st["fort_kills"] == int(kl.sum())
-    assert st["sum_length"] == 5295 * int(fin.sum())
+    assert st["sum_length"] == END_TICK * int(fin.sum())
     # frames of the step after a reset are first frames of a new episode (all envs share seed 1 -> the same spawn order
     # per env index): spot-check one finished env against its oracle
     env.close()
@@ -494,14 +487,14 @@ def test_installed_glyph_masks_are_drawn_by_kernels_and_oracle_alike():
             frames = env.render_frames(native=native)
             frames2 = env.render_frames(native=native)   # second pass: explosion memo path
             for i in range(n):
-                r = O.Record(); import ctypes as C; C.memmove(C.byref(r), C.byref(recs[i]), C.sizeof(O.Record))
+                r = to_oracle_record(recs[i])
                 exp = O.draw_native(r) if native else O.draw_obs(r)
                 assert np.array_equal(frames[i], exp) and np.array_equal(frames2[i], exp), (native, i)
         assert env.render_frames(native=True)[1][1:6, 32:59].max() > 0
         # stepping (cached boxes, score windows) with the installed masks
         oracles = [O.OracleEnv("youturn", 1) for _ in range(n)]
         for i in range(n):
-            r = O.Record(); C.memmove(C.byref(r), C.byref(recs[i]), C.sizeof(O.Record)); oracles[i].set_state(r)
+            oracles[i].set_state(to_oracle_record(recs[i]))
         for t in range(12):
             a = rng.randint(env.num_actions, size=n)
             obs, _, _, _ = env.step(a)
