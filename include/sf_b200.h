@@ -58,7 +58,8 @@ enum {
   SF_EV_COL_SHELL_SHIP = 1 << 15,
   SF_EV_PRESS_FIRE = 1 << 16, SF_EV_PRESS_THRUST = 1 << 17, SF_EV_PRESS_LEFT = 1 << 18, SF_EV_PRESS_RIGHT = 1 << 19,
   SF_EV_MISSED_SHOT = 1 << 20,
-  SF_EV_EPISODE_RESET = 1 << 21 /* the env was auto-reset after this step */
+  SF_EV_EPISODE_RESET = 1 << 21, /* the env was auto-reset after this step */
+  SF_EV_STICKY = 1 << 22         /* sticky actions: a tick of this agent step kept the held keys (sf_set_sticky_actions) */
 };
 
 /* sf_step / sf_rollout flags */
@@ -167,6 +168,37 @@ int sf_synthetic_action(uint32_t action_seed, long long global_env, long long t,
 #define SF_MAX_ACTION_REPEAT 5295
 int sf_set_action_repeat(sf_handle* h, int k);
 int sf_action_repeat(const sf_handle* h);
+
+/* Extension: sticky actions (ALE's repeat_action_probability, Machado et al. 2018; Gymnasium ALE v5 and EnvPool default
+ * to 0.25). A handle setting (p, sticky_seed), default p = 0, which is the plain step bit for bit. With p > 0 every
+ * executed tick of every env makes one draw before its key processing:
+ *     u = hash(sticky_seed, global_env, ((uint64)rng_count << 32) | tick)
+ * (written out: c = rng_count << 32 | (uint32)tick; z = global_env * 0x9E3779B97F4A7C15 ^ c * 0xC2B2AE3D27D4EB4F ^
+ * (sticky_seed << 32 | 0x57) in uint64; z ^= z >> 30; z *= 0xBF58476D1CE4E5B9; z ^= z >> 27; z *= 0x94D049BB133111EB;
+ * z ^= z >> 31; u = z >> 32: the synthetic action hash with 0x57 in place of its 0x5F)
+ * with global_env = first_global_env + i (the label of the synthetic action stream) and rng_count / tick the env's
+ * PRE-tick values (rand() calls consumed, Game::mTick; sf_state_record.rng_count / .tick). The previous keys stick iff
+ * (uint64)u < llround(p * 2^32): p = 0 never sticks, p = 1 always does. If they stick, the tick runs with the key mask
+ * the env already holds (the FIRE / THRUST / LEFT / RIGHT flags of the state), otherwise with the agent's key mask. Every
+ * key is sent every tick, so a sticky tick is a tick without press or release edges; fire stays edge-triggered.
+ * With action repeat k the draw happens on each of the up-to-k ticks: the switch to a new action is delayed by a
+ * geometric number of ticks. After an auto-reset the new game holds no keys, so a sticky first tick of an episode is
+ * "no keys" (ALE resets its previous action to NOOP). SF_EV_STICKY is set on an agent step when any of its executed ticks
+ * drew "stick", even if the held keys equal the action's. SF_FLAG_ACTIONS_ARE_KEYMASKS, SF_FLAG_NO_AUTORESET,
+ * SF_FLAG_RAW_REWARD and the synthetic stream work as before: the draw applies after the action became a key mask.
+ * The draw is a function of the env's state, not a counter: (rng_count, tick) never repeats within an env's life (tick
+ * rises within an episode and every new game consumes rand() calls) except after an explicit rewind (sf_seed,
+ * sf_set_ticks, sf_set_state), where repeating a draw is intended. So there is no per-env sticky state and no blob
+ * change: a restored env (sf_load_envs) continues with exactly the draws it would have made, given the same (p, seed,
+ * first_global_env); a fork into another slot has another label and diverges; results do not depend on the sharding
+ * over GPUs. The hash differs from the synthetic action hash: sticky_seed == action_seed gives uncorrelated draws.
+ * The setting applies to sf_step, sf_rollout, sf_step_host, sf_rollout_features and sf_step_host_features; sf_reset,
+ * sf_render, sf_features, the env blobs and sf_episode_stats do not depend on it. p not finite or outside [0, 1] ->
+ * SF_ERR_INVALID, setting unchanged. sf_sticky_actions returns p, -1 for a NULL handle. sf_sticky_draw (host only, no
+ * GPU needed) is the device's draw: 1 if the keys stick, 0 if not, -1 for a p outside [0, 1]. */
+int sf_set_sticky_actions(sf_handle* h, double p, uint32_t seed);
+double sf_sticky_actions(const sf_handle* h);
+int sf_sticky_draw(uint32_t seed, long long global_env, uint32_t rng_count, int32_t tick, double p);
 
 /* Render the current state without stepping (Game.draw + gray + resize). */
 int sf_render(sf_handle* h, uint8_t* d_obs, int flags, void* stream);

@@ -35,6 +35,7 @@ EVENT_BITS = {
 }
 COLLISION_BITS = {"bighex": 1 << 12, "smallhex": 1 << 13, "missile": 1 << 14, "shell": 1 << 15}
 EV_EPISODE_RESET = 1 << 21
+EV_STICKY = 1 << 22  # SF_EV_STICKY: a tick of the agent step kept the held keys (sticky actions)
 
 EPISODE_STAT_NAMES = ["episodes", "sum_return", "sum_return_sq", "sum_length", "bigHexDeaths", "smallHexDeaths",
                       "shellDeaths", "shipDeaths", "resets", "destroyedFortresses", "missedShots", "totalShots",
@@ -92,6 +93,9 @@ _PROTOTYPES = {
     "sf_synthetic_action": (C.c_int, [C.c_uint32, C.c_longlong, C.c_longlong, C.c_int]),
     "sf_set_action_repeat": (C.c_int, [C.c_void_p, C.c_int]),
     "sf_action_repeat": (C.c_int, [C.c_void_p]),
+    "sf_set_sticky_actions": (C.c_int, [C.c_void_p, C.c_double, C.c_uint32]),
+    "sf_sticky_actions": (C.c_double, [C.c_void_p]),
+    "sf_sticky_draw": (C.c_int, [C.c_uint32, C.c_longlong, C.c_uint32, C.c_int32, C.c_double]),
     "sf_render": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "sf_step_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "sf_host_delta_stats": (C.c_int, [C.c_void_p, C.c_void_p]),

@@ -16,6 +16,7 @@
 //                               env and tick (sf_rollout_features, sf_step_host_features).
 //   sf_step_repeat_kernel       action repeat (sf_set_action_repeat, k > 1): the state-only step with up to k ticks of one
 //                               action per agent step; with frames each agent step is followed by a SF_ROLL_DRAW launch.
+//                               <*, true>: sticky actions (sf_set_sticky_actions, p > 0), at any k.
 //   sf_features_kernel          the feature observation types of ssf_env.py:95-157 of the current state, one env per thread.
 //   sf_policy_input_kernel      4-frame stack -> the policy's first-layer input (bf16 or fp32, space-to-depth NHWC).
 //   sf_reset_kernel / sf_seed_kernel / sf_get_state_kernel / sf_set_state_kernel / sf_pack_static_kernel
@@ -25,6 +26,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -41,8 +43,8 @@
 // ------------------------------------------------------------------------------------------------
 // synthetic policy: stateless counter hash (SURVEY.md §8(d)); same function on host and device
 // ------------------------------------------------------------------------------------------------
-__host__ __device__ inline unsigned sf_hash3(unsigned seed, unsigned long long env, unsigned long long t) {
-  unsigned long long z = (env * 0x9E3779B97F4A7C15ull) ^ (t * 0xC2B2AE3D27D4EB4Full) ^ ((unsigned long long)seed << 32 | 0x5Fu);
+__host__ __device__ inline unsigned sf_hash3(unsigned seed, unsigned long long env, unsigned long long t, unsigned salt = 0x5Fu) {
+  unsigned long long z = (env * 0x9E3779B97F4A7C15ull) ^ (t * 0xC2B2AE3D27D4EB4Full) ^ ((unsigned long long)seed << 32 | salt);
   z ^= z >> 30; z *= 0xBF58476D1CE4E5B9ull;
   z ^= z >> 27; z *= 0x94D049BB133111EBull;
   z ^= z >> 31;
@@ -50,6 +52,14 @@ __host__ __device__ inline unsigned sf_hash3(unsigned seed, unsigned long long e
 }
 __host__ __device__ inline int sf_hash_action(unsigned seed, unsigned long long env, unsigned long long t, int num_actions) {
   return (int)(((unsigned long long)sf_hash3(seed, env, t) * (unsigned)num_actions) >> 32);
+}
+// Sticky actions (sf_set_sticky_actions): does the tick of env `env` whose pre-tick rand() count and tick are (rng_count,
+// tick) keep the keys the env holds? threshold = llround(p * 2^32). Keyed on the env's state, not on a counter: the pair
+// never repeats within an env's life, so a restored env makes the draws it would have made. Its own salt: with
+// sticky_seed == action_seed the draws are not the synthetic actions' hash.
+#define SF_STICKY_SALT 0x57u
+__host__ __device__ inline bool sf_sticky_hash(unsigned seed, unsigned long long env, unsigned rng_count, int tick, unsigned long long threshold) {
+  return (unsigned long long)sf_hash3(seed, env, (unsigned long long)rng_count << 32 | (unsigned)tick, SF_STICKY_SALT) < threshold;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -145,6 +155,11 @@ struct SfRollArgs {
 struct SfFeatArgs {
   float* out;      // NULL: no feature rows
   int kind, cols;  // SF_OBS_FEATURES / SF_OBS_NORMALIZED_FEATURES / SF_OBS_MONITORS, sf_feature_cols
+};
+// Sticky actions: a parameter of the repeat kernel of its own, for the same reason as SfFeatArgs
+struct SfStickyArgs {
+  unsigned long long threshold;  // llround(p * 2^32): 0 never sticks, 2^32 always
+  unsigned seed;
 };
 enum SfRollMode { SF_ROLL_STEP, SF_ROLL_STEP_HOST_DELTA, SF_ROLL_DRAW };
 // ticks per group, for both roles of a launch: a draw is the one frame of the current state
@@ -589,8 +604,13 @@ __global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_only_kernel(SfDev 
 // lane reaches the __any_sync of the episode accumulation. The pending Stats increments are 8-bit fields: they are
 // flushed every 8 iterations, that is every 8 ticks at most, whatever k is. A kernel of its own, with k a parameter:
 // sf_step_only_kernel keeps its code.
-template <bool FEAT>
-__global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDev D, SfRollArgs A, SfFeatArgs F, int repeat) {
+// STICKY (sf_set_sticky_actions): before each executed tick the env draws (sf_sticky_hash of its pre-tick rand() count
+// and tick); on "stick" the tick runs with the keys the env holds instead of the action's, so it has no press or release
+// edges, and the agent step reports SF_EV_STICKY.
+static_assert(SF_CORE_FIRE == SF_KEY_FIRE << 23 && SF_CORE_THRUST == SF_KEY_THRUST << 23 && SF_CORE_LEFT == SF_KEY_LEFT << 23 &&
+              SF_CORE_RIGHT == SF_KEY_RIGHT << 23, "the held keys are the key mask at bit 23 of the core word");
+template <bool FEAT, bool STICKY>
+__global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDev D, SfRollArgs A, SfFeatArgs F, int repeat, SfStickyArgs S) {
   const int env = A.env0 + blockIdx.x * blockDim.x + threadIdx.x;
   const int lane = threadIdx.x & 31;
   const bool mine = env < A.env0 + A.envn;
@@ -607,8 +627,15 @@ __global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDe
     for (int j = 0; j < repeat && __any_sync(0xffffffffu, ticking); j++, tick++) {
       bool finished = false;
       if (ticking) {
+        int keys = km;
+        if constexpr (STICKY) {
+          if (sf_sticky_hash(S.seed, (unsigned long long)(D.first_global_env + env), (unsigned)e.st3.z, e.q3.z, S.threshold)) {
+            keys = ((unsigned)e.q0.x >> 23) & 15;
+            acc.events |= SF_EV_STICKY;
+          }
+        }
         SfStepOut o;
-        sf_env_step(D, H, env, e, km, autoreset, raw, o);
+        sf_env_step(D, H, env, e, keys, autoreset, raw, o);
         acc.reward += o.reward; acc.events |= o.events; acc.fort_kill |= o.fort_kill;
         acc.done = o.done; ticking = !o.done;
         finished = o.done && autoreset;
@@ -875,6 +902,8 @@ struct sf_handle {
   int gametype;  // 0 youturn 1 autoturn 2 test-youturn 3 test-autoturn
   int num_sms;
   int action_repeat;  // ticks per agent step of every stepping entry point (sf_set_action_repeat), 1 by default
+  double sticky_p;      // sf_set_sticky_actions: p, and the kernel's form of (p, seed); 0 by default
+  SfStickyArgs sticky;
   void* slab;
   size_t slab_bytes;
   SfTables* h_tab;
@@ -1105,13 +1134,19 @@ static void group_shape(const sf_handle* h, int n, int* EB, int* ngroups, int* b
   *blocks = std::min(*ngroups, sms);
 }
 
+// Whether the stepping entry points run their ticks in sf_step_repeat_kernel (action repeat k > 1, or sticky actions
+// with p > 0) rather than in the kernels of the plain one-tick step. With frames they then come from draw launches.
+// (A p below 2^-33 rounds to threshold 0, which never sticks: the plain route gives the same bits.)
+static bool repeat_route(const sf_handle* h) { return h->action_repeat > 1 || h->sticky.threshold > 0; }
+
 // The launch shape (EB, ngroups, sched) and the instantiation are chosen here; callers set the other fields. f: feature
 // rows (render off only). a.T counts agent steps.
 static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st, bool draw = false, SfFeatArgs f = {}) {
   const SfDev& d = h->dev;
   bool render = (a.flags & SF_FLAG_RENDER) && a.obs;
-  if (!draw && h->action_repeat > 1) {
-    // Action repeat: the state-only repeat kernel runs the ticks. Without frames it takes all T agent steps in one launch.
+  if (!draw && repeat_route(h)) {
+    // Action repeat / sticky actions: the state-only repeat kernel runs the ticks (and the sticky draws). Without frames it
+    // takes all T agent steps in one launch.
     // With frames every agent step is two launches on `st`: the repeat kernel for that step (T = 1), then a draw of the
     // state it left into the step's frame slot. (The fused kernel's stepping warp is its critical side already: k ticks
     // per drawn tick would make it the bottleneck; DESIGN.md 4.6.)
@@ -1127,8 +1162,15 @@ static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st, bool draw
         s.reward = a.reward ? a.reward + o : nullptr; s.done = a.done ? a.done + o : nullptr;
         s.fortkill = a.fortkill ? a.fortkill + o : nullptr; s.events = a.events ? a.events + o : nullptr;
       }
-      if (f.out) sf_step_repeat_kernel<true><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, h->action_repeat);
-      else sf_step_repeat_kernel<false><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, h->action_repeat);
+      const int k = h->action_repeat;
+      const SfStickyArgs& y = h->sticky;
+      if (y.threshold) {
+        if (f.out) sf_step_repeat_kernel<true, true><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y);
+        else sf_step_repeat_kernel<false, true><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y);
+      } else {
+        if (f.out) sf_step_repeat_kernel<true, false><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y);
+        else sf_step_repeat_kernel<false, false><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y);
+      }
       CUDA_TRY(cudaGetLastError());
       if (render) {
         SfRollArgs r = {};
@@ -1332,6 +1374,21 @@ extern "C" int sf_set_action_repeat(sf_handle* h, int k) {
 }
 extern "C" int sf_action_repeat(const sf_handle* h) { return h ? h->action_repeat : -1; }
 
+static bool sticky_p_ok(double p) { return p >= 0.0 && p <= 1.0; }  // false for NaN
+static unsigned long long sticky_threshold(double p) { return (unsigned long long)std::llround(p * 4294967296.0); }
+extern "C" int sf_set_sticky_actions(sf_handle* h, double p, uint32_t seed) {
+  if (!h) return fail(SF_ERR_INVALID, "handle is NULL");
+  if (!sticky_p_ok(p)) return fail(SF_ERR_INVALID, "repeat_action_probability must be in [0, 1]");
+  h->sticky_p = p;
+  h->sticky = SfStickyArgs{sticky_threshold(p), seed};
+  return SF_OK;
+}
+extern "C" double sf_sticky_actions(const sf_handle* h) { return h ? h->sticky_p : -1.0; }
+extern "C" int sf_sticky_draw(uint32_t seed, long long global_env, uint32_t rng_count, int32_t tick, double p) {
+  if (!sticky_p_ok(p)) return fail(-1, "repeat_action_probability must be in [0, 1]");
+  return sf_sticky_hash(seed, (unsigned long long)global_env, rng_count, tick, sticky_threshold(p)) ? 1 : 0;
+}
+
 extern "C" int sf_synthetic_action(uint32_t action_seed, long long global_env, long long t, int num_actions) {
   return sf_hash_action(action_seed, (unsigned long long)global_env, (unsigned long long)t, num_actions);
 }
@@ -1407,8 +1464,8 @@ static int step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_obs, flo
     }
   }
   const bool delta = want_delta && mir->host == h_obs && mir->bytes == obs_bytes;
-  // the blocks of the step kernel send their own frames' changes (with action repeat the frames come from a draw launch)
-  const bool fused_delta = delta && per % 16 == 0 && h->action_repeat == 1;
+  // the blocks of the step kernel send their own frames' changes (on the repeat route the frames come from a draw launch)
+  const bool fused_delta = delta && per % 16 == 0 && !repeat_route(h);
   CUDA_TRY(cudaStreamSynchronize(cudaStreamLegacy));  // calls made with stream == NULL (sf_reset, sf_seed ...) come first
   // page-locked actions / rewards / dones / kills / events are read and written in place by the kernel
   const int* k_actions = (const int*)device_alias(h_actions);

@@ -48,7 +48,7 @@ def _torch():
 class SFVecEnv(object):
     def __init__(self, env_id="SpaceFortress-youturn-image-v0", num_envs=16, device=0, action_set=1, seeds=None,
                  render=True, native_obs=False, autoreset=True, first_global_env=0, copy_outputs=False, obs_type="image",
-                 host_delta=True, action_repeat=1):
+                 host_delta=True, action_repeat=1, repeat_action_probability=0.0, sticky_seed=0):
         """copy_outputs (numpy path): False = step() returns views of the env's page-locked output buffers, which the
         next step() overwrites, and `infos` as a bool ndarray (the fast path); True = fresh arrays every step and
         `infos` as a tuple of N bools, exactly what gym_vecenv's np.stack returns; "ring" (SubprocVecEnv / DummyVecEnv
@@ -65,7 +65,10 @@ class SFVecEnv(object):
         action_repeat: game ticks per agent step (gym's `frameskip`, sf_set_action_repeat): every step() and each of the T
         steps of rollout(T) repeats its action for up to action_repeat ticks, stopping at the tick an episode ends; the
         reward is the sum over those ticks, done / infos / events are set by any of them, and the observation is that of
-        the state after the last one. 1 (default) is the plain one-tick step."""
+        the state after the last one. 1 (default) is the plain one-tick step.
+        repeat_action_probability, sticky_seed: sticky actions (ALE's repeat_action_probability, sf_set_sticky_actions):
+        every game tick keeps the keys the env already holds with probability p instead of taking the action's, drawn on
+        the device from (sticky_seed, the env's global index, its rand() count and tick). 0.0 (default) never sticks."""
         self.L = _lib.lib()
         self.gametype = _gametype(env_id)
         self.num_envs = int(num_envs)
@@ -92,6 +95,18 @@ class SFVecEnv(object):
             self.L.sf_destroy(self.h)
             self.h = None
             raise ValueError("action_repeat must be in [1, %d]: %s" % (_lib.MAX_ACTION_REPEAT, msg.decode() if msg else "?"))
+        self.repeat_action_probability = float(repeat_action_probability)
+        self.sticky_seed = int(sticky_seed)
+        if not 0 <= self.sticky_seed < 1 << 32:  # the draw takes a uint32 seed: anything else would alias another seed
+            self.L.sf_destroy(self.h)
+            self.h = None
+            raise ValueError("sticky_seed must be in [0, 2**32)")
+        rc = self.L.sf_set_sticky_actions(self.h, self.repeat_action_probability, self.sticky_seed)
+        if rc != _lib.SF_OK:
+            msg = self.L.sf_last_error()
+            self.L.sf_destroy(self.h)
+            self.h = None
+            raise ValueError("repeat_action_probability must be in [0, 1]: %s" % (msg.decode() if msg else "?"))
         self.num_actions = self.L.sf_num_actions(self.h)
         self.action_space = Discrete(self.num_actions)
         self.obs_shape = (1, _lib.NATIVE_H, _lib.NATIVE_W) if native_obs else (1, _lib.OBS_H, _lib.OBS_W)
