@@ -200,6 +200,31 @@ int sf_set_sticky_actions(sf_handle* h, double p, uint32_t seed);
 double sf_sticky_actions(const sf_handle* h);
 int sf_sticky_draw(uint32_t seed, long long global_env, uint32_t rng_count, int32_t tick, double p);
 
+/* Extension: final observations at auto-reset (SB3's info["terminal_observation"], Gymnasium's same-step autoreset
+ * final_obs). Every episode ends at the time limit (5295 ticks) and the clock is not observed, so every `done` is a
+ * truncation: a learner bootstraps from V(final observation), which the in-kernel auto-reset would otherwise overwrite.
+ * A handle setting, off by default; off, every entry point behaves bit for bit as without it.
+ * d_final_step int32[n] is required when either buffer is set; all three NULL disables (the default).
+ * While enabled, every call of sf_step, sf_rollout, sf_step_host, sf_rollout_features and sf_step_host_features:
+ *   - writes d_final_step[i] for every env: the agent step index t (0 <= t < T) whose events carry SF_EV_EPISODE_RESET,
+ *     or -1 (final_step[i] == t <=> events[t][i] & SF_EV_EPISODE_RESET);
+ *   - in calls that draw frames, writes d_frames + i * frame_bytes for every env i that was auto-reset in the call: the
+ *     frame (84x84, or 92x90 with SF_FLAG_NATIVE_OBS, as the call's frames) of the state after the ending tick and
+ *     before the new game, bit for bit what sf_render gives for that state (the state SF_FLAG_NO_AUTORESET would leave);
+ *   - in the feature entry points, writes d_rows + i * F (F = the call's row width) with that state's row of the call's
+ *     obs_type, bit for bit what sf_features (float32) gives; a buffer of n * 19 floats covers every kind;
+ *   - leaves the frame and row slots of the envs that did not end untouched. Under SF_FLAG_NO_AUTORESET there is no
+ *     auto-reset: d_final_step is all -1 and nothing else is written.
+ * An env ends at most once in a call when T * k <= 5295 (k = action repeat): after an end, fewer than 5295 ticks remain.
+ * A call with T * k > 5295 while the setting is enabled returns SF_ERR_INVALID and launches nothing. Observations,
+ * rewards, done, kill, events, the env state after the call, sf_episode_stats and the rand() / sticky draw streams equal
+ * the disabled run's; sf_reset, sf_render, sf_features and the env blobs do not depend on the setting, and a blob row
+ * does not hold it. The buffers must stay valid while registered; sf_destroy forgets them. Every write is on the
+ * caller's stream without a host synchronise (CUDA graph capture works). sf_final_obs_enabled: 1 / 0, -1 for a NULL
+ * handle. */
+int sf_set_final_obs(sf_handle* h, uint8_t* d_frames, float* d_rows, int32_t* d_final_step);
+int sf_final_obs_enabled(const sf_handle* h);
+
 /* Render the current state without stepping (Game.draw + gray + resize). */
 int sf_render(sf_handle* h, uint8_t* d_obs, int flags, void* stream);
 

@@ -96,6 +96,8 @@ _PROTOTYPES = {
     "sf_set_sticky_actions": (C.c_int, [C.c_void_p, C.c_double, C.c_uint32]),
     "sf_sticky_actions": (C.c_double, [C.c_void_p]),
     "sf_sticky_draw": (C.c_int, [C.c_uint32, C.c_longlong, C.c_uint32, C.c_int32, C.c_double]),
+    "sf_set_final_obs": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "sf_final_obs_enabled": (C.c_int, [C.c_void_p]),
     "sf_render": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p]),
     "sf_step_host": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]),
     "sf_host_delta_stats": (C.c_int, [C.c_void_p, C.c_void_p]),

@@ -16,7 +16,9 @@
 //                               env and tick (sf_rollout_features, sf_step_host_features).
 //   sf_step_repeat_kernel       action repeat (sf_set_action_repeat, k > 1): the state-only step with up to k ticks of one
 //                               action per agent step; with frames each agent step is followed by a SF_ROLL_DRAW launch.
-//                               <*, true>: sticky actions (sf_set_sticky_actions, p > 0), at any k.
+//                               <*, true, *>: sticky actions (sf_set_sticky_actions, p > 0), at any k.
+//                               <*, *, SF_FINAL_IN_KERNEL / SF_FINAL_DEFERRED>: final observations (sf_set_final_obs).
+//   sf_final_reset_kernel       the deferred auto-reset of the envs whose final frames have just been drawn.
 //   sf_features_kernel          the feature observation types of ssf_env.py:95-157 of the current state, one env per thread.
 //   sf_policy_input_kernel      4-frame stack -> the policy's first-layer input (bf16 or fp32, space-to-depth NHWC).
 //   sf_reset_kernel / sf_seed_kernel / sf_get_state_kernel / sf_set_state_kernel / sf_pack_static_kernel
@@ -160,6 +162,17 @@ struct SfFeatArgs {
 struct SfStickyArgs {
   unsigned long long threshold;  // llround(p * 2^32): 0 never sticks, 2^32 always
   unsigned seed;
+};
+// Final observations at auto-reset (sf_set_final_obs): a parameter of the repeat kernel of its own, like SfStickyArgs.
+// SF_FINAL_IN_KERNEL: a finished env writes step[env] (and, with feature rows, its final row into rows) just before its
+// new game. SF_FINAL_DEFERRED (T = 1 launches with frames): a finished env writes step[env], is left finished and is
+// marked in `pending`; a masked draw and sf_final_reset_kernel follow.
+enum SfFinalMode { SF_FINAL_OFF, SF_FINAL_IN_KERNEL, SF_FINAL_DEFERRED };
+struct SfFinalArgs {
+  int* step;               // [n]: the agent step whose events carry SF_EV_EPISODE_RESET (written only for envs that end)
+  float* rows;             // [n][F.cols] or NULL: the final feature rows (SF_FINAL_IN_KERNEL with feature rows)
+  unsigned char* pending;  // [n]: SF_FINAL_DEFERRED's marks, cleared by sf_final_reset_kernel
+  int t0;                  // the agent step index of the launch's step 0
 };
 enum SfRollMode { SF_ROLL_STEP, SF_ROLL_STEP_HOST_DELTA, SF_ROLL_DRAW };
 // ticks per group, for both roles of a launch: a draw is the one frame of the current state
@@ -607,10 +620,15 @@ __global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_only_kernel(SfDev 
 // STICKY (sf_set_sticky_actions): before each executed tick the env draws (sf_sticky_hash of its pre-tick rand() count
 // and tick); on "stick" the tick runs with the keys the env holds instead of the action's, so it has no press or release
 // edges, and the agent step reports SF_EV_STICKY.
+// FINAL (sf_set_final_obs, SfFinalMode): IN_KERNEL stores the finished state's agent step index (and feature row) right
+// before sf_new_game; DEFERRED (launches of T = 1 only) stores the index, skips the episode accumulation and the new
+// game, and marks the env pending: the finished state is stored, drawn by a masked draw launch, and then reset by
+// sf_final_reset_kernel exactly as here. Events and shaping do not change: sf_env_step still runs with `autoreset`.
 static_assert(SF_CORE_FIRE == SF_KEY_FIRE << 23 && SF_CORE_THRUST == SF_KEY_THRUST << 23 && SF_CORE_LEFT == SF_KEY_LEFT << 23 &&
               SF_CORE_RIGHT == SF_KEY_RIGHT << 23, "the held keys are the key mask at bit 23 of the core word");
-template <bool FEAT, bool STICKY>
-__global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDev D, SfRollArgs A, SfFeatArgs F, int repeat, SfStickyArgs S) {
+template <bool FEAT, bool STICKY, int FINAL>
+__global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDev D, SfRollArgs A, SfFeatArgs F, int repeat, SfStickyArgs S, SfFinalArgs Z) {
+  static_assert(FINAL != SF_FINAL_DEFERRED || !FEAT, "the deferred reset serves the frame route, which has no feature rows");
   const int env = A.env0 + blockIdx.x * blockDim.x + threadIdx.x;
   const int lane = threadIdx.x & 31;
   const bool mine = env < A.env0 + A.envn;
@@ -640,9 +658,17 @@ __global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDe
         acc.done = o.done; ticking = !o.done;
         finished = o.done && autoreset;
       }
-      if (__any_sync(0xffffffffu, finished)) {
+      if constexpr (FINAL == SF_FINAL_DEFERRED) {
+        if (finished) { Z.step[env] = Z.t0 + t; Z.pending[env] = 1; }
+      } else if (__any_sync(0xffffffffu, finished)) {
         sf_accumulate_episode(D, env, e, finished, lane);
-        if (finished) sf_new_game(D, H, env, e);
+        if (finished) {
+          if constexpr (FINAL == SF_FINAL_IN_KERNEL) {
+            Z.step[env] = Z.t0 + t;
+            if constexpr (FEAT) if (Z.rows) sf_feature_row(e, D.autoturn != 0, F.kind, Z.rows + (size_t)env * F.cols);
+          }
+          sf_new_game(D, H, env, e);
+        }
       }
       if (mine && (tick & 7) == 7) sf_flush_stats(D, env, e);
     }
@@ -650,6 +676,25 @@ __global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDe
     if constexpr (FEAT) sf_feature_rows(D, A, F, e, mine, t);
   }
   if (mine) sf_store_env(D, env, e);
+}
+
+// The second half of SF_FINAL_DEFERRED's auto-reset, after the finished states have been drawn: the pending envs of
+// [env0, env0 + envn) are accumulated and get their new game as in the step kernels (one env per lane; the episode
+// statistics are integer sums and a max, so which lanes share a warp reduction does not change them). The step kernel's
+// sf_store_env has flushed the pending Stats increments: sf_accumulate_episode reads the counters the in-kernel reset
+// reads.
+__global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_final_reset_kernel(SfDev D, unsigned char* pending, int env0, int envn) {
+  const int env = env0 + blockIdx.x * blockDim.x + threadIdx.x;
+  const bool finished = env < env0 + envn && pending[env];
+  if (!__any_sync(0xffffffffu, finished)) return;
+  SfEnv e;
+  if (finished) sf_load_env(D, env, e);
+  sf_accumulate_episode(D, env, e, finished, threadIdx.x & 31);
+  if (finished) {
+    sf_new_game(D, &D.tab->hot, env, e);
+    sf_store_env(D, env, e);
+    pending[env] = 0;
+  }
 }
 
 // ---- state records (AoS <-> SoA), one thread per env ----
@@ -904,6 +949,10 @@ struct sf_handle {
   int action_repeat;  // ticks per agent step of every stepping entry point (sf_set_action_repeat), 1 by default
   double sticky_p;      // sf_set_sticky_actions: p, and the kernel's form of (p, seed); 0 by default
   SfStickyArgs sticky;
+  // sf_set_final_obs: the caller's device buffers (step == NULL: off), and the deferred reset's marks (uint8[n], zero
+  // between calls)
+  struct FinalObs { uint8_t* frames; float* rows; int32_t* step; } final_obs;
+  unsigned char* d_final_pending;
   void* slab;
   size_t slab_bytes;
   SfTables* h_tab;
@@ -1081,6 +1130,7 @@ extern "C" int sf_destroy(sf_handle* h) {
   if (h->d_kill) cudaFree(h->d_kill);
   if (h->d_events) cudaFree(h->d_events);
   if (h->d_sched) cudaFree(h->d_sched);
+  if (h->d_final_pending) cudaFree(h->d_final_pending);
   for (auto& m : h->mirrors) if (m.d) cudaFree(m.d);
   if (h->d_delta_stats) cudaFree(h->d_delta_stats);
   if (h->host_compute) cudaStreamDestroy(h->host_compute);
@@ -1134,10 +1184,22 @@ static void group_shape(const sf_handle* h, int n, int* EB, int* ngroups, int* b
   *blocks = std::min(*ngroups, sms);
 }
 
-// Whether the stepping entry points run their ticks in sf_step_repeat_kernel (action repeat k > 1, or sticky actions
-// with p > 0) rather than in the kernels of the plain one-tick step. With frames they then come from draw launches.
+// Whether the stepping entry points run their ticks in sf_step_repeat_kernel (action repeat k > 1, sticky actions with
+// p > 0, or final observations) rather than in the kernels of the plain one-tick step. With frames they then come from
+// draw launches.
 // (A p below 2^-33 rounds to threshold 0, which never sticks: the plain route gives the same bits.)
-static bool repeat_route(const sf_handle* h) { return h->action_repeat > 1 || h->sticky.threshold > 0; }
+static bool repeat_route(const sf_handle* h) {
+  return h->action_repeat > 1 || h->sticky.threshold > 0 || h->final_obs.step;
+}
+
+// the instantiation of the repeat kernel for a final-observation mode (the deferred reset has no feature rows)
+template <bool FEAT, bool STICKY>
+static void launch_step_repeat(int final_mode, int blocks, cudaStream_t st, const SfDev& d, const SfRollArgs& s, const SfFeatArgs& f, int k,
+                               const SfStickyArgs& y, const SfFinalArgs& z) {
+  if (final_mode == SF_FINAL_OFF) sf_step_repeat_kernel<FEAT, STICKY, SF_FINAL_OFF><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y, z);
+  else if (FEAT || final_mode == SF_FINAL_IN_KERNEL) sf_step_repeat_kernel<FEAT, STICKY, SF_FINAL_IN_KERNEL><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y, z);
+  else sf_step_repeat_kernel<false, STICKY, SF_FINAL_DEFERRED><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y, z);
+}
 
 // The launch shape (EB, ngroups, sched) and the instantiation are chosen here; callers set the other fields. f: feature
 // rows (render off only). a.T counts agent steps.
@@ -1145,12 +1207,22 @@ static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st, bool draw
   const SfDev& d = h->dev;
   bool render = (a.flags & SF_FLAG_RENDER) && a.obs;
   if (!draw && repeat_route(h)) {
-    // Action repeat / sticky actions: the state-only repeat kernel runs the ticks (and the sticky draws). Without frames it
-    // takes all T agent steps in one launch.
+    // Action repeat / sticky actions / final observations: the state-only repeat kernel runs the ticks (and the sticky
+    // draws). Without frames it takes all T agent steps in one launch.
     // With frames every agent step is two launches on `st`: the repeat kernel for that step (T = 1), then a draw of the
     // state it left into the step's frame slot. (The fused kernel's stepping warp is its critical side already: k ticks
-    // per drawn tick would make it the bottleneck; DESIGN.md 4.6.)
+    // per drawn tick would make it the bottleneck; DESIGN.md 4.6.) With final frames the repeat kernel defers the
+    // auto-reset, and a masked draw of the finished states and sf_final_reset_kernel come between the two (DESIGN.md 4.8).
     const int blocks = (a.envn + SF_STEP_ONLY_BLOCK - 1) / SF_STEP_ONLY_BLOCK;
+    const int k = h->action_repeat;
+    const sf_handle::FinalObs& fo = h->final_obs;
+    if (fo.step) {  // one end per env and call at most, so one slot per env is exact (sf_set_final_obs)
+      if ((long long)a.T * k > SF_GAME_TICKS)
+        return fail(SF_ERR_INVALID, "final observations: T * action_repeat must be <= " + std::to_string(SF_GAME_TICKS) + " (one episode end per env and call)");
+      CUDA_TRY(cudaMemsetAsync(fo.step + a.env0, 0xFF, sizeof(int32_t) * (size_t)a.envn, st));
+    }
+    const bool deferred = fo.step && render && fo.frames && !(a.flags & SF_FLAG_NO_AUTORESET);
+    const int final_mode = (!fo.step || (a.flags & SF_FLAG_NO_AUTORESET)) ? SF_FINAL_OFF : deferred ? SF_FINAL_DEFERRED : SF_FINAL_IN_KERNEL;
     SfRollArgs s = a;
     s.flags &= ~SF_FLAG_RENDER; s.obs = nullptr; s.host_obs = nullptr; s.mirror = nullptr; s.delta_stats = nullptr;
     if (render) s.T = 1;
@@ -1162,19 +1234,27 @@ static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st, bool draw
         s.reward = a.reward ? a.reward + o : nullptr; s.done = a.done ? a.done + o : nullptr;
         s.fortkill = a.fortkill ? a.fortkill + o : nullptr; s.events = a.events ? a.events + o : nullptr;
       }
-      const int k = h->action_repeat;
       const SfStickyArgs& y = h->sticky;
+      const SfFinalArgs z = {fo.step, f.out ? fo.rows : nullptr, h->d_final_pending, render ? t : 0};
       if (y.threshold) {
-        if (f.out) sf_step_repeat_kernel<true, true><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y);
-        else sf_step_repeat_kernel<false, true><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y);
+        if (f.out) launch_step_repeat<true, true>(final_mode, blocks, st, d, s, f, k, y, z);
+        else launch_step_repeat<false, true>(final_mode, blocks, st, d, s, f, k, y, z);
       } else {
-        if (f.out) sf_step_repeat_kernel<true, false><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y);
-        else sf_step_repeat_kernel<false, false><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y);
+        if (f.out) launch_step_repeat<true, false>(final_mode, blocks, st, d, s, f, k, y, z);
+        else launch_step_repeat<false, false>(final_mode, blocks, st, d, s, f, k, y, z);
       }
       CUDA_TRY(cudaGetLastError());
       if (render) {
         SfRollArgs r = {};
-        r.T = 1; r.obs = a.obs + (size_t)t * n * per; r.flags = a.flags; r.env0 = a.env0; r.envn = a.envn;
+        r.T = 1; r.flags = a.flags; r.env0 = a.env0; r.envn = a.envn;
+        if (deferred) {  // the finished states into their final-frame slots, then their new games
+          r.obs = fo.frames; r.draw_mask = h->d_final_pending;
+          if (int rc = launch_rollout(h, r, st, true)) return rc;
+          sf_final_reset_kernel<<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, h->d_final_pending, a.env0, a.envn);
+          CUDA_TRY(cudaGetLastError());
+          r.draw_mask = nullptr;
+        }
+        r.obs = a.obs + (size_t)t * n * per;
         if (int rc = launch_rollout(h, r, st, true)) return rc;
       }
     }
@@ -1388,6 +1468,19 @@ extern "C" int sf_sticky_draw(uint32_t seed, long long global_env, uint32_t rng_
   if (!sticky_p_ok(p)) return fail(-1, "repeat_action_probability must be in [0, 1]");
   return sf_sticky_hash(seed, (unsigned long long)global_env, rng_count, tick, sticky_threshold(p)) ? 1 : 0;
 }
+
+extern "C" int sf_set_final_obs(sf_handle* h, uint8_t* d_frames, float* d_rows, int32_t* d_final_step) {
+  if (!h) return fail(SF_ERR_INVALID, "handle is NULL");
+  if ((d_frames || d_rows) && !d_final_step) return fail(SF_ERR_INVALID, "final observations need d_final_step");
+  if (d_final_step && !h->d_final_pending) {
+    CUDA_TRY(cudaSetDevice(h->device));
+    CUDA_TRY(cudaMalloc(&h->d_final_pending, (size_t)h->dev.n));
+    CUDA_TRY(cudaMemset(h->d_final_pending, 0, (size_t)h->dev.n));
+  }
+  h->final_obs = sf_handle::FinalObs{d_frames, d_rows, d_final_step};
+  return SF_OK;
+}
+extern "C" int sf_final_obs_enabled(const sf_handle* h) { return h ? (h->final_obs.step != nullptr) : -1; }
 
 extern "C" int sf_synthetic_action(uint32_t action_seed, long long global_env, long long t, int num_actions) {
   return sf_hash_action(action_seed, (unsigned long long)global_env, (unsigned long long)t, num_actions);

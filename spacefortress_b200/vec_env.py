@@ -48,7 +48,7 @@ def _torch():
 class SFVecEnv(object):
     def __init__(self, env_id="SpaceFortress-youturn-image-v0", num_envs=16, device=0, action_set=1, seeds=None,
                  render=True, native_obs=False, autoreset=True, first_global_env=0, copy_outputs=False, obs_type="image",
-                 host_delta=True, action_repeat=1, repeat_action_probability=0.0, sticky_seed=0):
+                 host_delta=True, action_repeat=1, repeat_action_probability=0.0, sticky_seed=0, final_obs=False):
         """copy_outputs (numpy path): False = step() returns views of the env's page-locked output buffers, which the
         next step() overwrites, and `infos` as a bool ndarray (the fast path); True = fresh arrays every step and
         `infos` as a tuple of N bools, exactly what gym_vecenv's np.stack returns; "ring" (SubprocVecEnv / DummyVecEnv
@@ -68,7 +68,13 @@ class SFVecEnv(object):
         the state after the last one. 1 (default) is the plain one-tick step.
         repeat_action_probability, sticky_seed: sticky actions (ALE's repeat_action_probability, sf_set_sticky_actions):
         every game tick keeps the keys the env already holds with probability p instead of taking the action's, drawn on
-        the device from (sticky_seed, the env's global index, its rand() count and tick). 0.0 (default) never sticks."""
+        the device from (sticky_seed, the env's global index, its rand() count and tick). 0.0 (default) never sticks.
+        final_obs: keep the final observation of every episode that ends (sf_set_final_obs; SB3's
+        info["terminal_observation"]): every episode ends at the time limit, so `done` is a truncation and a learner
+        bootstraps from V(final observation). The env owns device buffers final_obs_buf [N] + obs_shape (uint8 frames or
+        float32 rows) and final_step_buf int32 [N]; rollout() adds them to its dict, final_observations() returns the
+        envs that ended in the last call and their observations. A rollout of T agent steps needs T * action_repeat <=
+        5295. False (default): nothing is kept."""
         self.L = _lib.lib()
         self.gametype = _gametype(env_id)
         self.num_envs = int(num_envs)
@@ -116,6 +122,10 @@ class SFVecEnv(object):
             self.obs_shape = (self.num_features,)
             self.observation_space = Box(-np.inf, np.inf, self.obs_shape, dtype=np.float32)  # ssf_env.py:176
         self.first_global_env = int(first_global_env)
+        self.final_obs = bool(final_obs)
+        self.final_obs_buf = self.final_step_buf = None
+        if self.final_obs:
+            self._register_final_obs(obs_type != "image")
         if seeds is not None or first_global_env:
             self.seed_streams(seeds, first_global_env)
         self._flags = (_lib.FLAG_RENDER if render else 0) | (_lib.FLAG_NATIVE_OBS if native_obs else 0) | \
@@ -129,6 +139,25 @@ class SFVecEnv(object):
         self.closed = False
 
     # ------------------------------------------------------------------ helpers
+    def _register_final_obs(self, features):
+        torch = _torch()
+        dev = self._device()
+        n = self.num_envs
+        if features or self.render_on:
+            dt = torch.float32 if features else torch.uint8
+            self.final_obs_buf = torch.zeros((n,) + self.obs_shape, dtype=dt, device=dev)
+        self.final_step_buf = torch.full((n,), -1, dtype=torch.int32, device=dev)
+        buf = self.final_obs_buf
+        rc = self.L.sf_set_final_obs(self.h, C.c_void_p(buf.data_ptr()) if buf is not None and not features else None,
+                                     C.c_void_p(buf.data_ptr()) if buf is not None and features else None,
+                                     C.c_void_p(self.final_step_buf.data_ptr()))
+        if rc != _lib.SF_OK:
+            msg = self.L.sf_last_error()
+            self.L.sf_destroy(self.h)
+            self.h = None
+            raise _lib.SFError("sf_set_final_obs: %s" % (msg.decode() if msg else "?"))
+        torch.cuda.synchronize(dev)  # the buffers' initial values are in place before any step reads or writes them
+
     def _device(self):
         return _torch().device("cuda", self.device_index)
 
@@ -352,7 +381,24 @@ class SFVecEnv(object):
             _lib.check(self.L.sf_rollout(self.h, int(T), aptr, int(action_seed), int(self._t), p("obs"), p("reward"), p("done"),
                                          p("kill"), flags, self._stream_ptr()))
         self._t += T
+        if self.final_obs:
+            out["final_step"] = self.final_step_buf
+            if self.final_obs_buf is not None:
+                out["final_obs"] = self.final_obs_buf
         return out
+
+    def final_observations(self, to_numpy=True):
+        """(idx, obs): the envs whose episode ended in the last stepping call (step() or rollout()) and their final
+        observations, the state after the ending tick and before the auto-reset (frames or feature rows as the env's
+        observations; None without them). Only those rows are copied. Needs final_obs=True."""
+        if not self.final_obs:
+            raise RuntimeError("final_observations() needs SFVecEnv(..., final_obs=True)")
+        self._stream_ptr()  # the gather below runs on torch's stream: a later host step waits for it
+        idx = (self.final_step_buf >= 0).nonzero().flatten()
+        obs = self.final_obs_buf.index_select(0, idx) if self.final_obs_buf is not None else None
+        if to_numpy:
+            return idx.cpu().numpy(), (obs.cpu().numpy() if obs is not None else None)
+        return idx, obs
 
     def synthetic_actions(self, T, action_seed=0, t0=None):
         """Host materialisation of the stream sf_rollout(actions=None) uses (parity runs)."""
