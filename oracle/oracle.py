@@ -88,6 +88,19 @@ def record_dtype():
     return dt
 
 
+def step_records(gametype, recs, keymask=0):
+    """One teacher-forced SSF_Env.step(keymask) from each state of `recs` (a record_dtype() array). Returns (the states
+    after the step, int32 [n, 4] of reward, done, fort_kill, events)."""
+    L = oracle_lib()
+    gt = L.sfo_gametype_from_name(gametype.encode())
+    if gt < 0:
+        raise RuntimeError("Unknown config value: `%s'" % gametype)
+    after = np.ascontiguousarray(recs, dtype=record_dtype()).copy()
+    out = np.zeros((len(after), 4), np.int32)
+    L.sfo_step_records(gt, after.ctypes.data, len(after), int(keymask), out.ctypes.data)
+    return after, out
+
+
 def build(force=False):
     """Compile libsforacle.so (always possible: gcc only) and _ref/libsfref.so (only where
     /root/reference exists; the prebuilt .so travels to the GPU box)."""
@@ -113,6 +126,7 @@ def oracle_lib():
         L.sfo_core_step.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_uint32)]
         L.sfo_env_step.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_int)]
         L.sfo_set_state.argtypes = [C.c_void_p, C.POINTER(Record)]
+        L.sfo_step_records.argtypes = [C.c_int, C.c_void_p, C.c_long, C.c_int, C.c_void_p]
         L.sfo_get_extra.argtypes = [C.c_void_p, C.POINTER(C.c_double)]
         L.sfo_dump.argtypes = [C.c_void_p, C.c_int, C.c_uint32, C.c_char_p, C.c_int]
         L.sfo_run.argtypes = [C.c_void_p, C.c_void_p, C.c_long, C.c_void_p]

@@ -413,6 +413,19 @@ void sfo_env_step(sfo_env* e, int keymask, int* out4) {
   out4[3] = (int)ev;
 }
 
+/* teacher-forced single steps over an array of states: recs[i] <- the state after sfo_env_step(keymask) from recs[i]
+ * (a fresh env of the game type each, the rand stream re-derived from the record); out4[4 * i ..] as sfo_env_step */
+void sfo_step_records(int gametype, sfr_record* recs, long n, int keymask, int* out4) {
+  sfo_env e;
+  for (long i = 0; i < n; i++) {
+    memset(&e, 0, sizeof(e));
+    e.gametype = gametype;
+    sfo_set_state(&e, &recs[i]);
+    sfo_env_step(&e, keymask, out4 + 4 * i);
+    recs[i] = e.s;
+  }
+}
+
 /* ---- P2: action tables (ssf_env.py:65-90) ---- */
 int sfo_num_actions(int gametype, int action_set) {
   int youturn = (gametype == SFO_YOUTURN || gametype == SFO_TEST_YOUTURN);

@@ -34,6 +34,7 @@ void sfo_reset(sfo_env* e);                               /* = SSF_Env.reset(): 
 int sfo_core_step(sfo_env* e, int keymask, uint32_t* events); /* = press/release keys + Game::stepOneTick(34) */
 void sfo_env_step(sfo_env* e, int keymask, int* out4);    /* = SSF_Env.step: out = reward, done, fort_kill, events */
 void sfo_set_state(sfo_env* e, const sfr_record* r);      /* teacher forcing (re-derives the rand stream) */
+void sfo_step_records(int gametype, sfr_record* recs, long n, int keymask, int* out4); /* sfo_set_state + sfo_env_step per record */
 void sfo_get_extra(const sfo_env* e, double* out4);       /* vdir, fdist, ndist, aim (game.cpp:282-312) */
 int sfo_dump(const sfo_env* e, int keymask, uint32_t events, char* buf, int cap); /* Game::dumpState */
 long sfo_run(sfo_env* e, const unsigned char* keymasks, long steps, unsigned char* obs84_last);

@@ -11,7 +11,7 @@ from oracle.oracle import Record
 GAMETYPES = ["youturn", "autoturn", "test-youturn", "test-autoturn"]
 KINDS = ["features", "normalized-features", "monitors"]
 END_TICK = 5295  # fixed episode length (game.cpp:487-489)
-FLOAT_REL_TOL = 1e-5  # north_star: continuous kinematics within 1e-5 relative per step
+SHELL_ABS_TOL = 1e-9  # shells carry the device fp64 atan2 / cos / sin (<= 2 ulp each): drift under 1e-11 over a shell's life
 FRAME_MATCH_FRACTION = 0.999
 FRAME_MAX_DELTA = 2
 STEP_OUTPUTS = ("reward", "done", "kill", "events")  # the per-env outputs of the stepping entry points, in argument order
@@ -39,13 +39,14 @@ def to_oracle_record(g):
 
 
 def assert_state_close(o, g, ctx):
-    """int_state() (stats included) exact; the shells within FLOAT_REL_TOL (device cos/sin), every other float bit-exact"""
+    """int_state() (stats included) exact; the shells within SHELL_ABS_TOL (device atan2 / cos / sin), every other float
+    bit-exact"""
     assert o.int_state() == to_oracle_record(g).int_state(), ctx
     fo, fg = o.float_state(), to_oracle_record(g).float_state()
     for key in fo:
         a, b = np.atleast_1d(np.array(fo[key], dtype=np.float64)), np.atleast_1d(np.array(fg[key], dtype=np.float64))
         if key.startswith("shell_"):
-            assert np.all(np.abs(a - b) <= FLOAT_REL_TOL * np.maximum(1.0, np.abs(a))), (ctx, key, a, b)
+            assert np.all(np.abs(a - b) <= SHELL_ABS_TOL), (ctx, key, a, b)
         else:
             assert np.array_equal(a, b), (ctx, key, a, b)
 
@@ -176,3 +177,27 @@ def step_host(env, actions, flags=0, pinned=True, want=("obs",) + STEP_OUTPUTS):
     if pinned and "obs" in buf:
         _lib.check(env.L.sf_host_forget(env.h, hp(buf["obs"])))  # the library may remember it for delta updates
     return out
+
+
+def oracle_features(o, kind, youturn):
+    """ssf_env.py:95-157 restated over the oracle's state and computeExtra (vdir, fdist, ndist, aim). Documented
+    divergences of the product are followed: len(shells) counts shells and the vulnerability timer is the real one (the
+    reference's getters for them are broken, pymodule.cpp:44-45,131-134)."""
+    s = o.get_state()
+    vdir, _fdist, ndist, aim = o.extra()
+    nm, ns = bin(s.missile_mask).count("1"), bin(s.shell_mask).count("1")
+    kill = 1 if s.vulnerability > 10 and s.fortress_vuln_timer < 250 else 0
+    timers = [s.fire_timer, s.thrust_timer, s.left_timer, s.right_timer]
+    timers = timers if youturn else timers[:2]
+    if kind == "monitors":
+        return np.array([0.5 if nm > 0 else -0.5, 0.5 if s.fortress_alive else -0.5, 0.5 if s.vulnerability > 10 else -0.5,
+                         0.5 if kill else -0.5, 0.5 if aim < 3 else -0.5, 0.5 if aim > 3 else -0.5, 0.5 if ndist > .75 else -0.5,
+                         0.5 if ndist > .25 else -0.5, 0.5 if ndist < -.25 else -0.5, 0.5 if ndist < -.75 else -0.5])
+    if kind == "normalized-features":
+        max_ticks = np.floor(180000 / 34)
+        f = [1 if s.ship_alive else 0, s.ship_x / 90, s.ship_y / 92, s.ship_vx / 10, s.ship_vy / 10, s.ship_angle / 360, aim / 180,
+             vdir % 360 / 360, ndist, 1 if s.fortress_alive else 0, s.fortress_angle / 360, max(s.vulnerability, 10) / 10, kill,
+             nm / 20, ns / 20] + [x / max_ticks for x in timers]
+        return np.clip(f, -1, 1)
+    return np.array([bool(s.ship_alive), s.ship_x, s.ship_y, s.ship_vx, s.ship_vy, s.ship_angle, aim, vdir, ndist, bool(s.fortress_alive),
+                     s.fortress_angle, s.vulnerability, kill, nm, ns] + timers, dtype=np.float64)

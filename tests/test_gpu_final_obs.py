@@ -8,10 +8,9 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from gpu_helpers import (GAMETYPES, KINDS, STEP_OUTPUTS, assert_state_close, make, outputs, ptrs, rollout, rollout_features,
-                         stagger, step_host, to_oracle_record, torch_cuda, vp)
+from gpu_helpers import (GAMETYPES, KINDS, STEP_OUTPUTS, assert_state_close, make, oracle_features, outputs, ptrs, rollout,
+                         rollout_features, stagger, step_host, to_oracle_record, torch_cuda, vp)
 from oracle.oracle import OracleEnv, draw_native, draw_obs
-from test_gpu_surface import oracle_features
 
 pytestmark = pytest.mark.gpu
 

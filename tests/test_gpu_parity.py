@@ -1,7 +1,6 @@
 """GPU (-m gpu): parity of the CUDA path, called through the C-ABI, against the oracle on the same seeded
-inputs. Bars (BASELINE.json north_star): integer state / events / episode boundaries bit-exact; continuous
-kinematics <= 1e-5 relative per step when teacher-forced (observed: bit-exact except shells, which carry the
-device cos/sin); frames >= 99.9 % identical pixels with max |delta| <= 2 (observed: bit-exact)."""
+inputs. Bars: integer state / events / episode boundaries bit-exact; continuous kinematics bit-exact except the
+shells, which carry the device fp64 atan2 / cos / sin and stay within 1e-9 absolute (gpu_helpers.SHELL_ABS_TOL); frames >= 99.9 % identical pixels with max |delta| <= 2 (observed: bit-exact)."""
 import ctypes as C
 import os
 
@@ -114,7 +113,7 @@ def test_kill_path_and_events():
 
 
 def test_teacher_forced_single_steps():
-    """load state -> one step -> compare (kinematics tolerance 1e-5 relative, ints exact)."""
+    """load state -> one step -> compare (shells within 1e-9 absolute, everything else exact)."""
     n = 64
     for gametype in ("youturn", "autoturn"):
         env = make(gametype, n, render=False, reset=False)
