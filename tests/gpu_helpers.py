@@ -12,8 +12,6 @@ GAMETYPES = ["youturn", "autoturn", "test-youturn", "test-autoturn"]
 KINDS = ["features", "normalized-features", "monitors"]
 END_TICK = 5295  # fixed episode length (game.cpp:487-489)
 SHELL_ABS_TOL = 1e-9  # shells carry the device fp64 atan2 / cos / sin (<= 2 ulp each): drift under 1e-11 over a shell's life
-FRAME_MATCH_FRACTION = 0.999
-FRAME_MAX_DELTA = 2
 STEP_OUTPUTS = ("reward", "done", "kill", "events")  # the per-env outputs of the stepping entry points, in argument order
 
 
@@ -51,10 +49,16 @@ def assert_state_close(o, g, ctx):
             assert np.array_equal(a, b), (ctx, key, a, b)
 
 
+def frame_diff(expected, got):
+    """(differing pixels, first differing pixel (row, column), largest |delta|) of two frames of the same shape"""
+    d = np.abs(np.asarray(expected, np.int32) - np.asarray(got, np.int32))
+    nz = np.argwhere(d)
+    return int(len(nz)), tuple(int(v) for v in nz[0]) if len(nz) else None, int(d.max())
+
+
 def assert_frame_close(expected, got, ctx):
-    d = np.abs(expected.astype(np.int32) - got.astype(np.int32))
-    assert d.max() <= FRAME_MAX_DELTA, (ctx, int(d.max()))
-    assert (d == 0).mean() >= FRAME_MATCH_FRACTION, (ctx, float((d == 0).mean()))
+    """frames bit-exact"""
+    assert np.array_equal(expected, got), (ctx,) + frame_diff(expected, got)
 
 
 def make(gametype, n, seeds=None, reset=True, warm=0, ends=None, device=0, **kw):

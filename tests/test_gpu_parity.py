@@ -1,6 +1,6 @@
 """GPU (-m gpu): parity of the CUDA path, called through the C-ABI, against the oracle on the same seeded
 inputs. Bars: integer state / events / episode boundaries bit-exact; continuous kinematics bit-exact except the
-shells, which carry the device fp64 atan2 / cos / sin and stay within 1e-9 absolute (gpu_helpers.SHELL_ABS_TOL); frames >= 99.9 % identical pixels with max |delta| <= 2 (observed: bit-exact)."""
+shells, which carry the device fp64 atan2 / cos / sin and stay within 1e-9 absolute (gpu_helpers.SHELL_ABS_TOL); frames bit-exact (gpu_helpers.assert_frame_close)."""
 import ctypes as C
 import os
 
