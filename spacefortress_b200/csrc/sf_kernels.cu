@@ -12,12 +12,14 @@
 //                               tables arrive as one bulk copy of a per-handle image (sf_pack_static_kernel).
 //                               Three instantiations (SfRollMode): step, step with host delta (sf_step_host), and draw
 //                               (sf_render, sf_reset: warp 0 loads the current state instead of stepping it).
-//   sf_step_only_kernel         state-only variant (render off), one env per thread; <true> also writes a feature row per
-//                               env and tick (sf_rollout_features, sf_step_host_features).
-//   sf_step_repeat_kernel       action repeat (sf_set_action_repeat, k > 1): the state-only step with up to k ticks of one
-//                               action per agent step; with frames each agent step is followed by a SF_ROLL_DRAW launch.
-//                               <*, true, *>: sticky actions (sf_set_sticky_actions, p > 0), at any k.
-//                               <*, *, SF_FINAL_IN_KERNEL / SF_FINAL_DEFERRED>: final observations (sf_set_final_obs).
+//   sf_step_state_kernel        the state-only step (render off), one env per thread, T agent steps of up to k ticks of
+//                               one action (sf_set_action_repeat). <FEAT, PLAIN, STICKY, FINAL>:
+//                               FEAT: a feature row per env and agent step (sf_rollout_features, sf_step_host_features);
+//                               PLAIN: one tick per agent step, no sticky actions, no final observations;
+//                               STICKY: sticky actions (sf_set_sticky_actions, p > 0), at any k;
+//                               FINAL = SF_FINAL_IN_KERNEL / SF_FINAL_DEFERRED: final observations (sf_set_final_obs).
+//                               When frames need the split route (frames_need_split), each agent step is this kernel at
+//                               T = 1 followed by a SF_ROLL_DRAW launch.
 //   sf_final_reset_kernel       the deferred auto-reset of the envs whose final frames have just been drawn.
 //   sf_features_kernel          the feature observation types of ssf_env.py:95-157 of the current state, one env per thread.
 //   sf_policy_input_kernel      4-frame stack -> the policy's first-layer input (bf16 or fp32, space-to-depth NHWC).
@@ -134,7 +136,7 @@ struct SfSched {
 };
 
 struct SfRollArgs {
-  int T, EB, ngroups, flags;  // EB = envs per group (<= 32), ngroups = ceil(n / EB): set by launch_rollout
+  int T, EB, ngroups, flags;  // EB = envs per group (<= 32), ngroups = ceil(n / EB): set by group_shape
   const int* actions;  // [T][n] or NULL
   unsigned action_seed;
   long long t0;
@@ -143,7 +145,7 @@ struct SfRollArgs {
   unsigned char* done;
   unsigned char* fortkill;
   unsigned* events;
-  SfSched* sched;      // NULL: static assignment (block b owns groups b, b + gridDim.x, ...; no hand-out); set by launch_rollout
+  SfSched* sched;      // NULL: static assignment (block b owns groups b, b + gridDim.x, ...; no hand-out); set by launch_fused / launch_draw
   int env0, envn;      // the envs this launch steps: [env0, env0 + envn) (sf_step_host steps the slab in slices)
   // SF_FLAG_HOST_DELTA (sf_step_host, T == 1): every block ends by sending the changed granules of its own frames
   uint4* host_obs;     // device alias of the caller's page-locked observation buffer, or NULL
@@ -158,12 +160,12 @@ struct SfFeatArgs {
   float* out;      // NULL: no feature rows
   int kind, cols;  // SF_OBS_FEATURES / SF_OBS_NORMALIZED_FEATURES / SF_OBS_MONITORS, sf_feature_cols
 };
-// Sticky actions: a parameter of the repeat kernel of its own, for the same reason as SfFeatArgs
+// Sticky actions: a parameter of the state-only kernel of its own, for the same reason as SfFeatArgs
 struct SfStickyArgs {
   unsigned long long threshold;  // llround(p * 2^32): 0 never sticks, 2^32 always
   unsigned seed;
 };
-// Final observations at auto-reset (sf_set_final_obs): a parameter of the repeat kernel of its own, like SfStickyArgs.
+// Final observations at auto-reset (sf_set_final_obs): a parameter of the state-only kernel of its own, like SfStickyArgs.
 // SF_FINAL_IN_KERNEL: a finished env writes step[env] (and, with feature rows, its final row into rows) just before its
 // new game. SF_FINAL_DEFERRED (T = 1 launches with frames): a finished env writes step[env], is left finished and is
 // marked in `pending`; a masked draw and sf_final_reset_kernel follow.
@@ -192,12 +194,6 @@ __device__ __forceinline__ void sf_store_step_out(const SfDev& D, const SfRollAr
   if (A.done) A.done[oi] = o.done;
   if (A.fortkill) A.fortkill[oi] = o.fort_kill;
   if (A.events) A.events[oi] = o.events;
-}
-// one tick of one env (both step kernels; H: the step's tables): its action, the step, the step's outputs
-__device__ __forceinline__ void sf_tick_env(const SfDev& D, const SfHot* H, const SfRollArgs& A, int env, int t, bool autoreset, SfEnv& e, SfStepOut& o) {
-  const int km = sf_step_keys(D, A, env, t);
-  sf_env_step(D, H, env, e, km, autoreset, (A.flags & SF_FLAG_RAW_REWARD) != 0, o);
-  sf_store_step_out(D, A, env, t, o);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -229,7 +225,8 @@ __device__ __noinline__ void sf_step_group(const SfDev& D, const SfRollArgs& A, 
     SF_ST_USE(e.q0.x, e.q0.y);
     SF_ST(8);
     SfStepOut o;
-    sf_tick_env(D, H, A, env, t, autoreset, e, o);
+    sf_env_step(D, H, env, e, sf_step_keys(D, A, env, t), autoreset, (A.flags & SF_FLAG_RAW_REWARD) != 0, o);
+    sf_store_step_out(D, A, env, t, o);
     finished = o.done && autoreset;
     shell_vis = o.shell_vis;
   }
@@ -243,7 +240,7 @@ __device__ __noinline__ void sf_step_group(const SfDev& D, const SfRollArgs& A, 
     else {
       SS.pos[lane] = e.pos; SS.vel[lane] = e.vel;
       SS.q0[lane] = e.q0; SS.q1[lane] = e.q1; SS.q2[lane] = e.q2; SS.q3[lane] = e.q3; SS.st3[lane] = e.st3;
-      if ((t & 7) == 7) sf_flush_stats(D, env, e);  // the pending Stats increments are 8-bit fields: every 8 ticks is often enough (as in sf_step_only_kernel)
+      if ((t & 7) == 7) sf_flush_stats(D, env, e);  // the pending Stats increments are 8-bit fields: every 8 ticks is often enough (as in sf_step_state_kernel)
       SS.d0[lane] = e.d0; SS.d1[lane] = e.d1; SS.d2[lane] = e.d2;
     }
     sf_make_env_rec(e, env, shell_vis, recs[lane]);
@@ -464,7 +461,7 @@ __global__ void sf_reset_kernel(SfDev D, const unsigned char* mask, int clear_pr
 
 // ------------------------------------------------------------------------------------------------
 // feature observations (ssf_env.py:95-157), one thread per env: of the current state (sf_features_kernel) or of the
-// state after every tick (sf_step_only_kernel<true>)
+// state after every agent step (sf_step_state_kernel<true, ...>)
 // ------------------------------------------------------------------------------------------------
 // columns of a row: 15 + the key timers (4 youturn, 2 autoturn) for features / normalized-features, 10 for monitors
 __host__ __device__ inline int sf_feature_cols(int autoturn, int kind) { return kind == SF_OBS_MONITORS ? 10 : 15 + (autoturn ? 2 : 4); }
@@ -565,7 +562,7 @@ __device__ __forceinline__ void sf_store_span(float* out, const float* S, int pr
 // state-only step (render off): one env per thread
 // ------------------------------------------------------------------------------------------------
 #define SF_STEP_ONLY_BLOCK 128
-// The feature rows of step t (both state-only step kernels, all threads of the block): each env's row of its state e.
+// The feature rows of step t (the state-only step kernel, all threads of the block): each env's row of its state e.
 // In one step the rows of a block's envs are one contiguous span of the output: they are staged in shared memory (two
 // buffers, so one barrier per step) and leave as consecutive stores across each warp. One thread storing its own row
 // would scatter 4-byte stores 4 * nfeat bytes apart: in HBM, and across PCIe where sf_step_host_features writes straight
@@ -581,42 +578,15 @@ __device__ __forceinline__ void sf_feature_rows(const SfDev& D, const SfRollArgs
   sf_store_span(span, R, pre, min(SF_STEP_ONLY_BLOCK, A.env0 + A.envn - b0) * F.cols);
 }
 
-// FEAT: every tick also writes the feature row of each env's state after the tick (auto-reset included, sf_feature_rows).
-template <bool FEAT>
-__global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_only_kernel(SfDev D, SfRollArgs A, SfFeatArgs F) {
-  const int env = A.env0 + blockIdx.x * blockDim.x + threadIdx.x;
-  const int lane = threadIdx.x & 31;
-  const bool mine = env < A.env0 + A.envn;
-  const bool autoreset = !(A.flags & SF_FLAG_NO_AUTORESET);
-  SfEnv e;
-  if (mine) sf_load_env(D, env, e);
-  for (int t = 0; t < A.T; t++) {
-    bool finished = false;
-    if (mine) {
-      SfStepOut o;
-      sf_tick_env(D, &D.tab->hot, A, env, t, autoreset, e, o);
-      finished = o.done && autoreset;
-    }
-    if (__any_sync(0xffffffffu, finished)) {
-      sf_accumulate_episode(D, env, e, finished, lane);
-      if (finished) sf_new_game(D, &D.tab->hot, env, e);
-    }
-    if (mine && (t & 7) == 7) sf_flush_stats(D, env, e);  // the pending increments are 8-bit fields
-    if constexpr (FEAT) sf_feature_rows(D, A, F, e, mine, t);
-  }
-  if (mine) sf_store_env(D, env, e);
-}
-
-// ------------------------------------------------------------------------------------------------
-// action repeat (sf_set_action_repeat, k > 1): the state-only step, up to k ticks per agent step
-// ------------------------------------------------------------------------------------------------
 // Agent step t of an env ticks with the one key mask of its action until k ticks have run or one of them ends the
 // episode (gym's `frameskip`); index t of the outputs holds the sum of those ticks' rewards and the OR of their done, kill
 // and event bits, and FEAT's row t is the state after the agent step. The k iterations are warp-uniform (the loop ends
 // early only when no lane of the warp is still ticking), and a lane whose agent step is over just stops ticking: every
 // lane reaches the __any_sync of the episode accumulation. The pending Stats increments are 8-bit fields: they are
-// flushed every 8 iterations, that is every 8 ticks at most, whatever k is. A kernel of its own, with k a parameter:
-// sf_step_only_kernel keeps its code.
+// flushed every 8 iterations, that is every 8 ticks at most, whatever k is.
+// PLAIN (k = 1, no sticky actions, no final observations): the inner loop is one tick and asks no vote. The runtime-k
+// loop costs registers: <false, false, false, SF_FINAL_OFF> uses 94 against the plain step's 72, which at 128-thread
+// blocks is 20 resident warps per SM instead of 28 on the path that is HBM-bound at T = 1.
 // STICKY (sf_set_sticky_actions): before each executed tick the env draws (sf_sticky_hash of its pre-tick rand() count
 // and tick); on "stick" the tick runs with the keys the env holds instead of the action's, so it has no press or release
 // edges, and the agent step reports SF_EV_STICKY.
@@ -626,9 +596,10 @@ __global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_only_kernel(SfDev 
 // sf_final_reset_kernel exactly as here. Events and shaping do not change: sf_env_step still runs with `autoreset`.
 static_assert(SF_CORE_FIRE == SF_KEY_FIRE << 23 && SF_CORE_THRUST == SF_KEY_THRUST << 23 && SF_CORE_LEFT == SF_KEY_LEFT << 23 &&
               SF_CORE_RIGHT == SF_KEY_RIGHT << 23, "the held keys are the key mask at bit 23 of the core word");
-template <bool FEAT, bool STICKY, int FINAL>
-__global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDev D, SfRollArgs A, SfFeatArgs F, int repeat, SfStickyArgs S, SfFinalArgs Z) {
+template <bool FEAT, bool PLAIN, bool STICKY, int FINAL>
+__global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_state_kernel(SfDev D, SfRollArgs A, SfFeatArgs F, int repeat, SfStickyArgs S, SfFinalArgs Z) {
   static_assert(FINAL != SF_FINAL_DEFERRED || !FEAT, "the deferred reset serves the frame route, which has no feature rows");
+  static_assert(!PLAIN || (!STICKY && FINAL == SF_FINAL_OFF), "the plain step is one tick of the action's keys");
   const int env = A.env0 + blockIdx.x * blockDim.x + threadIdx.x;
   const int lane = threadIdx.x & 31;
   const bool mine = env < A.env0 + A.envn;
@@ -642,7 +613,7 @@ __global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDe
     SfStepOut acc;
     acc.reward = 0; acc.events = 0u; acc.done = false; acc.fort_kill = false;
     bool ticking = mine;
-    for (int j = 0; j < repeat && __any_sync(0xffffffffu, ticking); j++, tick++) {
+    for (int j = 0; j < (PLAIN ? 1 : repeat) && (PLAIN || __any_sync(0xffffffffu, ticking)); j++, tick++) {
       bool finished = false;
       if (ticking) {
         int keys = km;
@@ -657,6 +628,9 @@ __global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDe
         acc.reward += o.reward; acc.events |= o.events; acc.fort_kill |= o.fort_kill;
         acc.done = o.done; ticking = !o.done;
         finished = o.done && autoreset;
+        // the plain step stores its outputs now: kept until after the loop they live across the out-of-line episode
+        // accumulation, which made the feature-row instantiation 136 instructions longer and ~2 % slower
+        if constexpr (PLAIN) sf_store_step_out(D, A, env, t, o);
       }
       if constexpr (FINAL == SF_FINAL_DEFERRED) {
         if (finished) { Z.step[env] = Z.t0 + t; Z.pending[env] = 1; }
@@ -672,7 +646,7 @@ __global__ void __launch_bounds__(SF_STEP_ONLY_BLOCK) sf_step_repeat_kernel(SfDe
       }
       if (mine && (tick & 7) == 7) sf_flush_stats(D, env, e);
     }
-    if (mine) sf_store_step_out(D, A, env, t, acc);
+    if (!PLAIN && mine) sf_store_step_out(D, A, env, t, acc);
     if constexpr (FEAT) sf_feature_rows(D, A, F, e, mine, t);
   }
   if (mine) sf_store_env(D, env, e);
@@ -1184,97 +1158,94 @@ static void group_shape(const sf_handle* h, int n, int* EB, int* ngroups, int* b
   *blocks = std::min(*ngroups, sms);
 }
 
-// Whether the stepping entry points run their ticks in sf_step_repeat_kernel (action repeat k > 1, sticky actions with
-// p > 0, or final observations) rather than in the kernels of the plain one-tick step. With frames they then come from
-// draw launches.
-// (A p below 2^-33 rounds to threshold 0, which never sticks: the plain route gives the same bits.)
-static bool repeat_route(const sf_handle* h) {
+// Whether frames come from separate launches: the state kernel for each agent step, then a SF_ROLL_DRAW of the state it
+// left (action repeat k > 1, sticky actions with p > 0, or final observations), rather than from the fused kernel. The
+// fused kernel's stepping warp is its critical side already: k ticks per drawn tick would make it the bottleneck
+// (DESIGN.md 4.6). (A p below 2^-33 rounds to threshold 0, which never sticks: the fused kernel gives the same bits.)
+static bool frames_need_split(const sf_handle* h) {
   return h->action_repeat > 1 || h->sticky.threshold > 0 || h->final_obs.step;
 }
 
-// the instantiation of the repeat kernel for a final-observation mode (the deferred reset has no feature rows)
-template <bool FEAT, bool STICKY>
-static void launch_step_repeat(int final_mode, int blocks, cudaStream_t st, const SfDev& d, const SfRollArgs& s, const SfFeatArgs& f, int k,
-                               const SfStickyArgs& y, const SfFinalArgs& z) {
-  if (final_mode == SF_FINAL_OFF) sf_step_repeat_kernel<FEAT, STICKY, SF_FINAL_OFF><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y, z);
-  else if (FEAT || final_mode == SF_FINAL_IN_KERNEL) sf_step_repeat_kernel<FEAT, STICKY, SF_FINAL_IN_KERNEL><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y, z);
-  else sf_step_repeat_kernel<false, STICKY, SF_FINAL_DEFERRED><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, s, f, k, y, z);
+// The state-only step of a.T agent steps. step0: the call's agent step index of a's step 0 (final_step's values).
+static int launch_state(sf_handle* h, const SfRollArgs& a, const SfFeatArgs& f, int final_mode, int step0, cudaStream_t st) {
+  typedef void (*Kernel)(SfDev, SfRollArgs, SfFeatArgs, int, SfStickyArgs, SfFinalArgs);
+  // [FEAT][STICKY][final mode]; the deferred reset serves the frame route, which has no feature rows
+  static const Kernel kernels[2][2][3] = {
+      {{sf_step_state_kernel<false, false, false, SF_FINAL_OFF>, sf_step_state_kernel<false, false, false, SF_FINAL_IN_KERNEL>,
+        sf_step_state_kernel<false, false, false, SF_FINAL_DEFERRED>},
+       {sf_step_state_kernel<false, false, true, SF_FINAL_OFF>, sf_step_state_kernel<false, false, true, SF_FINAL_IN_KERNEL>,
+        sf_step_state_kernel<false, false, true, SF_FINAL_DEFERRED>}},
+      {{sf_step_state_kernel<true, false, false, SF_FINAL_OFF>, sf_step_state_kernel<true, false, false, SF_FINAL_IN_KERNEL>, nullptr},
+       {sf_step_state_kernel<true, false, true, SF_FINAL_OFF>, sf_step_state_kernel<true, false, true, SF_FINAL_IN_KERNEL>, nullptr}}};
+  static const Kernel plain_kernels[2] = {sf_step_state_kernel<false, true, false, SF_FINAL_OFF>, sf_step_state_kernel<true, true, false, SF_FINAL_OFF>};
+  const bool feat = f.out != nullptr, sticky = h->sticky.threshold > 0;
+  const bool plain = h->action_repeat == 1 && !sticky && final_mode == SF_FINAL_OFF;
+  const Kernel k = plain ? plain_kernels[feat] : kernels[feat][sticky][final_mode];
+  const sf_handle::FinalObs& fo = h->final_obs;
+  const SfFinalArgs z = {fo.step, feat ? fo.rows : nullptr, h->d_final_pending, step0};
+  k<<<(a.envn + SF_STEP_ONLY_BLOCK - 1) / SF_STEP_ONLY_BLOCK, SF_STEP_ONLY_BLOCK, 0, st>>>(h->dev, a, f, h->action_repeat, h->sticky, z);
+  CUDA_TRY(cudaGetLastError());
+  return SF_OK;
 }
 
-// The launch shape (EB, ngroups, sched) and the instantiation are chosen here; callers set the other fields. f: feature
-// rows (render off only). a.T counts agent steps.
-static int launch_rollout(sf_handle* h, SfRollArgs a, cudaStream_t st, bool draw = false, SfFeatArgs f = {}) {
-  const SfDev& d = h->dev;
-  bool render = (a.flags & SF_FLAG_RENDER) && a.obs;
-  if (!draw && repeat_route(h)) {
-    // Action repeat / sticky actions / final observations: the state-only repeat kernel runs the ticks (and the sticky
-    // draws). Without frames it takes all T agent steps in one launch.
-    // With frames every agent step is two launches on `st`: the repeat kernel for that step (T = 1), then a draw of the
-    // state it left into the step's frame slot. (The fused kernel's stepping warp is its critical side already: k ticks
-    // per drawn tick would make it the bottleneck; DESIGN.md 4.6.) With final frames the repeat kernel defers the
-    // auto-reset, and a masked draw of the finished states and sf_final_reset_kernel come between the two (DESIGN.md 4.8).
-    const int blocks = (a.envn + SF_STEP_ONLY_BLOCK - 1) / SF_STEP_ONLY_BLOCK;
-    const int k = h->action_repeat;
-    const sf_handle::FinalObs& fo = h->final_obs;
-    if (fo.step) {  // one end per env and call at most, so one slot per env is exact (sf_set_final_obs)
-      if ((long long)a.T * k > SF_GAME_TICKS)
-        return fail(SF_ERR_INVALID, "final observations: T * action_repeat must be <= " + std::to_string(SF_GAME_TICKS) + " (one episode end per env and call)");
-      CUDA_TRY(cudaMemsetAsync(fo.step + a.env0, 0xFF, sizeof(int32_t) * (size_t)a.envn, st));
-    }
-    const bool deferred = fo.step && render && fo.frames && !(a.flags & SF_FLAG_NO_AUTORESET);
-    const int final_mode = (!fo.step || (a.flags & SF_FLAG_NO_AUTORESET)) ? SF_FINAL_OFF : deferred ? SF_FINAL_DEFERRED : SF_FINAL_IN_KERNEL;
-    SfRollArgs s = a;
-    s.flags &= ~SF_FLAG_RENDER; s.obs = nullptr; s.host_obs = nullptr; s.mirror = nullptr; s.delta_stats = nullptr;
-    if (render) s.T = 1;
-    const size_t n = (size_t)d.n, per = (a.flags & SF_FLAG_NATIVE_OBS) ? (size_t)SF_NAT_H * SF_NAT_W : (size_t)84 * 84;
-    for (int t = 0; t < (render ? a.T : 1); t++) {
-      if (render) {  // agent step t alone: its slot of every time-major array
-        const size_t o = (size_t)t * n;
-        s.actions = a.actions ? a.actions + o : nullptr; s.t0 = a.t0 + t;
-        s.reward = a.reward ? a.reward + o : nullptr; s.done = a.done ? a.done + o : nullptr;
-        s.fortkill = a.fortkill ? a.fortkill + o : nullptr; s.events = a.events ? a.events + o : nullptr;
-      }
-      const SfStickyArgs& y = h->sticky;
-      const SfFinalArgs z = {fo.step, f.out ? fo.rows : nullptr, h->d_final_pending, render ? t : 0};
-      if (y.threshold) {
-        if (f.out) launch_step_repeat<true, true>(final_mode, blocks, st, d, s, f, k, y, z);
-        else launch_step_repeat<false, true>(final_mode, blocks, st, d, s, f, k, y, z);
-      } else {
-        if (f.out) launch_step_repeat<true, false>(final_mode, blocks, st, d, s, f, k, y, z);
-        else launch_step_repeat<false, false>(final_mode, blocks, st, d, s, f, k, y, z);
-      }
-      CUDA_TRY(cudaGetLastError());
-      if (render) {
-        SfRollArgs r = {};
-        r.T = 1; r.flags = a.flags; r.env0 = a.env0; r.envn = a.envn;
-        if (deferred) {  // the finished states into their final-frame slots, then their new games
-          r.obs = fo.frames; r.draw_mask = h->d_final_pending;
-          if (int rc = launch_rollout(h, r, st, true)) return rc;
-          sf_final_reset_kernel<<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, h->d_final_pending, a.env0, a.envn);
-          CUDA_TRY(cudaGetLastError());
-          r.draw_mask = nullptr;
-        }
-        r.obs = a.obs + (size_t)t * n * per;
-        if (int rc = launch_rollout(h, r, st, true)) return rc;
-      }
-    }
-    return SF_OK;
-  }
-  if (render) {
-    int blocks;
-    group_shape(h, a.envn, &a.EB, &a.ngroups, &blocks);
-    // the hand-out counters serve full-slab steps only; draws, slices of the slab (sf_step_host) and in-kernel delta
-    // launches take static groups
-    a.sched = (!draw && a.env0 == 0 && a.envn == d.n && !a.host_obs) ? h->d_sched : nullptr;
-    if (draw) sf_rollout_kernel<SF_ROLL_DRAW><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
-    else if (a.host_obs) sf_rollout_kernel<SF_ROLL_STEP_HOST_DELTA><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
-    else sf_rollout_kernel<SF_ROLL_STEP><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(d, a);
-  } else {
-    const int blocks = (a.envn + SF_STEP_ONLY_BLOCK - 1) / SF_STEP_ONLY_BLOCK;
-    if (f.out) sf_step_only_kernel<true><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, a, f);
-    else sf_step_only_kernel<false><<<blocks, SF_STEP_ONLY_BLOCK, 0, st>>>(d, a, f);
-  }
+// SF_ROLL_DRAW: the frames of the current state (a.T = 1) of the envs a.draw_mask selects (NULL: all), static groups
+static int launch_draw(sf_handle* h, SfRollArgs a, cudaStream_t st) {
+  int blocks;
+  group_shape(h, a.envn, &a.EB, &a.ngroups, &blocks);
+  a.sched = nullptr;
+  sf_rollout_kernel<SF_ROLL_DRAW><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(h->dev, a);
   CUDA_TRY(cudaGetLastError());
+  return SF_OK;
+}
+
+// The fused step + render of a.T agent steps of one tick. The hand-out counters serve full-slab steps only; slices of the
+// slab (sf_step_host) and in-kernel delta launches take static groups.
+static int launch_fused(sf_handle* h, SfRollArgs a, cudaStream_t st) {
+  int blocks;
+  group_shape(h, a.envn, &a.EB, &a.ngroups, &blocks);
+  a.sched = (a.env0 == 0 && a.envn == h->dev.n && !a.host_obs) ? h->d_sched : nullptr;
+  if (a.host_obs) sf_rollout_kernel<SF_ROLL_STEP_HOST_DELTA><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(h->dev, a);
+  else sf_rollout_kernel<SF_ROLL_STEP><<<blocks, SF_BLOCK, SF_RENDER_SMEM_BYTES(SF_RENDER_WARPS), st>>>(h->dev, a);
+  CUDA_TRY(cudaGetLastError());
+  return SF_OK;
+}
+
+// a.T agent steps of [a.env0, a.env0 + a.envn): the launches of every stepping entry point. Frames when a.flags has
+// SF_FLAG_RENDER and a.obs is set; f: feature rows (render off only). Only enqueues on st (CUDA graph capture).
+static int launch_steps(sf_handle* h, const SfRollArgs& a, const SfFeatArgs& f, cudaStream_t st) {
+  const sf_handle::FinalObs& fo = h->final_obs;
+  const bool render = (a.flags & SF_FLAG_RENDER) && a.obs, autoreset = !(a.flags & SF_FLAG_NO_AUTORESET);
+  if (fo.step) {  // one end per env and call at most, so one slot per env is exact (sf_set_final_obs)
+    if ((long long)a.T * h->action_repeat > SF_GAME_TICKS)
+      return fail(SF_ERR_INVALID, "final observations: T * action_repeat must be <= " + std::to_string(SF_GAME_TICKS) + " (one episode end per env and call)");
+    CUDA_TRY(cudaMemsetAsync(fo.step + a.env0, 0xFF, sizeof(int32_t) * (size_t)a.envn, st));
+  }
+  // With final frames the state kernel defers the auto-reset: a masked draw of the finished states and
+  // sf_final_reset_kernel come between it and the step's draw (DESIGN.md 4.8).
+  const bool deferred = fo.step && render && fo.frames && autoreset;
+  const int final_mode = (!fo.step || !autoreset) ? SF_FINAL_OFF : deferred ? SF_FINAL_DEFERRED : SF_FINAL_IN_KERNEL;
+  if (!render) return launch_state(h, a, f, final_mode, 0, st);
+  if (!frames_need_split(h)) return launch_fused(h, a, st);
+  const size_t n = (size_t)h->dev.n, per = (a.flags & SF_FLAG_NATIVE_OBS) ? (size_t)SF_NAT_H * SF_NAT_W : (size_t)84 * 84;
+  SfRollArgs s = a, r = {};
+  s.T = 1;
+  r.T = 1; r.flags = a.flags; r.env0 = a.env0; r.envn = a.envn;
+  for (int t = 0; t < a.T; t++) {
+    const size_t o = (size_t)t * n;  // agent step t alone: its slot of every time-major array
+    s.actions = a.actions ? a.actions + o : nullptr; s.t0 = a.t0 + t;
+    s.reward = a.reward ? a.reward + o : nullptr; s.done = a.done ? a.done + o : nullptr;
+    s.fortkill = a.fortkill ? a.fortkill + o : nullptr; s.events = a.events ? a.events + o : nullptr;
+    if (int rc = launch_state(h, s, f, final_mode, t, st)) return rc;
+    if (deferred) {  // the finished states into their final-frame slots, then their new games
+      r.obs = fo.frames; r.draw_mask = h->d_final_pending;
+      if (int rc = launch_draw(h, r, st)) return rc;
+      sf_final_reset_kernel<<<(a.envn + SF_STEP_ONLY_BLOCK - 1) / SF_STEP_ONLY_BLOCK, SF_STEP_ONLY_BLOCK, 0, st>>>(h->dev, h->d_final_pending, a.env0, a.envn);
+      CUDA_TRY(cudaGetLastError());
+      r.draw_mask = nullptr;
+    }
+    r.obs = a.obs + o * per;
+    if (int rc = launch_draw(h, r, st)) return rc;
+  }
   return SF_OK;
 }
 
@@ -1393,7 +1364,7 @@ extern "C" int sf_reset(sf_handle* h, const uint8_t* d_mask, int clear_prev_vlne
   if (!d_obs) return SF_OK;
   SfRollArgs a = {};
   a.T = 1; a.obs = d_obs; a.flags = flags | SF_FLAG_RENDER; a.envn = h->dev.n; a.draw_mask = d_mask;
-  return launch_rollout(h, a, st, true);
+  return launch_draw(h, a, st);
 }
 
 extern "C" int sf_render(sf_handle* h, uint8_t* d_obs, int flags, void* stream) {
@@ -1401,7 +1372,7 @@ extern "C" int sf_render(sf_handle* h, uint8_t* d_obs, int flags, void* stream) 
   CUDA_TRY(cudaSetDevice(h->device));
   SfRollArgs a = {};
   a.T = 1; a.obs = d_obs; a.flags = flags | SF_FLAG_RENDER; a.envn = h->dev.n;
-  return launch_rollout(h, a, (cudaStream_t)stream, true);
+  return launch_draw(h, a, (cudaStream_t)stream);
 }
 
 extern "C" int sf_step(sf_handle* h, const int32_t* d_actions, uint8_t* d_obs, int32_t* d_reward, uint8_t* d_done,
@@ -1411,7 +1382,7 @@ extern "C" int sf_step(sf_handle* h, const int32_t* d_actions, uint8_t* d_obs, i
   SfRollArgs a = {};
   a.T = 1; a.flags = flags; a.actions = d_actions;
   a.obs = d_obs; a.reward = d_reward; a.done = d_done; a.fortkill = d_fortkill; a.events = d_events; a.envn = h->dev.n;
-  return launch_rollout(h, a, (cudaStream_t)stream);
+  return launch_steps(h, a, {}, (cudaStream_t)stream);
 }
 
 extern "C" int sf_rollout(sf_handle* h, int T, const int32_t* d_actions, uint32_t action_seed, long long t0, uint8_t* d_obs,
@@ -1421,7 +1392,7 @@ extern "C" int sf_rollout(sf_handle* h, int T, const int32_t* d_actions, uint32_
   SfRollArgs a = {};
   a.T = T; a.flags = flags; a.actions = d_actions; a.action_seed = action_seed; a.t0 = t0;
   a.obs = d_obs; a.reward = d_reward; a.done = d_done; a.fortkill = d_fortkill; a.envn = h->dev.n;
-  return launch_rollout(h, a, (cudaStream_t)stream);
+  return launch_steps(h, a, {}, (cudaStream_t)stream);
 }
 
 // the checks both feature steps share; *nf = the row width
@@ -1443,7 +1414,7 @@ extern "C" int sf_rollout_features(sf_handle* h, int obs_type, int T, const int3
   SfRollArgs a = {};
   a.T = T; a.flags = flags; a.actions = d_actions; a.action_seed = action_seed; a.t0 = t0;
   a.reward = d_reward; a.done = d_done; a.fortkill = d_fortkill; a.events = d_events; a.envn = h->dev.n;
-  return launch_rollout(h, a, (cudaStream_t)stream, false, SfFeatArgs{d_features, obs_type, nf});
+  return launch_steps(h, a, SfFeatArgs{d_features, obs_type, nf}, (cudaStream_t)stream);
 }
 
 extern "C" int sf_set_action_repeat(sf_handle* h, int k) {
@@ -1557,8 +1528,8 @@ static int step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_obs, flo
     }
   }
   const bool delta = want_delta && mir->host == h_obs && mir->bytes == obs_bytes;
-  // the blocks of the step kernel send their own frames' changes (on the repeat route the frames come from a draw launch)
-  const bool fused_delta = delta && per % 16 == 0 && !repeat_route(h);
+  // the blocks of the fused kernel send their own frames' changes (split frames come from draw launches)
+  const bool fused_delta = delta && per % 16 == 0 && !frames_need_split(h);
   CUDA_TRY(cudaStreamSynchronize(cudaStreamLegacy));  // calls made with stream == NULL (sf_reset, sf_seed ...) come first
   // page-locked actions / rewards / dones / kills / events are read and written in place by the kernel
   const int* k_actions = (const int*)device_alias(h_actions);
@@ -1579,7 +1550,7 @@ static int step_host(sf_handle* h, const int32_t* h_actions, uint8_t* h_obs, flo
   for (int k = 0; k < slices; k++) {
     const size_t e0 = n * k / slices, e1 = n * (k + 1) / slices;
     a.env0 = (int)e0; a.envn = (int)(e1 - e0);
-    rc = launch_rollout(h, a, sc, false, f);
+    rc = launch_steps(h, a, f, sc);
     if (rc) { cudaStreamSynchronize(sc); cudaStreamSynchronize(sx); return rc; }
     if (render && !delta) {
       CUDA_TRY(cudaEventRecord(h->host_ev[k], sc));

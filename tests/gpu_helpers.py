@@ -6,7 +6,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from oracle.oracle import Record
+from oracle.oracle import OracleEnv, Record
 
 GAMETYPES = ["youturn", "autoturn", "test-youturn", "test-autoturn"]
 KINDS = ["features", "normalized-features", "monitors"]
@@ -181,6 +181,50 @@ def step_host(env, actions, flags=0, pinned=True, want=("obs",) + STEP_OUTPUTS):
     if pinned and "obs" in buf:
         _lib.check(env.L.sf_host_forget(env.h, hp(buf["obs"])))  # the library may remember it for delta updates
     return out
+
+
+def oracles(gametype, recs):
+    """one OracleEnv per record, set to it"""
+    orc = []
+    for r in recs:
+        o = OracleEnv(gametype, 1)
+        o.set_state(to_oracle_record(r))
+        orc.append(o)
+    return orc
+
+
+def held_keys(s):
+    """the key mask an env holds (its FIRE / THRUST / LEFT / RIGHT flags)"""
+    from spacefortress_b200 import _lib
+    return ((_lib.KEY_FIRE if s.fire_flag else 0) | (_lib.KEY_THRUST if s.thrust_flag else 0) |
+            (_lib.KEY_LEFT if s.left_flag else 0) | (_lib.KEY_RIGHT if s.right_flag else 0))
+
+
+def oracle_agent_step(o, km, k=1, p=0.0, sticky_seed=0, genv=0, autoreset=True, features_of=None):
+    """One agent step of the oracle (gym's frameskip loop): up to k ticks with key mask km, stopping on the tick the
+    episode ends. With p > 0 each tick first draws sf_sticky_draw(sticky_seed, genv, ...) from the pre-tick state and on
+    "stick" runs with the held keys instead. (reward sum, done, kill, events OR, ticks run, end): end is None unless the
+    episode ended with autoreset, then the record of the finished state, or (record, features_of(o)) when features_of is
+    given (a function of the oracle in the finished state)."""
+    from spacefortress_b200 import _lib
+    R, K, EV = 0, False, 0
+    for j in range(k):
+        keys = km
+        if p:
+            s = o.state
+            if _lib.lib().sf_sticky_draw(sticky_seed, genv, s.rng_count, s.tick, p):
+                keys = held_keys(s)
+                EV |= _lib.EV_STICKY
+        r, d, kl, e = o.step(keys)
+        R += r; K |= kl; EV |= e
+        if d:
+            end = None
+            if autoreset:
+                EV |= _lib.EV_EPISODE_RESET
+                end = o.get_state() if features_of is None else (o.get_state(), features_of(o))
+                o.reset()
+            return R, True, K, EV, j + 1, end
+    return R, False, K, EV, k, None
 
 
 def oracle_features(o, kind, youturn):

@@ -7,38 +7,11 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from gpu_helpers import (END_TICK, GAMETYPES, KINDS, STEP_OUTPUTS, assert_state_close, hp, make, outputs, ptrs, rollout,
-                         rollout_features, single_steps, stagger, step_host, to_oracle_record, torch_cuda, vp)
-from oracle.oracle import OracleEnv, draw_native, draw_obs
+from gpu_helpers import (END_TICK, GAMETYPES, KINDS, STEP_OUTPUTS, assert_state_close, hp, make, oracle_agent_step, oracles,
+                         outputs, ptrs, rollout, rollout_features, single_steps, stagger, step_host, torch_cuda, vp)
+from oracle.oracle import draw_native, draw_obs
 
 pytestmark = pytest.mark.gpu
-
-
-def oracle_agent_step(o, km, k, autoreset=True):
-    """The wrapper loop: (reward sum, done, kill, events OR, ticks run, the record at the episode end or None)."""
-    from spacefortress_b200 import _lib
-    R, D, K, EV, end = 0, False, False, 0, None
-    for j in range(k):
-        r, d, kl, e = o.step(km)
-        R += r; K |= kl; EV |= e
-        if d:
-            D = True
-            if autoreset:
-                EV |= _lib.EV_EPISODE_RESET
-                end = o.get_state()
-                o.reset()
-            return R, D, K, EV, j + 1, end
-    return R, D, K, EV, k, end
-
-
-def oracles(gametype, recs):
-    """one OracleEnv per record, set to it"""
-    orc = []
-    for r in recs:
-        o = OracleEnv(gametype, 1)
-        o.set_state(to_oracle_record(r))
-        orc.append(o)
-    return orc
 
 
 # ------------------------------------------------------------------------------------------------ 1 + 4: the oracle
@@ -65,7 +38,7 @@ def run_against_oracle(gametype, k, n=48, T=160, flags=0, frame_every=4):
     ret = list(ret0)
     for t in range(T):
         for i in range(n):
-            R, D, K, EV, ran, end = oracle_agent_step(orc[i], orc[i].keymask(int(acts[t, i])), k, autoreset)
+            R, D, K, EV, ran, end = oracle_agent_step(orc[i], orc[i].keymask(int(acts[t, i])), k, autoreset=autoreset)
             assert (R, D, K) == (int(ga["reward"][t, i]), bool(ga["done"][t, i]), bool(ga["kill"][t, i])), (gametype, k, t, i)
             ret[i] += R
             if D:

@@ -8,9 +8,9 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from gpu_helpers import (GAMETYPES, KINDS, STEP_OUTPUTS, assert_state_close, make, oracle_features, outputs, ptrs, rollout,
-                         rollout_features, stagger, step_host, to_oracle_record, torch_cuda, vp)
-from oracle.oracle import OracleEnv, draw_native, draw_obs
+from gpu_helpers import (GAMETYPES, KINDS, STEP_OUTPUTS, assert_state_close, make, oracle_agent_step, oracle_features, oracles,
+                         outputs, ptrs, rollout, rollout_features, stagger, step_host, torch_cuda, vp)
+from oracle.oracle import draw_native, draw_obs
 
 pytestmark = pytest.mark.gpu
 
@@ -52,28 +52,6 @@ def kill_some(env, every=3):
     env.set_state(recs)
 
 
-def oracle_step(o, km, k, p, seed, genv, youturn):
-    """one agent step of the oracle: up to k ticks with sticky draws, stopping on the tick the episode ends.
-    (reward, done, kill, events, ticks run, (record, {kind: features}) of the finished state or None)"""
-    from spacefortress_b200 import _lib
-    L = _lib.lib()
-    R, K, EV = 0, False, 0
-    for j in range(k):
-        s = o.state
-        keys = km
-        if L.sf_sticky_draw(seed, genv, s.rng_count, s.tick, p):
-            keys = ((_lib.KEY_FIRE if s.fire_flag else 0) | (_lib.KEY_THRUST if s.thrust_flag else 0) |
-                    (_lib.KEY_LEFT if s.left_flag else 0) | (_lib.KEY_RIGHT if s.right_flag else 0))
-            EV |= _lib.EV_STICKY
-        r, d, kl, e = o.step(keys)
-        R += r; K |= kl; EV |= e
-        if d:
-            end = (o.get_state(), {kind: oracle_features(o, kind, youturn) for kind in KINDS})
-            o.reset()
-            return R, True, K, EV | _lib.EV_EPISODE_RESET, j + 1, end
-    return R, False, K, EV, k, None
-
-
 # ------------------------------------------------------------------------------------------------ the oracle
 @pytest.mark.parametrize("p", [0.0, 0.25])
 @pytest.mark.parametrize("k", [1, 3])
@@ -96,11 +74,7 @@ def test_final_observations_equal_the_oracle(gametype, k, p):
         stagger(env, ends)
     start = a.save_envs()
     fa, fb, fc = register(a), register(b), register(c)
-    orc = []
-    for r in a.get_state():
-        o = OracleEnv(gametype, 1)
-        o.set_state(to_oracle_record(r))
-        orc.append(o)
+    orc = oracles(gametype, a.get_state())
     acts = np.random.RandomState(k * 7 + len(gametype)).randint(a.num_actions, size=(T, n)).astype(np.int32)
     da = torch.from_numpy(acts).cuda()
     ga = {key: v.cpu().numpy() for key, v in rollout(a, T, da, flags=a._flags).items()}
@@ -115,11 +89,12 @@ def test_final_observations_equal_the_oracle(gametype, k, p):
     ev = gc["features"]["events"].cpu().numpy().view(np.uint32)
     fra, frb = frames_of(fa, 84 * 84).cpu().numpy(), frames_of(fb, NAT).cpu().numpy()
     youturn = gametype in ("youturn", "test-youturn")
+    features_of = lambda o: {kind: oracle_features(o, kind, youturn) for kind in KINDS}  # noqa: E731
     positions, dead = set(), 0
     for i in range(n):
         end_t = -1
         for t in range(T):
-            R, D, K, EV, ran, end = oracle_step(orc[i], orc[i].keymask(int(acts[t, i])), k, p, seed, i, youturn)
+            R, D, K, EV, ran, end = oracle_agent_step(orc[i], orc[i].keymask(int(acts[t, i])), k, p, seed, i, features_of=features_of)
             assert (R, D, K, EV) == (int(ga["reward"][t, i]), bool(ga["done"][t, i]), bool(ga["kill"][t, i]), int(ev[t, i])), (t, i)
             if D:
                 end_t = t

@@ -7,51 +7,11 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from gpu_helpers import (GAMETYPES, KINDS, STEP_OUTPUTS, assert_state_close, make, outputs, ptrs, rollout,
-                         rollout_features, stagger, step_host, to_oracle_record, torch_cuda, vp)
-from oracle.oracle import OracleEnv, draw_native, draw_obs
+from gpu_helpers import (GAMETYPES, KINDS, STEP_OUTPUTS, assert_state_close, make, oracle_agent_step, oracles, outputs, ptrs,
+                         rollout, rollout_features, stagger, step_host, torch_cuda, vp)
+from oracle.oracle import draw_native, draw_obs
 
 pytestmark = pytest.mark.gpu
-
-
-def held_keys(s):
-    """the key mask an env holds (its FIRE / THRUST / LEFT / RIGHT flags)"""
-    from spacefortress_b200 import _lib
-    return ((_lib.KEY_FIRE if s.fire_flag else 0) | (_lib.KEY_THRUST if s.thrust_flag else 0) |
-            (_lib.KEY_LEFT if s.left_flag else 0) | (_lib.KEY_RIGHT if s.right_flag else 0))
-
-
-def oracle_sticky_step(o, km, k, p, seed, genv, autoreset=True):
-    """One agent step of the oracle: up to k ticks, each drawing from the pre-tick state whether it keeps the held keys,
-    stopping on the tick the episode ends. (reward sum, done, kill, events OR, ticks run, the record at the episode end)"""
-    from spacefortress_b200 import _lib
-    L = _lib.lib()
-    R, D, K, EV, end = 0, False, False, 0, None
-    for j in range(k):
-        s = o.state
-        keys = km
-        if L.sf_sticky_draw(seed, genv, s.rng_count, s.tick, p):
-            keys = held_keys(s)
-            EV |= _lib.EV_STICKY
-        r, d, kl, e = o.step(keys)
-        R += r; K |= kl; EV |= e
-        if d:
-            D = True
-            if autoreset:
-                EV |= _lib.EV_EPISODE_RESET
-                end = o.get_state()
-                o.reset()
-            return R, D, K, EV, j + 1, end
-    return R, D, K, EV, k, end
-
-
-def oracles(gametype, recs):
-    orc = []
-    for r in recs:
-        o = OracleEnv(gametype, 1)
-        o.set_state(to_oracle_record(r))
-        orc.append(o)
-    return orc
 
 
 # ------------------------------------------------------------------------------------------------ the oracle
@@ -84,7 +44,7 @@ def test_sticky_steps_equal_the_oracle(gametype, p, k):
     positions, sticky = set(), 0
     for t in range(T):
         for i in range(n):
-            R, D, K, EV, ran, _ = oracle_sticky_step(orc[i], orc[i].keymask(int(acts[t, i])), k, p, seed, i)
+            R, D, K, EV, ran, _ = oracle_agent_step(orc[i], orc[i].keymask(int(acts[t, i])), k, p, seed, i)
             assert (R, D, K, EV) == (int(ga["reward"][t, i]), bool(ga["done"][t, i]), bool(ga["kill"][t, i]), int(ev[t, i])), (gametype, p, k, t, i)
             sticky += bool(EV & _lib.EV_STICKY)
             if D:
